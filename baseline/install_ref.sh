@@ -1,16 +1,18 @@
 #!/usr/bin/env bash
-# Installs the UNMODIFIED reference (DRCL-USC/isaac, /root/reference) into baseline/_ref (git-ignored, travels to the GPU
-# box with gpurun).  bench.py --impl reference and the runner test import `humanoid` from there.
+# Installs the UNMODIFIED reference (DRCL-USC/isaac) from a checkout of it into baseline/_ref (git-ignored).
+# bench.py --impl reference, the runner test and the live oracle-pinning tests import `humanoid` from there.
 #
-# /root/reference is read-only and setup.py writes build/ + egg-info next to itself, so pip installs from a copy under
-# /tmp.  The reference's setup.py uses find_packages(), which skips the directories that have no __init__.py
-# (humanoid/envs/base, humanoid/envs/custom: the reference is meant to be used with `pip install -e .`); the same source
-# files are added to the installed tree afterwards so that baseline/_ref holds the whole package.  --no-deps: the
-# declared dependencies (isaacgym preview4, mujoco, opencv, numpy==1.23.5, ...) are not installable here and are not
-# needed by the hot path (isaacgym is stubbed by oracle/ref_harness.py).
+#     baseline/install_ref.sh [checkout of DRCL-USC/isaac]     (default: $ISAAC_REFERENCE, else /root/reference)
+#
+# setup.py writes build/ + egg-info next to itself, so pip installs from a copy under a temporary directory (the
+# checkout may be read-only).  The reference's setup.py uses find_packages(), which skips the directories that have no
+# __init__.py (humanoid/envs/base, humanoid/envs/custom: the reference is meant to be used with `pip install -e .`); the
+# same source files are added to the installed tree afterwards so that baseline/_ref holds the whole package.
+# --no-deps: the declared dependencies (isaacgym preview4, mujoco, opencv, numpy==1.23.5, ...) are not needed by the hot
+# path (isaacgym is stubbed by oracle/ref_harness.py).
 set -euo pipefail
 ROOT="$(cd "$(dirname "$0")/.." && pwd)"
-SRC="${1:-/root/reference}"
+SRC="${1:-${ISAAC_REFERENCE:-/root/reference}}"
 TMP="$(mktemp -d)"
 cp -r "$SRC/humanoid" "$SRC/setup.py" "$TMP/"
 find "$TMP" -name __pycache__ -type d -prune -exec rm -rf {} +

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the hector hot path on B200 (contract: one JSON line on stdout from rank 0).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--envs E] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--envs E] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one `env.step(actions)` over E environments per GPU with the opaque physics stage
 stubbed (SURVEY.md §8d): action prologue + `decimation`=10 PD-torque sub-steps (10 launches), the fused
@@ -131,10 +131,36 @@ def workload_name(n):
     return f"hector task, {n} envs per GPU, env.step with stubbed physics (BASELINE configs[1])"
 
 
+DUMP_LIMIT_BYTES = 64_000_000          # 64 MB in all
+
+
+def dump_outputs(path, out):
+    """--dump-outputs: what env.step() returned in the last timed step, one float32 .npy per array - obs,
+    privileged_obs, rewards, resets, time_outs ([N, ...] rows per env) and episode_<name> (the scalars of
+    extras["episode"]).  Above 64 MB in all, the per-env arrays keep a fixed sample of env rows (seed 0, ascending
+    ids, the same rows in every array), so that runs with the same arguments write comparable files."""
+    import numpy as np
+    obs, priv, rew, reset, extras = out
+    per_env = {"obs": obs, "privileged_obs": priv, "rewards": rew, "resets": reset}
+    if "time_outs" in extras:
+        per_env["time_outs"] = extras["time_outs"]
+    n = obs.shape[0]
+    row_bytes = sum(4 * t[0].numel() for t in per_env.values())
+    if n * row_bytes > DUMP_LIMIT_BYTES:          # (one row less leaves room for the .npy headers and the episode scalars)
+        rows = np.sort(np.random.default_rng(0).choice(n, DUMP_LIMIT_BYTES // row_bytes - 1, replace=False))
+        ids = torch.from_numpy(rows).to(obs.device)
+        per_env = {k: t.index_select(0, ids) for k, t in per_env.items()}
+    arrays = {k: t.detach().float().cpu().numpy() for k, t in per_env.items()}
+    arrays.update({"episode_" + k: np.float32(float(v)) for k, v in extras.get("episode", {}).items()})
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), np.asarray(a, dtype=np.float32))
+
+
 # ------------------------------------------------------------------------------------ reference arm
 def reference_env(n, frames, seed):
     """The reference's CPU implementation of env.step on the workload's tape: the UNMODIFIED reference
-    (baseline/_ref, or /root/reference in the build container) through oracle/ref_harness.py when it is there
+    (found by oracle/ref_harness.py) when it is there
     (kind "reference"), else the oracle port (kind "port").  Returns (step(i), kind, description)."""
     from isaac_b200.envs.hector_config import HectorCfg
     tape = make_workload(n, frames, seed)
@@ -143,6 +169,8 @@ def reference_env(n, frames, seed):
         ref = ref_harness.ReferenceEnv(tape.statics, tape.physics[0], tape.noise[0])
         return (lambda i: ref.step(tape.physics[i % frames], tape.noise[i % frames]), "reference",
                 f"unmodified reference HectorFreeEnv.step ({ref_harness.reference_root()}), isaacgym stubbed")
+    print("bench.py: the unmodified reference is not found (set ISAAC_REFERENCE to a checkout of DRCL-USC/isaac); "
+          "the CPU arm times the oracle port instead (cpu_baseline.kind = \"port\")", file=sys.stderr, flush=True)
     from oracle.hector_oracle import OracleHectorEnv
     env = OracleHectorEnv(HectorCfg(), tape.statics, tape.physics[0], tape.noise[0])
     return (lambda i: env.step(tape.physics[i % frames], tape.noise[i % frames]), "port", "torch CPU oracle port")
@@ -170,8 +198,10 @@ def _reference_line(args):
         step(i)
     t0 = time.perf_counter()
     for i in range(args.steps):
-        step(args.warmup + i)
+        out = step(args.warmup + i)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out)
     value = n * args.steps / dt
     g = torch.Generator().manual_seed(0)
     r, v = torch.rand(T_GAE, n, 1, generator=g), torch.randn(T_GAE, n, 1, generator=g)
@@ -474,6 +504,8 @@ def run_b200(args, rank, world):
         if world > 1:
             dist.barrier()
 
+    last_out = [None]
+
     def one_step(i, timed):
         f = i % frames
         phys.load_frame(phys_frames[f])
@@ -483,7 +515,7 @@ def run_b200(args, rank, world):
         if timed:
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record(stream)
-        env.step(noise_frames[f].actions)
+        last_out[0] = env.step(noise_frames[f].actions)
         if timed:
             e1.record(stream)
             return e0, e1
@@ -500,6 +532,8 @@ def run_b200(args, rank, world):
     wall = time.perf_counter() - t0
     launches = lib.hb_launch_count() + (0 if args.no_graph else args.steps * env.graph_launches_per_step)
     dev_ms = sum(a.elapsed_time(b) for a, b in evs)
+    if args.dump_outputs and rank == 0:          # before the kernel timings below reuse the env's buffers
+        dump_outputs(args.dump_outputs, last_out[0])
 
     # ---- per-kernel timings for the roofline (each launch alone, L2 flushed before it) ----
     def time_launch(fn, reps=10):
@@ -805,7 +839,11 @@ def main():
     ap.add_argument("--skip-ppo", action="store_true", help="env stage only (tuning sweeps)")
     ap.add_argument("--ppo-updates", type=int, default=3, help="timed PPO updates (after one warm-up)")
     ap.add_argument("--skip-3xtf32", action="store_true", help="do not time the fp32-grade (3xTF32) update as well")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what env.step() returned in the last timed step as "
+                                                          "DIR/<name>.npy (float32, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
     if args.impl == "reference":

@@ -4,14 +4,14 @@ A torch-on-CPU restatement of the reference's per-environment hot path:
 PD torque law, action prologue, derived base quantities, heading command,
 termination, the 18 active reward terms, reset bookkeeping, frame-stacked
 observations and the `last_*` copies.  Each function cites the reference lines it
-follows (paths relative to /root/reference/humanoid).
+follows (paths relative to humanoid/ in DRCL-USC/isaac).
 
 Pinning: `tests/test_oracle_pinning.py` checks this file against golden vectors that
-`oracle/make_golden.py` produced by running the UNMODIFIED reference in the build
-container (`oracle/ref_harness.py`); in that container the same test also steps the
-reference live, side by side, and demands bit equality.  The quaternion helpers come
+`oracle/make_golden.py` produced by running the UNMODIFIED reference
+(`oracle/ref_harness.py`); where the reference is found, the same test also steps it
+live, side by side, and demands bit equality.  The quaternion helpers come
 from the closed third-party `isaacgym.torch_utils` (setup.py:43, `isaacgym # preview4`,
-absent from /root/reference): they are restated from the public definitions and have
+absent from the reference checkout): they are restated from the public definitions and have
 no reference-side test → *parity unpinned* for those three helpers; they are
 cross-checked against scipy instead.
 

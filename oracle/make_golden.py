@@ -1,8 +1,8 @@
-"""TEST INFRASTRUCTURE — build-container only: writes tests/golden/*.npz.
+"""TEST INFRASTRUCTURE — needs the reference (oracle/ref_harness.py): writes tests/golden/*.npz.
 
-Runs the UNMODIFIED reference from /root/reference (through `oracle/ref_harness.py`) on
-seeded synthetic tapes and records what it produced.  The GPU box has no
-/root/reference; there the oracle and the CUDA path are checked against these files.
+Runs the UNMODIFIED reference (through `oracle/ref_harness.py`) on seeded synthetic
+tapes and records what it produced.  Without the reference, the oracle and the CUDA
+path are checked against these files.
 
     python -m oracle.make_golden            # regenerate everything
 

@@ -1,16 +1,15 @@
 """TEST INFRASTRUCTURE — CPU oracle for the RL stage (not a product path).
 
-torch-on-CPU restatement of the rsl_rl fork under /root/reference/humanoid/algo/ppo:
+torch-on-CPU restatement of the rsl_rl fork under humanoid/algo/ppo of DRCL-USC/isaac:
 rollout storage + GAE (rollout_storage.py:52-136), minibatch generator (:146-182),
 ActorCritic MLPs with a diagonal Gaussian head (actor_critic.py:36-128) and the PPO
 act / process_env_step / compute_returns / update cycle (ppo.py:91-184).
 
 `torch` itself (nn.functional.linear/elu, autograd, optim.Adam, clip_grad_norm_) is
-part of the oracle: the reference pins no torch version (setup.py:43-52) and the image
-ships the same torch on the build container and on the GPU box.
+part of the oracle: the reference pins no torch version (setup.py:43-52).
 
-Pinned against the unmodified reference by `tests/test_oracle_pinning.py` (live in the
-build container, via golden vectors elsewhere).  Random draws are injected: `eps` for
+Pinned against the unmodified reference by `tests/test_oracle_pinning.py` (live where the
+reference is found, see `oracle/ref_harness.py`; via golden vectors everywhere).  Random draws are injected: `eps` for
 the action sample (a = mu + sigma*eps) and the minibatch permutation.
 
 Only `tests/`, `__graft_entry__.smoke()` and the `cpu_baseline` / `--impl reference`

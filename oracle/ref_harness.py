@@ -3,12 +3,12 @@
 Runs the UNMODIFIED reference (`humanoid/...`) on the CPU so that
 (a) the oracle restatement in `oracle/hector_oracle.py` can be pinned against it,
 (b) golden vectors can be generated for `tests/golden/` (see `oracle/make_golden.py`) and
-(c) `bench.py --impl reference` can time the reference's own code on the GPU box's host cores.
+(c) `bench.py --impl reference` can time the reference's own code on the host cores.
 
-The reference is imported from where it lies: `/root/reference` in the build container,
-else the installed copy under `baseline/_ref` (written by `baseline/install_ref.sh`;
-git-ignored, it travels to the GPU box with the snapshot).  No reference source is part
-of this repository's history.  `reference_root()` is None when neither exists.
+The reference is imported from a checkout of DRCL-USC/isaac: the one `$ISAAC_REFERENCE` names,
+else `/root/reference` (its default location), else the copy that `baseline/install_ref.sh`
+installed under `baseline/_ref` (git-ignored).  No reference source is part of this
+repository's history.  `reference_root()` is None when none of them exists.
 
 How (SURVEY.md §8c): the reference needs the closed third-party `isaacgym` package.
 We register stub modules for it — `isaacgym.torch_utils` is a restatement of the
@@ -37,9 +37,22 @@ import os
 _REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
+def _is_reference(root):
+    return bool(root) and os.path.isfile(os.path.join(root, "humanoid", "envs", "custom", "hector_env.py"))
+
+
+def reference_source():
+    """The upstream checkout given by $ISAAC_REFERENCE, else the default location; None when neither holds it."""
+    for root in (os.environ.get("ISAAC_REFERENCE"), "/root/reference"):
+        if _is_reference(root):
+            return root
+    return None
+
+
 def reference_root():
-    for root in ("/root/reference", os.path.join(_REPO, "baseline", "_ref")):
-        if os.path.isfile(os.path.join(root, "humanoid", "envs", "custom", "hector_env.py")):
+    """Where `humanoid` is imported from: the upstream checkout, else its copy under baseline/_ref."""
+    for root in (reference_source(), os.path.join(_REPO, "baseline", "_ref")):
+        if _is_reference(root):
             return root
     return None
 
@@ -111,8 +124,8 @@ def _normalize(x, eps: float = 1e-9):
 
 def install_isaacgym_stub():
     if REFERENCE_ROOT is None:
-        raise ImportError("the reference is neither at /root/reference nor installed under baseline/_ref "
-                          "(run baseline/install_ref.sh in the build container)")
+        raise ImportError("the reference is not found: set ISAAC_REFERENCE to a checkout of DRCL-USC/isaac "
+                          "or install one with baseline/install_ref.sh")
     if "isaacgym" in sys.modules:
         return
     tu = types.ModuleType("isaacgym.torch_utils")

@@ -9,7 +9,7 @@ import torch
 pytestmark = pytest.mark.gpu
 
 
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two GPUs (gpurun --gpus 2)")
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two GPUs")
 def test_data_parallel_update_matches_single_gpu(lib):
     here = os.path.dirname(os.path.abspath(__file__))
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node=2", "--master-addr", "127.0.0.1",
