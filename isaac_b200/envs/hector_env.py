@@ -360,7 +360,9 @@ class HectorFreeEnvB200:
         """Bind the draws of the next launch sequence: the injected tape if there is one, otherwise the device
         generator (Philox; key and step counter in `self._rng_state`): the tensors the reference
         draws with torch.rand / randn_like (hector_env.py:166,168,241; legged_robot.py:327-332,366,384) are never
-        materialised."""
+        materialised.  Every draw of one step uses the same counter; the step's last finalize launch advances it by one
+        (fused or staged hooks alike), and so does a reset_idx() called outside step().  The constructor's reset draws
+        at counter 0, step t of a freshly seeded env at counter t (oracle/device_rng.py mirrors the draws)."""
         nz = self._nz
         if self._injected is not None:
             f = self._injected
@@ -505,7 +507,8 @@ class HectorFreeEnvB200:
         """legged_robot.py:118-153 (termination, rewards, resets, observations, last_* copies): ONE fused launch plus the
         frame-stack / finalisation launch.  If a subclass overrides one of the reference's hooks (check_termination,
         compute_reward, reset_idx, compute_observations), the step instead calls the hooks one after the other in the
-        reference's order, each a launch of the same kernel restricted to that span - same results, six launches."""
+        reference's order, each a launch of the same kernel restricted to that span - same results and the same
+        device-generator draws (the reset inside the staged step draws at the step's counter and does not advance it)."""
         self.physics.refresh_post_physics()
         if not self._hooks_overridden():
             self._launch_post(HB_STAGE_STEP | (HB_STAGE_PUSH if push else 0))
@@ -516,6 +519,7 @@ class HectorFreeEnvB200:
 
     # ------------------------------------------------------------------ the reference's hooks, one by one
     _HOOKS = ("check_termination", "compute_reward", "reset_idx", "compute_observations")
+    _hold_rng_counter = False       # set while the staged step runs reset_idx: its finalize launch leaves the counter alone
 
     def _hooks_overridden(self) -> bool:
         cls = type(self)
@@ -543,7 +547,11 @@ class HectorFreeEnvB200:
         self.compute_reward()                                                      # :140
         env_ids = self.reset_buf.nonzero(as_tuple=False).flatten()                 # :142
         self._injected = keep
-        self.reset_idx(env_ids)                                                    # :143
+        self._hold_rng_counter = True       # reset_idx draws at this step's counter; compute_observations advances it
+        try:
+            self.reset_idx(env_ids)                                                # :143
+        finally:
+            self._hold_rng_counter = False
         self._injected = keep
         self.compute_observations()                                                # :144
         self._injected = keep
@@ -600,8 +608,9 @@ class HectorFreeEnvB200:
                                                  obs_new, priv_new, self._host_count.data_ptr(), noise.rng_counter, st),
                        "hb_env_stack_finalize")
         else:
+            counter = None if self._hold_rng_counter else noise.rng_counter
             _lib.check(lib.hb_env_reset_finalize(self._pp, self._pb, None, None, self._host_count.data_ptr(),
-                                                 noise.rng_counter, st), "hb_env_reset_finalize")
+                                                 counter, st), "hb_env_reset_finalize")
 
     def _apply_pending_resets(self):
         """The two opaque calls of _reset_dofs/_reset_root_states (legged_robot.py:370-372,394-396) need
@@ -642,7 +651,9 @@ class HectorFreeEnvB200:
         return self.privileged_obs_buf
 
     def reset_idx(self, env_ids):
-        """legged_robot.py:162-214 + hector_env.py:256-261 for an explicit id list (outside step())."""
+        """legged_robot.py:162-214 + hector_env.py:256-261 for an explicit id list.  Called outside step(), it takes
+        its draws at the current counter and advances it; inside the staged step it leaves that to
+        compute_observations."""
         env_ids = torch.as_tensor(env_ids, device=self.device, dtype=torch.long)
         if env_ids.numel() == 0:
             return

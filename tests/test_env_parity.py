@@ -9,7 +9,7 @@ import numpy as np
 import pytest
 import torch
 
-from _util import GOLDEN, assert_close, assert_equal, to_np
+from _util import ENV_ATOL, GOLDEN, assert_close, assert_equal, to_np
 from isaac_b200.envs.hector_config import HectorCfg
 from isaac_b200.synthetic import make_tape
 from oracle import make_golden as mg
@@ -19,7 +19,8 @@ pytestmark = pytest.mark.gpu
 EXACT = ("reset", "time_outs", "episode_length_buf", "last_contacts")
 
 
-def make_cuda_env(tape, dev, cfg=None, cls=None):
+def make_cuda_env(tape, dev, cfg=None, cls=None, device_rng=False):
+    """`device_rng`: the constructor's reset takes its draws from the device generator (cfg.seed) instead of the tape."""
     from isaac_b200.envs.hector_env import HectorFreeEnvB200
     from isaac_b200.physics import SyntheticPhysics
     from isaac_b200.synthetic import task_dims
@@ -28,7 +29,7 @@ def make_cuda_env(tape, dev, cfg=None, cls=None):
     phys = SyntheticPhysics(n, num_dof=dims.ndof, num_bodies=dims.nbody, device=dev)
     phys.load_frame(tape.physics[0].to(dev))
     env = (cls or HectorFreeEnvB200)(cfg or HectorCfg(), sim_device=str(dev), physics=phys, statics=tape.statics,
-                                     initial_noise=tape.noise[0].to(dev))
+                                     initial_noise=None if device_rng else tape.noise[0].to(dev))
     env.episode_length_buf.copy_(tape.statics.episode_length0)
     return env, phys
 
@@ -69,7 +70,9 @@ def run_cuda_case(tape, dev, step_counter0=0, cfg=None, cls=None):
     return rec, ids_per_step, env, phys
 
 
-def compare_records(got, want):
+def compare_records(got, want, extra_atol=None):
+    """`extra_atol`: {record key: array broadcast against that record}, added to the suite's absolute tolerance."""
+    extra_atol = extra_atol or {}
     for k in EXACT:
         assert_equal(k, got[k], want[k])
     for k in want:
@@ -78,7 +81,7 @@ def compare_records(got, want):
         w = want[k]
         if k.endswith("_init"):      # the constructor's compute_observations() is not clipped by the reference
             w = np.clip(w, -100.0, 100.0)   # (only step() clips, legged_robot.py:104-107); history frames are equal after the clip
-        assert_close(k, got[k], w)
+        assert_close(k, got[k], w, atol=ENV_ATOL + extra_atol.get(k, 0.0))
 
 
 @pytest.mark.parametrize("bulk", [1, 0])
