@@ -1396,34 +1396,10 @@ using ShapeXBot = StackShape<47, 15, 73, 3>;
 constexpr int ROW_OBS = ShapeHector::ROW_A, ROW_PRIV = ShapeHector::ROW_B, OBS = 41, PRIV = 70;      // hb_stack_shift's fast paths
 
 template <typename S>
-int shape_layout(const hb_env_params *p) {      // 0 = other shape, 1 = dense rows, 2 = 16-byte pitch
-    const int row_a = p->frame_stack * p->num_single_obs, row_b = p->c_frame_stack * p->num_single_priv;
-    if (row_a != S::ROW_A || p->num_single_obs != S::FRAME_A || row_b != S::ROW_B || p->num_single_priv != S::FRAME_B) return 0;
-    const int ld_a = p->obs_ld ? p->obs_ld : row_a, ld_b = p->priv_ld ? p->priv_ld : row_b;
-    if (ld_a == S::ROW_A && ld_b == S::ROW_B) return 1;
-    if (ld_a == S::LD_A && ld_b == S::LD_B) return 2;
-    return 0;
-}
+struct DenseRows : S { static constexpr int LD_A = S::ROW_A, LD_B = S::ROW_B; };     // a built shape with dense rows
 
-// shape id (0 hector, 1 hector_full, 2 XBot-L) and layout of the buffers described by p; layout 0 = not a built shape
-int stack_layout(const hb_env_params *p, int *shape) {
-    int l;
-    if ((l = shape_layout<ShapeHector>(p))) return *shape = 0, l;
-    if ((l = shape_layout<ShapeHectorFull>(p))) return *shape = 1, l;
-    if ((l = shape_layout<ShapeXBot>(p))) return *shape = 2, l;
-    return *shape = -1, 0;
-}
-
-int shift_any(const float *prev, float *next, const uint8_t *reset_buf, int num_envs, int row, int ld, int frame,
-              cudaStream_t st);
-
-template <int ROW, int FRAME>
-void launch_stack_fixed(const float *prev, float *next, int n, cudaStream_t st) {
-    const uint32_t total = (uint32_t)n * ROW;
-    const uint32_t vecs = (total + 3u) / 4u;
-    const uint32_t blocks = (vecs + 4 * 256 - 1) / (4 * 256);
-    stack_shift_fixed_kernel<ROW, FRAME, 4><<<blocks, 256, 0, st>>>(prev, next, total);
-}
+// blocks of stack_shift_fixed (256 threads, 4 float4 each) over `total` floats
+uint32_t shift_blocks(uint32_t total) { return ((total + 3u) / 4u + 4 * 256 - 1) / (4 * 256); }
 
 bool fits_u32(int n, int row) { return (long long)n * row + 64 * 1024 < (1ll << 32); }
 
@@ -1432,10 +1408,11 @@ int shift_any(const float *prev, float *next, const uint8_t *reset_buf, int num_
     HB_REQUIRE(prev && next && prev != next, "hb_stack_shift: null or aliasing buffers");
     HB_REQUIRE(num_envs > 0 && frame > 0 && row > frame && ld >= row, "hb_stack_shift: bad shape");
     const bool fast = !reset_buf && ld == row && hb::aligned16(prev) && hb::aligned16(next) && fits_u32(num_envs, row);
+    const uint32_t dense_total = (uint32_t)num_envs * row;
     if (fast && row == ROW_OBS && frame == OBS) {
-        launch_stack_fixed<ROW_OBS, OBS>(prev, next, num_envs, st);
+        stack_shift_fixed_kernel<ROW_OBS, OBS, 4><<<shift_blocks(dense_total), 256, 0, st>>>(prev, next, dense_total);
     } else if (fast && row == ROW_PRIV && frame == PRIV) {
-        launch_stack_fixed<ROW_PRIV, PRIV>(prev, next, num_envs, st);
+        stack_shift_fixed_kernel<ROW_PRIV, PRIV, 4><<<shift_blocks(dense_total), 256, 0, st>>>(prev, next, dense_total);
     } else {
         const long long total = (long long)num_envs * ld;
         stack_shift_scalar_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(prev, next, reset_buf, total, row, ld, frame);
@@ -1444,31 +1421,85 @@ int shift_any(const float *prev, float *next, const uint8_t *reset_buf, int num_
     return HB_OK;
 }
 
-template <typename T>
+template <typename T, bool kBulk>
 int launch_post_physics(const hb_env_params *p, const hb_env_buffers *buf, const hb_env_noise *noise, float *obs_new,
-                               float *priv_new, int32_t stages, bool bulk, cudaStream_t st) {
+                        float *priv_new, int32_t stages, cudaStream_t st) {
     const bool with_noise = p->add_noise && (noise->z_obs || noise->rng_counter);
     const TileLayout L = make_layout(p->num_bodies, with_noise, T::NDOF, T::OBS, T::PRIV);
     const size_t smem = (size_t)L.total * sizeof(float);
     const int tiles = (p->num_envs + TILE - 1) / TILE;
-    static bool attr_set[2] = {false, false};
-    if (bulk) {
-        if (!attr_set[1]) {
-            HB_CUDA(cudaFuncSetAttribute(post_physics_kernel<true, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024));
-            attr_set[1] = true;
-        }
-        HB_CUDA(hb::launch_pdl(hb::use_pdl_post(p->num_envs), post_physics_kernel<true, T>, dim3(tiles), dim3(4 * TILE), smem, st, *p, *buf,
-                               *noise, obs_new, priv_new, (int)stages));
-    } else {
-        if (!attr_set[0]) {
-            HB_CUDA(cudaFuncSetAttribute(post_physics_kernel<false, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024));
-            attr_set[0] = true;
-        }
-        HB_CUDA(hb::launch_pdl(hb::use_pdl_post(p->num_envs), post_physics_kernel<false, T>, dim3(tiles), dim3(4 * TILE), smem, st, *p, *buf,
-                               *noise, obs_new, priv_new, (int)stages));
+    static bool attr_set = false;
+    if (!attr_set) {
+        HB_CUDA(cudaFuncSetAttribute(post_physics_kernel<kBulk, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024));
+        attr_set = true;
     }
+    HB_CUDA(hb::launch_pdl(hb::use_pdl_post(p->num_envs), post_physics_kernel<kBulk, T>, dim3(tiles), dim3(4 * TILE), smem, st, *p, *buf,
+                           *noise, obs_new, priv_new, (int)stages));
     HB_CHECK_LAUNCH("post_physics_kernel");
     return HB_OK;
+}
+
+// The frame-stack shift of both histories: rows and pitches, built shape (0 hector, 1 hector_full, 2 XBot-L) and layout
+// (0 = not a built shape, 1 = dense rows, 2 = 128-byte pitch), and whether the fixed-shape kernels apply, with their grid
+struct StackPlan {
+    int row_a, row_b, ld_a, ld_b, shape, layout;
+    bool fast;
+    uint32_t total_a, total_b, blocks_a, blocks_b;
+};
+
+template <typename S>
+int shape_layout(const StackPlan &s, const hb_env_params *p) {
+    if (s.row_a != S::ROW_A || p->num_single_obs != S::FRAME_A || s.row_b != S::ROW_B || p->num_single_priv != S::FRAME_B) return 0;
+    return s.ld_a == S::ROW_A && s.ld_b == S::ROW_B ? 1 : (s.ld_a == S::LD_A && s.ld_b == S::LD_B ? 2 : 0);
+}
+
+StackPlan stack_plan(const hb_env_params *p, const float *obs_prev, const float *priv_prev, const float *obs_new,
+                     const float *priv_new) {
+    StackPlan s;
+    s.row_a = p->frame_stack * p->num_single_obs, s.row_b = p->c_frame_stack * p->num_single_priv;
+    s.ld_a = p->obs_ld ? p->obs_ld : s.row_a, s.ld_b = p->priv_ld ? p->priv_ld : s.row_b;
+    const int layouts[3] = {shape_layout<ShapeHector>(s, p), shape_layout<ShapeHectorFull>(s, p), shape_layout<ShapeXBot>(s, p)};
+    s.shape = layouts[0] ? 0 : (layouts[1] ? 1 : 2);
+    s.layout = layouts[s.shape];
+    s.fast = hb::aligned16(obs_prev) && hb::aligned16(obs_new) && hb::aligned16(priv_prev) && hb::aligned16(priv_new) &&
+             s.layout != 0 && fits_u32(p->num_envs, s.ld_a > s.ld_b ? s.ld_a : s.ld_b);
+    s.total_a = (uint32_t)p->num_envs * s.ld_a, s.total_b = (uint32_t)p->num_envs * s.ld_b;
+    s.blocks_a = shift_blocks(s.total_a), s.blocks_b = shift_blocks(s.total_b);
+    return s;
+}
+
+// The fixed-shape kernel of a fast plan: instantiate(R{}) with R = the StackShape (pitched rows) or its DenseRows, whose
+// ROW / LD / FRAME constants are the kernel's template arguments
+template <typename F>
+auto stack_kernel(const StackPlan &s, F &&instantiate) {
+    auto rows = [&](auto shape) {
+        using S = decltype(shape);
+        return s.layout == 2 ? instantiate(S{}) : instantiate(DenseRows<S>{});
+    };
+    return s.shape == 0 ? rows(ShapeHector{}) : (s.shape == 1 ? rows(ShapeHectorFull{}) : rows(ShapeXBot{}));
+}
+
+// Grid of the shard-wide reset finalisation: each CTA owns a contiguous segment of at least 8 32-env tiles
+struct FinalizeGrid { int tiles, seg, blocks; };
+
+FinalizeGrid finalize_grid(int num_envs) {
+    const int tiles = (num_envs + TILE - 1) / TILE;
+    int seg = (tiles + hb::sm_count() - 1) / hb::sm_count();
+    if (seg < 8) seg = 8;
+    return {tiles, seg, (tiles + seg - 1) / seg};
+}
+
+PdConsts pd_consts(const hb_env_params *p) {
+    PdConsts c;
+    for (int j = 0; j < HB_MAX_DOF; ++j) c.q0[j] = p->default_dof_pos[j], c.lim[j] = p->torque_limits[j];
+    return c;
+}
+
+// two DOFs per thread: an even joint count, 16-byte (pos, vel) pairs and 8-byte aligned per-DOF buffers
+bool pd_vectorizable(const hb_env_params *p, const hb_env_buffers *buf) {
+    return (p->num_dof % 2 == 0) && hb::aligned16(buf->dof_state) &&
+           ((reinterpret_cast<uintptr_t>(buf->actions) | reinterpret_cast<uintptr_t>(buf->p_gains) |
+             reinterpret_cast<uintptr_t>(buf->d_gains) | reinterpret_cast<uintptr_t>(buf->torques)) & 7u) == 0;
 }
 
 }  // namespace
@@ -1552,22 +1583,17 @@ int hb_env_prologue_torques(const hb_env_params *p, const hb_env_buffers *buf, c
     if (int rc = check_params(p, buf, "hb_env_prologue_torques")) return rc;
     HB_REQUIRE(actions_in && buf->actions && buf->dof_state && buf->p_gains && buf->d_gains && buf->torques,
                "hb_env_prologue_torques: null buffer");
-    const bool vec = (p->num_dof % 2 == 0) && hb::aligned16(buf->dof_state) &&
-                     ((reinterpret_cast<uintptr_t>(buf->actions) | reinterpret_cast<uintptr_t>(buf->p_gains) |
-                       reinterpret_cast<uintptr_t>(buf->d_gains) | reinterpret_cast<uintptr_t>(buf->torques)) & 7u) == 0;
-    if (!vec) {        // unaligned buffers / odd joint count: the two separate launches
+    if (!pd_vectorizable(p, buf)) {        // unaligned buffers / odd joint count: the two separate launches
         if (int rc = hb_env_action_prologue(p, buf, actions_in, noise, stream)) return rc;
         return hb_env_compute_torques(p, buf, stream);
     }
-    PdConsts c;
-    for (int j = 0; j < HB_MAX_DOF; ++j) c.q0[j] = p->default_dof_pos[j], c.lim[j] = p->torque_limits[j];
     const int pairs = p->num_envs * p->num_dof / 2;
     hb_env_noise none = {};
     prologue_pd_kernel<<<(pairs + 255) / 256, 256, 0, (cudaStream_t)stream>>>(
         actions_in, buf->actions, noise ? *noise : none, p->clip_actions, p->action_delay, p->action_noise,
         reinterpret_cast<const float4 *>(buf->dof_state), reinterpret_cast<const float2 *>(buf->p_gains),
         reinterpret_cast<const float2 *>(buf->d_gains), reinterpret_cast<float2 *>(buf->torques), pairs, p->num_dof,
-        p->action_scale, c);
+        p->action_scale, pd_consts(p));
     HB_CHECK_LAUNCH("prologue_pd_kernel");
     return HB_OK;
 }
@@ -1576,13 +1602,9 @@ int hb_env_compute_torques(const hb_env_params *p, const hb_env_buffers *buf, vo
     if (int rc = check_params(p, buf, "hb_env_compute_torques")) return rc;
     HB_REQUIRE(buf->dof_state && buf->actions && buf->p_gains && buf->d_gains && buf->torques,
                "hb_env_compute_torques: null buffer");
-    PdConsts c;
-    for (int j = 0; j < HB_MAX_DOF; ++j) c.q0[j] = p->default_dof_pos[j], c.lim[j] = p->torque_limits[j];
+    const PdConsts c = pd_consts(p);
     const int total = p->num_envs * p->num_dof;
-    const bool vec = (p->num_dof % 2 == 0) && hb::aligned16(buf->dof_state) &&
-                     ((reinterpret_cast<uintptr_t>(buf->actions) | reinterpret_cast<uintptr_t>(buf->p_gains) |
-                       reinterpret_cast<uintptr_t>(buf->d_gains) | reinterpret_cast<uintptr_t>(buf->torques)) & 7u) == 0;
-    if (vec) {
+    if (pd_vectorizable(p, buf)) {
         const int pairs = total / 2;
         HB_CUDA(hb::launch_pdl(hb::use_pdl_small_kernel(p->num_envs), pd_torque_kernel, dim3((pairs + 255) / 256), dim3(256), 0, (cudaStream_t)stream,
                                reinterpret_cast<const float4 *>(buf->dof_state), reinterpret_cast<const float2 *>(buf->actions),
@@ -1637,13 +1659,14 @@ int hb_env_post_physics(const hb_env_params *p, const hb_env_buffers *buf, const
     // a config that scales none of the optional terms runs the kernel compiled without them
     const bool opt = p->reward_scale[HB_R_JOINT_POS] != 0.0f || p->reward_scale[HB_R_VEL_MISMATCH_EXP] != 0.0f ||
                      p->reward_scale[HB_R_TRACK_VEL_HARD] != 0.0f || p->reward_scale[HB_R_LOW_SPEED] != 0.0f;
-    if (matches(10, HB_TASK_HECTOR, Hector::OBS, Hector::PRIV))
-        return opt ? launch_post_physics<Hector>(p, buf, noise, obs_new, priv_new, stages, bulk, st)
-                   : launch_post_physics<HectorSlim>(p, buf, noise, obs_new, priv_new, stages, bulk, st);
-    if (matches(18, HB_TASK_HECTOR, HectorFull::OBS, HectorFull::PRIV))
-        return opt ? launch_post_physics<HectorFull>(p, buf, noise, obs_new, priv_new, stages, bulk, st)
-                   : launch_post_physics<HectorFullSlim>(p, buf, noise, obs_new, priv_new, stages, bulk, st);
-    if (matches(12, HB_TASK_XBOT, XBot::OBS, XBot::PRIV)) return launch_post_physics<XBot>(p, buf, noise, obs_new, priv_new, stages, bulk, st);
+    auto launch = [&](auto task) {
+        using T = decltype(task);
+        return bulk ? launch_post_physics<T, true>(p, buf, noise, obs_new, priv_new, stages, st)
+                    : launch_post_physics<T, false>(p, buf, noise, obs_new, priv_new, stages, st);
+    };
+    if (matches(10, HB_TASK_HECTOR, Hector::OBS, Hector::PRIV)) return opt ? launch(Hector{}) : launch(HectorSlim{});
+    if (matches(18, HB_TASK_HECTOR, HectorFull::OBS, HectorFull::PRIV)) return opt ? launch(HectorFull{}) : launch(HectorFullSlim{});
+    if (matches(12, HB_TASK_XBOT, XBot::OBS, XBot::PRIV)) return launch(XBot{});
     hb::set_error("hb_env_post_physics: no kernel for num_dof=%d task_kind=%d frames %d/%d (built: hector 10/41/70, hector_full "
                   "18/65/94, XBot-L 12/47/73)", p->num_dof, p->task_kind, p->num_single_obs, p->num_single_priv);
     return HB_ERR_UNSUPPORTED;
@@ -1673,29 +1696,19 @@ int hb_env_stack_observations(const hb_env_params *p, const hb_env_buffers *buf,
     HB_REQUIRE(obs_prev && priv_prev && obs_new && priv_new, "hb_env_stack_observations: null buffer");
     HB_REQUIRE(obs_prev != obs_new && priv_prev != priv_new, "hb_env_stack_observations: prev and new must not alias");
     cudaStream_t st = (cudaStream_t)stream;
-    const int row_a = p->frame_stack * p->num_single_obs, row_b = p->c_frame_stack * p->num_single_priv;
-    const int ld_a = p->obs_ld ? p->obs_ld : row_a, ld_b = p->priv_ld ? p->priv_ld : row_b;
-    int shape = -1;
-    const int layout = stack_layout(p, &shape);
-    const bool fast = hb::aligned16(obs_prev) && hb::aligned16(obs_new) && hb::aligned16(priv_prev) &&
-                      hb::aligned16(priv_new) && layout != 0 && fits_u32(p->num_envs, ld_a > ld_b ? ld_a : ld_b);
-    if (fast) {
-        const uint32_t total_a = (uint32_t)p->num_envs * ld_a, total_b = (uint32_t)p->num_envs * ld_b;
-        constexpr uint32_t PER = 4 * 256;
-        const uint32_t blocks_a = ((total_a + 3u) / 4u + PER - 1) / PER, blocks_b = ((total_b + 3u) / 4u + PER - 1) / PER;
-        using PairKernel = void (*)(const float *, float *, uint32_t, uint32_t, const float *, float *, uint32_t);
-#define HB_PAIR(S, PITCH) (PITCH ? (PairKernel)stack_shift_pair_kernel<S::ROW_A, S::LD_A, S::FRAME_A, S::ROW_B, S::LD_B, S::FRAME_B, 4> \
-                                 : (PairKernel)stack_shift_pair_kernel<S::ROW_A, S::ROW_A, S::FRAME_A, S::ROW_B, S::ROW_B, S::FRAME_B, 4>)
-        const bool pitch = layout == 2;
-        PairKernel kernel = shape == 0 ? HB_PAIR(ShapeHector, pitch) : (shape == 1 ? HB_PAIR(ShapeHectorFull, pitch) : HB_PAIR(ShapeXBot, pitch));
-#undef HB_PAIR
-        HB_CUDA(hb::launch_pdl(hb::use_pdl(p->num_envs), kernel, dim3(blocks_a + blocks_b), dim3(256), 0,
-                               st, obs_prev, obs_new, total_a, blocks_a, priv_prev, priv_new, total_b));
+    const StackPlan s = stack_plan(p, obs_prev, priv_prev, obs_new, priv_new);
+    if (s.fast) {
+        auto kernel = stack_kernel(s, [](auto rows) {
+            using R = decltype(rows);
+            return stack_shift_pair_kernel<R::ROW_A, R::LD_A, R::FRAME_A, R::ROW_B, R::LD_B, R::FRAME_B, 4>;
+        });
+        HB_CUDA(hb::launch_pdl(hb::use_pdl(p->num_envs), kernel, dim3(s.blocks_a + s.blocks_b), dim3(256), 0, st, obs_prev, obs_new,
+                               s.total_a, s.blocks_a, priv_prev, priv_new, s.total_b));
         HB_CHECK_LAUNCH("stack_shift_pair_kernel");
         return HB_OK;
     }
-    if (int rc = shift_any(obs_prev, obs_new, nullptr, p->num_envs, row_a, ld_a, p->num_single_obs, st)) return rc;
-    return shift_any(priv_prev, priv_new, nullptr, p->num_envs, row_b, ld_b, p->num_single_priv, st);
+    if (int rc = shift_any(obs_prev, obs_new, nullptr, p->num_envs, s.row_a, s.ld_a, p->num_single_obs, st)) return rc;
+    return shift_any(priv_prev, priv_new, nullptr, p->num_envs, s.row_b, s.ld_b, p->num_single_priv, st);
 }
 
 int hb_env_stack_finalize(const hb_env_params *p, const hb_env_buffers *buf, const float *obs_prev, const float *priv_prev,
@@ -1705,34 +1718,19 @@ int hb_env_stack_finalize(const hb_env_params *p, const hb_env_buffers *buf, con
     HB_REQUIRE(obs_prev != obs_new && priv_prev != priv_new, "hb_env_stack_finalize: prev and new must not alias");
     HB_REQUIRE(buf->scratch_ballots && buf->scratch_sums && buf->reset_env_ids && buf->reset_count && buf->episode_means,
                "hb_env_stack_finalize: null scratch/result buffers");
-    const int row_b = p->c_frame_stack * p->num_single_priv;
-    const int ld_a = p->obs_ld ? p->obs_ld : p->frame_stack * p->num_single_obs, ld_b = p->priv_ld ? p->priv_ld : row_b;
-    int shape = -1;
-    const int layout = stack_layout(p, &shape);
-    const bool fast = hb::aligned16(obs_prev) && hb::aligned16(obs_new) && hb::aligned16(priv_prev) &&
-                      hb::aligned16(priv_new) && layout != 0 && fits_u32(p->num_envs, ld_a > ld_b ? ld_a : ld_b);
-    if (!fast) {        // other layouts: the two separate launches
+    const StackPlan s = stack_plan(p, obs_prev, priv_prev, obs_new, priv_new);
+    if (!s.fast) {        // other layouts: the two separate launches
         if (int rc = hb_env_stack_observations(p, buf, obs_prev, priv_prev, obs_new, priv_new, stream)) return rc;
         return hb_env_reset_finalize(p, buf, obs_new, priv_new, host_count, rng_counter, stream);
     }
-    constexpr uint32_t PER = 4 * 256;
-    const uint32_t total_a = (uint32_t)p->num_envs * ld_a, total_b = (uint32_t)p->num_envs * ld_b;
-    const uint32_t blocks_a = ((total_a + 3u) / 4u + PER - 1) / PER, blocks_b = ((total_b + 3u) / 4u + PER - 1) / PER;
-    const int tiles = (p->num_envs + TILE - 1) / TILE;
-    int seg = (tiles + hb::sm_count() - 1) / hb::sm_count();
-    if (seg < 8) seg = 8;
-    const uint32_t fin_blocks = (uint32_t)((tiles + seg - 1) / seg);
-    using FinKernel = void (*)(const float *, float *, uint32_t, uint32_t, const float *, float *, uint32_t, uint32_t, hb_env_params,
-                               hb_env_buffers, int, int, int32_t *, unsigned long long *);
-#define HB_FIN(S, PITCH) (PITCH ? (FinKernel)stack_finalize_kernel<S::ROW_A, S::LD_A, S::FRAME_A, S::ROW_B, S::LD_B, S::FRAME_B, 4> \
-                                : (FinKernel)stack_finalize_kernel<S::ROW_A, S::ROW_A, S::FRAME_A, S::ROW_B, S::ROW_B, S::FRAME_B, 4>)
-    const bool pitch = layout == 2;
-    FinKernel kernel = shape == 0 ? HB_FIN(ShapeHector, pitch) : (shape == 1 ? HB_FIN(ShapeHectorFull, pitch) : HB_FIN(ShapeXBot, pitch));
-#undef HB_FIN
-    HB_CUDA(hb::launch_pdl(hb::use_pdl_stack(p->num_envs), kernel,
-                           dim3(blocks_a + blocks_b + fin_blocks), dim3(256), 0, (cudaStream_t)stream, obs_prev, obs_new, total_a,
-                           blocks_a, priv_prev, priv_new, total_b, blocks_b, *p, *buf, tiles, seg, host_count,
-                           reinterpret_cast<unsigned long long *>(rng_counter)));
+    const FinalizeGrid g = finalize_grid(p->num_envs);
+    auto kernel = stack_kernel(s, [](auto rows) {
+        using R = decltype(rows);
+        return stack_finalize_kernel<R::ROW_A, R::LD_A, R::FRAME_A, R::ROW_B, R::LD_B, R::FRAME_B, 4>;
+    });
+    HB_CUDA(hb::launch_pdl(hb::use_pdl_stack(p->num_envs), kernel, dim3(s.blocks_a + s.blocks_b + (uint32_t)g.blocks), dim3(256), 0,
+                           (cudaStream_t)stream, obs_prev, obs_new, s.total_a, s.blocks_a, priv_prev, priv_new, s.total_b, s.blocks_b,
+                           *p, *buf, g.tiles, g.seg, host_count, reinterpret_cast<unsigned long long *>(rng_counter)));
     HB_CHECK_LAUNCH("stack_finalize_kernel");
     return HB_OK;
 }
@@ -1786,12 +1784,9 @@ int hb_env_reset_finalize(const hb_env_params *p, const hb_env_buffers *buf, flo
                "hb_env_reset_finalize: null scratch/result buffers");
     HB_REQUIRE((obs_new == nullptr) == (priv_new == nullptr), "hb_env_reset_finalize: pass both frame stacks or neither");
     HB_REQUIRE(!buf->time_outs_latched || buf->time_out_buf, "hb_env_reset_finalize: latch without time_out_buf");
-    const int tiles = (p->num_envs + TILE - 1) / TILE;
-    int seg = (tiles + hb::sm_count() - 1) / hb::sm_count();
-    if (seg < 8) seg = 8;
-    const int grid = (tiles + seg - 1) / seg;
-    HB_CUDA(hb::launch_pdl(hb::use_pdl(p->num_envs), reset_finalize_kernel, dim3(grid), dim3(FIN_THREADS), 0, (cudaStream_t)stream, *p, *buf, obs_new,
-                           priv_new, tiles, seg, host_count, reinterpret_cast<unsigned long long *>(rng_counter)));
+    const FinalizeGrid g = finalize_grid(p->num_envs);
+    HB_CUDA(hb::launch_pdl(hb::use_pdl(p->num_envs), reset_finalize_kernel, dim3(g.blocks), dim3(FIN_THREADS), 0, (cudaStream_t)stream, *p, *buf,
+                           obs_new, priv_new, g.tiles, g.seg, host_count, reinterpret_cast<unsigned long long *>(rng_counter)));
     HB_CHECK_LAUNCH("reset_finalize_kernel");
     return HB_OK;
 }

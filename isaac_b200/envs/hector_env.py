@@ -32,7 +32,7 @@ right before the next `physics.simulate()`.
 from __future__ import annotations
 
 import ctypes as C
-from typing import Dict, Optional
+from typing import Dict, NamedTuple, Optional
 
 import numpy as np
 import torch
@@ -45,6 +45,17 @@ from .hector_config import class_to_dict
 from .tasks import layout_for
 
 _EXTRAS_RING = 256       # >= num_steps_per_env: episode-mean slots handed out through extras["episode"]
+
+
+class _BufferPair(NamedTuple):
+    """Observation and privileged-observation buffers of one step; `key` = their addresses, which key the step graphs."""
+    obs: torch.Tensor
+    priv: torch.Tensor
+    key: tuple
+
+    @classmethod
+    def of(cls, obs, priv):
+        return cls(obs, priv, (obs.data_ptr(), priv.data_ptr()))
 
 
 def _find(names, patterns):
@@ -251,9 +262,8 @@ class HectorFreeEnvB200:
         # after next (PPO.act keeps references until process_env_step, ppo.py:99-100,111).  Rows sit at a
         # 128-byte pitch (640 / 1056 floats); a caller may hand the env the buffers of the NEXT step
         # (set_next_observation_buffers: the rollout storage's slots), else it alternates between its own two.
-        # Each buffer pair travels as (obs, priv, (obs address, priv address)): the addresses key the step graphs.
-        self._own = [self._buffer_pair(z(N, self._p.obs_ld)[:, :self.num_obs],
-                                       z(N, self._p.priv_ld)[:, :self.num_privileged_obs]) for _ in range(2)]
+        self._own = [_BufferPair.of(z(N, self._p.obs_ld)[:, :self.num_obs],
+                                    z(N, self._p.priv_ld)[:, :self.num_privileged_obs]) for _ in range(2)]
         self._cur_buf = self._own[0]
         self._next_out = None
         # reset compaction + extras
@@ -289,11 +299,12 @@ class HectorFreeEnvB200:
         self.seed(int(getattr(cfg, "seed", 1)))
         self._b = EnvBuffers()
         self._nz = EnvNoise()
+        self._draws_bound = False           # a launch sequence is open: _nz holds its draws (_in_sequence)
         self._bind_buffers()
         self.init_done = True
         # HectorFreeEnv.__init__ tail (hector_env.py:48-51): reset_idx(all) + compute_observations,
         # preceded by the derived quantities of _init_buffers (legged_robot.py:452,477-479)
-        self._launch_post(HB_STAGE_DERIVE | HB_STAGE_RESET_ALL | HB_STAGE_OBS)
+        self._in_sequence(self._launch_post, HB_STAGE_DERIVE | HB_STAGE_RESET_ALL | HB_STAGE_OBS)
         self._apply_pending_resets()
 
     # ------------------------------------------------------------------ plumbing
@@ -333,39 +344,50 @@ class HectorFreeEnvB200:
             if (t.device != self.device or t.dtype != torch.float32 or tuple(t.shape) != (self.num_envs, width)
                     or t.stride() != (ld, 1) or t.data_ptr() % 16):
                 raise ValueError(f"observation buffer must be a [{self.num_envs}, {width}] fp32 view with row pitch {ld} on {self.device}")
-        pair = self._buffer_pair(obs, privileged_obs)
-        if pair[2][0] == self._cur_buf[2][0] or pair[2][1] == self._cur_buf[2][1]:
+        pair = _BufferPair.of(obs, privileged_obs)
+        if pair.key[0] == self._cur_buf.key[0] or pair.key[1] == self._cur_buf.key[1]:
             raise ValueError("the next observation buffers must not alias the current ones")
         self._next_out = pair
-
-    @staticmethod
-    def _buffer_pair(obs, priv):
-        return (obs, priv, (obs.data_ptr(), priv.data_ptr()))
 
     def _take_output(self):
         """Where this step's observations go: the caller's buffers if it supplied any, else the own pair not in use."""
         out, cur = self._next_out, self._cur_buf
         if out is not None:
             self._next_out = None
-            if out[2][0] != cur[2][0] and out[2][1] != cur[2][1]:
+            if out.key[0] != cur.key[0] and out.key[1] != cur.key[1]:
                 return out
         return self._own[1] if cur is self._own[0] else self._own[0]
 
     def inject_noise(self, frame) -> None:
-        """Use the supplied draws (isaac_b200.synthetic.NoiseFrame on this device) for the next step
-        instead of the env's own generator — "noise injected as a supplied tensor"."""
+        """Use the supplied draws (isaac_b200.synthetic.NoiseFrame on this device) instead of the env's own generator for
+        the next launch sequence - the next step(), or a hook or reset_idx() called on its own - "noise injected as a
+        supplied tensor"."""
         self._injected = frame
 
+    def _in_sequence(self, launch, *args):
+        """Run launch(*args) inside a launch sequence: an eager step(), the constructor's reset, or a hook, reset_idx() or
+        post_physics_step() called on its own.  The outermost call binds the sequence's draws once (_draw_noise) and
+        releases them when it returns; the calls nested in it (the hooks of the staged step) use that binding.  Every
+        draw of a sequence is taken at one counter value: the frame-stack finalize launch (HB_STAGE_STEP / OBS) advances
+        the counter by one after them, and a reset-only finalize only when reset_idx() opened the sequence itself."""
+        if self._draws_bound:
+            return launch(*args)
+        self._draw_noise(False)
+        self._draws_bound = True
+        try:
+            return launch(*args)
+        finally:
+            self._draws_bound = False
+
     def _draw_noise(self, push: bool):
-        """Bind the draws of the next launch sequence: the injected tape if there is one, otherwise the device
-        generator (Philox; key and step counter in `self._rng_state`): the tensors the reference
-        draws with torch.rand / randn_like (hector_env.py:166,168,241; legged_robot.py:327-332,366,384) are never
-        materialised.  Every draw of one step uses the same counter; the step's last finalize launch advances it by one
-        (fused or staged hooks alike), and so does a reset_idx() called outside step().  The constructor's reset draws
-        at counter 0, step t of a freshly seeded env at counter t (oracle/device_rng.py mirrors the draws)."""
+        """Fill `_nz` with draws and leave it so, without opening a launch sequence (_in_sequence): the injected tape if
+        there is one (consumed here), otherwise the device generator (Philox; key and step counter in `self._rng_state`):
+        the tensors the reference draws with torch.rand / randn_like (hector_env.py:166,168,241;
+        legged_robot.py:327-332,366,384) are never materialised.  The constructor's reset draws at counter 0, step t of a
+        freshly seeded env at counter t (oracle/device_rng.py mirrors the draws).  `push` is unused, kept for callers."""
         nz = self._nz
         if self._injected is not None:
-            f = self._injected
+            f, self._injected = self._injected, None
             self._noise_keepalive = f
             nz.u_delay, nz.z_action = f.u_delay.data_ptr(), f.z_action.data_ptr()
             nz.u_cmd, nz.u_push, nz.u_reset, nz.z_obs = (f.u_cmd.data_ptr(), f.u_push.data_ptr(),
@@ -385,14 +407,11 @@ class HectorFreeEnvB200:
         self._rng_seed = int(seed) & 0xFFFFFFFFFFFFFFFF
         signed = self._rng_seed - (1 << 64) if self._rng_seed >= (1 << 63) else self._rng_seed
         self._rng_state.copy_(torch.tensor([0, signed], dtype=torch.int64), non_blocking=False)
-        if hasattr(self, "_nz"):
-            self._nz.u_reset = self._nz.rng_counter = None
 
     # ------------------------------------------------------------------ the hot path
     def step(self, actions: torch.Tensor):
         """hector_env.py:158-169 + legged_robot.py:84-108."""
-        lib, st = self._lib, self._stream()
-        self._st = st
+        self._st = self._stream()
         staged = actions.device != self.device or actions.dtype != torch.float32 or not actions.is_contiguous()
         if staged:
             actions = actions.to(self.device, dtype=torch.float32).contiguous()
@@ -400,7 +419,10 @@ class HectorFreeEnvB200:
         push = bool(self.cfg.domain_rand.push_robots) and (self.common_step_counter % self.push_interval == 0)
         if self._graphs is not None and not push and self._injected is None and not self._hooks_overridden():
             return self._step_graph(actions, staged)
-        self._draw_noise(push)
+        return self._in_sequence(self._step_eager, actions, push)
+
+    def _step_eager(self, actions, push):
+        lib, st = self._lib, self._st
         _lib.check(lib.hb_env_action_prologue(self._pp, self._pb, actions.data_ptr(), self._pn, st),
                    "hb_env_action_prologue")
         phys, torques, pd, pp, pb = self.physics, self.torques, lib.hb_env_compute_torques, self._pp, self._pb
@@ -464,7 +486,7 @@ class HectorFreeEnvB200:
         return g
 
     def _graph_b(self, prev, out):
-        key = (prev[2], out[2])
+        key = (prev.key, out.key)
         entry = self._graphs.get(key)
         if entry is None:
             if len(self._graphs) >= 256:      # buffers keep changing (new storage): drop the stale graphs
@@ -472,7 +494,7 @@ class HectorFreeEnvB200:
             def launches(st):
                 for _ in range(self.cfg.control.decimation - 1):
                     _lib.check(self._lib.hb_env_compute_torques(self._pp, self._pb, st), "hb_env_compute_torques")
-                self._launch_post_kernels(HB_STAGE_STEP, C.byref(self._g_nz), prev, out, True, st)
+                self._launch_post_kernels(HB_STAGE_STEP, self._g_nz, prev, out, True, st)
             gb = _lib.LaunchGraph(self.device).record(launches)
             entry = self._graphs[key] = (gb, prev, out)      # the graph keeps its buffers alive
         return entry[0]
@@ -483,20 +505,14 @@ class HectorFreeEnvB200:
         if staged:          # a converted temporary: its address is not worth a graph of its own
             self._g_actions.copy_(actions, non_blocking=True)
             actions = self._g_actions
-        slot = self._step_index % _EXTRAS_RING
         st = self._st
         self._graph_a(actions).replay(st)
         self._apply_pending_resets()          # gym.set_*_indexed of the previous step's resets
         out = self._take_output()
         self._graph_b(self._cur_buf, out).replay(st)
         self._cur_buf = out
-        self._pending_event = self._events[self._step_index & 1]
-        self._pending_event.record(torch.cuda.current_stream(self.device))
-        self.extras["episode"] = self._extras_episode[slot]
-        if self.cfg.env.send_timeouts:
-            self.extras["time_outs"] = self._time_outs_latched
-        self._step_index += 1
-        return out[0], out[1], self.rew_buf, self.reset_buf, self.extras
+        self._after_finalize()
+        return out.obs, out.priv, self.rew_buf, self.reset_buf, self.extras
 
     def _compute_torques(self, actions=None):
         """legged_robot.py:339-355 on self.actions (one decimation sub-step)."""
@@ -507,19 +523,19 @@ class HectorFreeEnvB200:
         """legged_robot.py:118-153 (termination, rewards, resets, observations, last_* copies): ONE fused launch plus the
         frame-stack / finalisation launch.  If a subclass overrides one of the reference's hooks (check_termination,
         compute_reward, reset_idx, compute_observations), the step instead calls the hooks one after the other in the
-        reference's order, each a launch of the same kernel restricted to that span - same results and the same
-        device-generator draws (the reset inside the staged step draws at the step's counter and does not advance it)."""
+        reference's order, each a launch of the same kernel restricted to that span - same results and the same draws,
+        all taken in one launch sequence (_in_sequence): the reset inside it does not advance the counter, the frame-stack
+        launch of compute_observations does."""
         self.physics.refresh_post_physics()
         if not self._hooks_overridden():
-            self._launch_post(HB_STAGE_STEP | (HB_STAGE_PUSH if push else 0))
+            self._in_sequence(self._launch_post, HB_STAGE_STEP | (HB_STAGE_PUSH if push else 0))
         else:
-            self._post_physics_step_staged(push)
+            self._in_sequence(self._post_physics_step_staged, push)
         if push:
             self.physics.set_root_state()
 
     # ------------------------------------------------------------------ the reference's hooks, one by one
     _HOOKS = ("check_termination", "compute_reward", "reset_idx", "compute_observations")
-    _hold_rng_counter = False       # set while the staged step runs reset_idx: its finalize launch leaves the counter alone
 
     def _hooks_overridden(self) -> bool:
         cls = type(self)
@@ -532,85 +548,71 @@ class HectorFreeEnvB200:
     def _launch_stage(self, stages: int) -> None:
         """One launch of the post-physics kernel restricted to `stages` (PREPARE / TERMINATION / REWARD / LAST bits): it
         resets nothing, so no finalisation launch follows and the extras ring does not advance."""
-        if self._nz.u_reset is None and self._nz.rng_counter is None:
-            self._draw_noise(False)
-        out = self._cur_buf          # not written: no HB_STAGE_OBS bit
-        _lib.check(self._lib.hb_env_post_physics(self._pp, self._pb, self._pn, out[0].data_ptr(), out[1].data_ptr(), stages,
-                                                 self._stream()), "hb_env_post_physics")
+        _lib.check(self._lib.hb_env_post_physics(self._pp, self._pb, self._pn, *self._cur_buf.key, stages, self._stream()),
+                   "hb_env_post_physics")        # the current buffers are not written: no HB_STAGE_OBS bit
 
     def _post_physics_step_staged(self, push: bool) -> None:
         """post_physics_step as the reference spells it (legged_robot.py:118-153), through the overridable hooks."""
-        keep = self._injected         # the step's tape (if any) serves every stage
         self._measure_heights(self._stream())
         self._launch_stage(HB_STAGE_PREPARE | (HB_STAGE_PUSH if push else 0))      # :127-137
         self.check_termination()                                                   # :139
         self.compute_reward()                                                      # :140
         env_ids = self.reset_buf.nonzero(as_tuple=False).flatten()                 # :142
-        self._injected = keep
-        self._hold_rng_counter = True       # reset_idx draws at this step's counter; compute_observations advances it
-        try:
-            self.reset_idx(env_ids)                                                # :143
-        finally:
-            self._hold_rng_counter = False
-        self._injected = keep
+        self.reset_idx(env_ids)                                                    # :143
         self.compute_observations()                                                # :144
-        self._injected = keep
         self._launch_stage(HB_STAGE_LAST)                                          # :146-150
-        self._injected = None
-        self._nz.u_reset = self._nz.rng_counter = None
 
     def check_termination(self):
         """legged_robot.py:155-160: reset_buf = contact on a termination body | time-out; time_out_buf."""
-        self._launch_stage(HB_STAGE_TERMINATION)
+        self._in_sequence(self._launch_stage, HB_STAGE_TERMINATION)
 
     def compute_reward(self):
         """legged_robot.py:216-234: rew_buf, episode_sums (alphabetical accumulation over the 18 active terms) and the
         stateful reward buffers (feet_air_time, last_contacts, feet_height, last_feet_z)."""
-        self._launch_stage(HB_STAGE_REWARD)
+        self._in_sequence(self._launch_stage, HB_STAGE_REWARD)
 
     def compute_observations(self):
         """hector_env.py:172-254: the newest obs / privileged frames from the current state, pushed onto the 15-frame
         histories (the frame-stack launch)."""
-        self._launch_post(HB_STAGE_OBS)
+        self._in_sequence(self._launch_post, HB_STAGE_OBS)
 
-    def _launch_post(self, stages: int):
-        lib, st = self._lib, self._stream()
-        if self._nz.u_reset is None and self._nz.rng_counter is None:
-            self._draw_noise(False)
+    def _launch_post(self, stages: int, advance: bool = True):
+        """The post-physics launch restricted to `stages` and its finalize launch, on the bound draws (`_nz`)."""
         emit = bool(stages & (HB_STAGE_STEP | HB_STAGE_OBS))
         prev = self._cur_buf
         out = self._take_output() if emit else self._own[1 if prev is self._own[0] else 0]
-        slot = self._step_index % _EXTRAS_RING          # = the ring cursor on the device: every finalize launch advances both
-        self._launch_post_kernels(stages, self._pn, prev, out, emit, st)
+        self._launch_post_kernels(stages, self._nz, prev, out, emit, self._stream(), advance)
         if emit:
             self._cur_buf = out
+        self._after_finalize()
+
+    def _launch_post_kernels(self, stages, nz, prev, out, emit, st, advance=True):
+        """post-physics -> frame-stack shift + reset finalisation, on one stream, with the draws of the EnvNoise `nz`;
+        prev / out = _BufferPair.  The finalize launch advances the generator counter unless `advance` is false."""
+        lib = self._lib
+        obs_new, priv_new = out.key
+        if stages & HB_STAGE_STEP:
+            self._measure_heights(st)        # _post_physics_step_callback, before anything is reset (legged_robot.py:315-316)
+        _lib.check(lib.hb_env_post_physics(self._pp, self._pb, C.byref(nz), obs_new, priv_new, stages, st),
+                   "hb_env_post_physics")
+        counter = nz.rng_counter if advance else None
+        if emit:        # shift + shard-wide reset results in one launch
+            _lib.check(lib.hb_env_stack_finalize(self._pp, self._pb, *prev.key, obs_new, priv_new, self._host_count.data_ptr(),
+                                                 counter, st), "hb_env_stack_finalize")
+        else:
+            _lib.check(lib.hb_env_reset_finalize(self._pp, self._pb, None, None, self._host_count.data_ptr(),
+                                                 counter, st), "hb_env_reset_finalize")
+
+    def _after_finalize(self):
+        """Host side of a finalize launch: the extras slot it filled (the device ring cursor advances with _step_index),
+        the event the reset count waits on, and time_outs."""
         if self._events:
             self._pending_event = self._events[self._step_index & 1]
             self._pending_event.record(torch.cuda.current_stream(self.device))
-        self.extras["episode"] = self._extras_episode[slot]
+        self.extras["episode"] = self._extras_episode[self._step_index % _EXTRAS_RING]
         if self.cfg.env.send_timeouts:
             self.extras["time_outs"] = self._time_outs_latched
         self._step_index += 1
-        self._injected = None
-        self._nz.u_reset = self._nz.rng_counter = None
-
-    def _launch_post_kernels(self, stages, noise_ref, prev, out, emit, st):
-        """post-physics -> frame-stack shift + reset finalisation, on one stream; prev / out = (obs, priv) tensors."""
-        lib = self._lib
-        obs_new, priv_new = out[0].data_ptr(), out[1].data_ptr()
-        if stages & HB_STAGE_STEP:
-            self._measure_heights(st)        # _post_physics_step_callback, before anything is reset (legged_robot.py:315-316)
-        _lib.check(lib.hb_env_post_physics(self._pp, self._pb, noise_ref, obs_new, priv_new, stages, st),
-                   "hb_env_post_physics")
-        noise = noise_ref._obj          # the EnvNoise behind the byref
-        if emit:        # shift + shard-wide reset results in one launch
-            _lib.check(lib.hb_env_stack_finalize(self._pp, self._pb, prev[0].data_ptr(), prev[1].data_ptr(),
-                                                 obs_new, priv_new, self._host_count.data_ptr(), noise.rng_counter, st),
-                       "hb_env_stack_finalize")
-        else:
-            counter = None if self._hold_rng_counter else noise.rng_counter
-            _lib.check(lib.hb_env_reset_finalize(self._pp, self._pb, None, None, self._host_count.data_ptr(),
-                                                 counter, st), "hb_env_reset_finalize")
 
     def _apply_pending_resets(self):
         """The two opaque calls of _reset_dofs/_reset_root_states (legged_robot.py:370-372,394-396) need
@@ -638,11 +640,11 @@ class HectorFreeEnvB200:
 
     @property
     def obs_buf(self):
-        return self._cur_buf[0]
+        return self._cur_buf.obs
 
     @property
     def privileged_obs_buf(self):
-        return self._cur_buf[1]
+        return self._cur_buf.priv
 
     def get_observations(self):
         return self.obs_buf
@@ -651,16 +653,16 @@ class HectorFreeEnvB200:
         return self.privileged_obs_buf
 
     def reset_idx(self, env_ids):
-        """legged_robot.py:162-214 + hector_env.py:256-261 for an explicit id list.  Called outside step(), it takes
-        its draws at the current counter and advances it; inside the staged step it leaves that to
-        compute_observations."""
+        """legged_robot.py:162-214 + hector_env.py:256-261 for an explicit id list.  Called on its own, it is a launch
+        sequence: it takes its draws at the current counter and advances it; inside the staged step it draws at the
+        step's counter and leaves the advance to compute_observations (_in_sequence)."""
         env_ids = torch.as_tensor(env_ids, device=self.device, dtype=torch.long)
         if env_ids.numel() == 0:
             return
         self.reset_buf.zero_()
         self.reset_buf[env_ids] = True
-        self._launch_post(HB_STAGE_RESET_MASK)
-        for hist in self._cur_buf[:2]:
+        self._in_sequence(self._launch_post, HB_STAGE_RESET_MASK, not self._draws_bound)
+        for hist in (self._cur_buf.obs, self._cur_buf.priv):
             hist[env_ids] = 0.0
         self._apply_pending_resets()
 
@@ -694,13 +696,17 @@ class HectorFreeEnvB200:
         """measured_heights = _get_heights() of the callback (legged_robot.py:315-316), when the config asks for it; a
         plain launch on `st`, so it also sits in the captured step graph."""
         if getattr(self.cfg.terrain, "measure_heights", False) and getattr(self, "height_samples", None) is not None:
-            t = self.cfg.terrain
-            _lib.check(self._lib.hb_env_get_heights(self.root_states.data_ptr(), self._height_points_xy.data_ptr(),
-                                                    self.num_height_points, self.height_samples.data_ptr(),
-                                                    self.height_samples.shape[0], self.height_samples.shape[1],
-                                                    float(t.border_size), float(t.horizontal_scale), float(t.vertical_scale),
-                                                    None, self.num_envs, self.measured_heights.data_ptr(), st),
-                       "hb_env_get_heights")
+            self._launch_get_heights(None, self.measured_heights, st)
+
+    def _launch_get_heights(self, ids, out, st) -> None:
+        """Heights under the grid of points into `out`: of every env, or of the int32 env ids `ids`."""
+        t = self.cfg.terrain
+        _lib.check(self._lib.hb_env_get_heights(self.root_states.data_ptr(), self._height_points_xy.data_ptr(),
+                                                self.num_height_points, self.height_samples.data_ptr(),
+                                                self.height_samples.shape[0], self.height_samples.shape[1],
+                                                float(t.border_size), float(t.horizontal_scale), float(t.vertical_scale),
+                                                None if ids is None else ids.data_ptr(), out.shape[0], out.data_ptr(), st),
+                   "hb_env_get_heights")
 
     def _get_heights(self, env_ids=None):
         """legged_robot.py:759-795: terrain height under the grid of points around each robot -> [N, P] (or [len(env_ids),
@@ -712,17 +718,9 @@ class HectorFreeEnvB200:
             raise NameError("Can't measure height with terrain mesh type 'none'")
         if getattr(self, "height_samples", None) is None:
             raise RuntimeError("no height field installed: call set_height_field(terrain.heightsamples ...) first")
-        ids, count = None, self.num_envs
-        if env_ids is not None:
-            ids = torch.as_tensor(env_ids, device=self.device, dtype=torch.int32).contiguous()
-            count = ids.numel()
-        out = self.measured_heights if ids is None else torch.empty(count, self.num_height_points, device=self.device)
-        _lib.check(self._lib.hb_env_get_heights(self.root_states.data_ptr(), self._height_points_xy.data_ptr(),
-                                                self.num_height_points, self.height_samples.data_ptr(),
-                                                self.height_samples.shape[0], self.height_samples.shape[1],
-                                                float(t.border_size), float(t.horizontal_scale), float(t.vertical_scale),
-                                                ids.data_ptr() if ids is not None else None, count, out.data_ptr(),
-                                                self._stream()), "hb_env_get_heights")
+        ids = None if env_ids is None else torch.as_tensor(env_ids, device=self.device, dtype=torch.int32).contiguous()
+        out = self.measured_heights if ids is None else torch.empty(ids.numel(), self.num_height_points, device=self.device)
+        self._launch_get_heights(ids, out, self._stream())
         return out
 
     @property

@@ -180,7 +180,8 @@ def test_env_step_device_draws_cross_the_counter_carry(lib, cuda_device):
 def test_staged_hooks_draw_like_the_fused_step(lib, cuda_device):
     """A subclass that overrides the four hooks (pass-through) runs the staged step; on the device generator it must take
     the same draws as the fused step - same results, same counter after every step, resets included - and a reset_idx()
-    outside step() still advances the counter by one."""
+    outside step() still advances the counter by one.  Of the other hooks called on their own, only compute_observations()
+    advances it, and the next step() still advances it by exactly one."""
     from isaac_b200.envs.hector_config import HectorCfg
     from isaac_b200.envs.hector_env import HectorFreeEnvB200
 
@@ -221,10 +222,19 @@ def test_staged_hooks_draw_like_the_fused_step(lib, cuda_device):
                                                          f"{int(staged._rng_state[0].item())}, fused {t + 1}")
         compare_records({k: np.stack(v) for k, v in got.items()}, {k: np.stack(v) for k, v in want.items()})
     assert np.stack(want["reset"]).sum() > steps
+    counter = lambda env: int(env._rng_state[0].item())
     for env, *_ in runs:
         before = int(env._rng_state[0].item())
         env.reset_idx(torch.tensor([0, 5, n - 1]))
         assert int(env._rng_state[0].item()) == before + 1, "reset_idx() outside step() advances the counter"
+        before = counter(env)
+        env.check_termination()
+        env.compute_reward()
+        assert counter(env) == before, "check_termination() / compute_reward() on their own leave the counter alone"
+        env.compute_observations()
+        assert counter(env) == before + 1, "compute_observations() on its own advances the counter by one"
+        env.step(tape.noise[steps - 1].actions.to(dev))
+        assert counter(env) == before + 2, "a step() after the hooks on their own advances the counter by one"
 
 
 # --------------------------------------------------------------------------- (d) PPO.act on the library's draws
