@@ -96,6 +96,8 @@ class ActorCritic:
                 L = _Layer(net, 2 * i, dims[i], dims[i + 1], i == 3, off)
                 self.layers.append(L)
                 off += L.numel
+        self.net_layers = {net: tuple(L for L in self.layers if L.net == net) for net in ("actor", "critic")}
+        self.output_layers = (self.net_layers["actor"][-1], self.net_layers["critic"][-1])
         self._std_offset = off
         off += (num_actions + 15) // 16 * 16
         self.flat = torch.zeros(off, device=self.device)
@@ -116,8 +118,9 @@ class ActorCritic:
         # "tf32": operands truncated to TF32 by the tensor core (fast path).  "3xtf32": hi/lo split operands, three
         # partial products in one fp32 accumulator - fp32-grade results like the reference's nn.Linear (parity mode)
         self.precision = precision
-        self.grouped = True          # the actor's and the critic's GEMM of a layer share one launch (hb_gemm_tf32_grouped)
-        self._scratch = {"actor": [None, self.device], "critic": [None, self.device]}     # one per stream / network
+        # 3xTF32 workspaces, one per network: a grouped launch takes both networks' at once, so growing a shared buffer for
+        # the second descriptor would free the first one's
+        self._scratch = {"actor": [None, self.device], "critic": [None, self.device]}
 
     def rebind(self, flat: torch.Tensor, grad_wire: torch.Tensor) -> None:
         """Move the flat parameter / gradient buffers to caller-provided storage of the same size (symmetric memory for
@@ -135,20 +138,20 @@ class ActorCritic:
     def std(self):
         return self.flat[self._std_offset:self._std_offset + self.num_actions]
 
-    def named_parameters(self):
-        """Views in the order of the reference module's `parameters()` (std first, then actor, critic)."""
-        yield "std", self.std
+    def named_views(self, buf):
+        """Named views of any buffer with the flat layout (parameters, gradients, Adam moments), in the order of the
+        reference module's `parameters()` (std first, then actor, critic)."""
+        yield "std", buf[self._std_offset:self._std_offset + self.num_actions]
         for L in self.layers:
-            P = self._matrix(self.flat, L)
+            P = self._matrix(buf, L)
             yield f"{L.net}.{L.index}.weight", P[:L.fan_out, :L.fan_in]
             yield f"{L.net}.{L.index}.bias", P[:L.fan_out, L.fan_in]
 
+    def named_parameters(self):
+        return self.named_views(self.flat)
+
     def named_gradients(self):
-        yield "std", self.grad[self._std_offset:self._std_offset + self.num_actions]
-        for L in self.layers:
-            G = self._matrix(self.grad, L)
-            yield f"{L.net}.{L.index}.weight", G[:L.fan_out, :L.fan_in]
-            yield f"{L.net}.{L.index}.bias", G[:L.fan_out, L.fan_in]
+        return self.named_views(self.grad)
 
     def parameters(self):
         return [p for _, p in self.named_parameters()]
@@ -189,8 +192,7 @@ class ActorCritic:
         if ws is None:
             z = lambda r, c: torch.zeros(r, c, device=self.device)
             ws = {"m": m}
-            for net in ("actor", "critic"):
-                Ls = [L for L in self.layers if L.net == net]
+            for net, Ls in self.net_layers.items():
                 hs = []
                 for L in Ls[:-1]:
                     h = z(m, pitch(L.fan_out + 1))
@@ -204,108 +206,87 @@ class ActorCritic:
     def _scratch_for(self, net: str):
         return self._scratch[net] if self.precision == "3xtf32" else None
 
-    # ------------------------------------------------------------------ forward
+    # ------------------------------------------------------------------ GEMM descriptors
     @property
     def fused_head(self) -> bool:
         """Both last hidden layers are 128 wide (and at most 15 actions): the update path evaluates the output layers inside
         the loss kernel (hb_ppo_head_fused) instead of as 128-row tensor-core tiles with 10 / 1 useful columns."""
-        return all(L.fan_in == 128 for L in self.layers if L.last) and self.num_actions <= 15
+        return all(L.fan_in == 128 for L in self.output_layers) and self.num_actions <= 15
 
-    def _mlp_forward(self, net: str, x: torch.Tensor, ws: dict, hidden_only: bool = False):
-        """x: [m, ld] with ld % 4 == 0 (only the first fan_in columns are read).  Returns out [m,16]
-        (or, with hidden_only, the last hidden activations [m, pitch(width + 1)])."""
-        lib, st = self._lib, torch.cuda.current_stream(self.device).cuda_stream
-        Ls = [L for L in self.layers if L.net == net]
-        a, lda = x, x.stride(0)
-        m = x.shape[0]
-        for i, L in enumerate(Ls):
-            if L.last and hidden_only:
-                return ws[net]["h"][-1]
-            P = self._matrix(self.flat, L)
-            d = ws[net]["out"] if L.last else ws[net]["h"][i]
-            gemm(lib, st, self._scratch_for(net), A=a.data_ptr(), B=P.data_ptr(), D=d.data_ptr(), M=m, N=L.rows if L.last else L.fan_out,
-                 K=L.fan_in, lda=lda, ldb=L.ld, ldd=d.stride(0), epilogue=HB_EPI_BIAS if L.last else HB_EPI_BIAS_ELU,
-                 bias=P.data_ptr() + L.fan_in * 4, bias_stride=L.ld)
-            a, lda = d, d.stride(0)
-        return ws[net]["out"]
-
-    # ------------------------------------------------------------------ both networks, layer by layer, grouped launches
-    def _fwd_kw(self, net, i, a, lda, m, ws):
-        L = [L for L in self.layers if L.net == net][i]
+    def _fwd_desc(self, net: str, i: int, a: torch.Tensor, ws: dict):
+        """Forward GEMM of layer i of `net` on a [m, ld] (ld % 4 == 0, only the first fan_in columns are read), bias and (hidden
+        layers) ELU in the epilogue.  Returns the kwargs of gemm / gemm2 and the output the GEMM writes."""
+        L = self.net_layers[net][i]
         P = self._matrix(self.flat, L)
         d = ws[net]["out"] if L.last else ws[net]["h"][i]
-        return dict(A=a.data_ptr(), B=P.data_ptr(), D=d.data_ptr(), M=m, N=L.rows if L.last else L.fan_out, K=L.fan_in,
-                    lda=lda, ldb=L.ld, ldd=d.stride(0), epilogue=HB_EPI_BIAS if L.last else HB_EPI_BIAS_ELU,
+        return dict(A=a.data_ptr(), B=P.data_ptr(), D=d.data_ptr(), M=ws["m"], N=L.rows if L.last else L.fan_out, K=L.fan_in,
+                    lda=a.stride(0), ldb=L.ld, ldd=d.stride(0), epilogue=HB_EPI_BIAS if L.last else HB_EPI_BIAS_ELU,
                     bias=P.data_ptr() + L.fan_in * 4, bias_stride=L.ld), d
 
+    def _wgrad_desc(self, net: str, i: int, d_cur: torch.Tensor, x: torch.Tensor, ws: dict):
+        """Weight gradient of layer i from d_cur, the gradient w.r.t. the layer's pre-activation output (x: the network's
+        input): G[rows, fan_in + 1] += d_cur^T [rows, m] * [act_in | 1] [m, fan_in + 1], split-K atomics into self.grad."""
+        L = self.net_layers[net][i]
+        act_in = x if i == 0 else ws[net]["h"][i - 1]      # [m, fan_in (+ ones column)]
+        return dict(A=d_cur.data_ptr(), B=act_in.data_ptr(), D=self._matrix(self.grad, L).data_ptr(), M=L.rows, N=L.fan_in + 1,
+                    K=ws["m"], lda=d_cur.stride(0), ldb=act_in.stride(0), ldd=L.ld, a_mn_major=1, b_mn_major=1,
+                    epilogue=HB_EPI_ATOMIC_ADD, split_k=0)
+
+    def _dgrad_desc(self, net: str, i: int, d_cur: torch.Tensor, ws: dict):
+        """Data gradient of layer i > 0 through the previous ELU: dz_prev = (d_cur * W) . elu'(h_prev).  Returns the kwargs
+        and dz_prev, the d_cur of layer i - 1."""
+        L = self.net_layers[net][i]
+        h_prev, dz = ws[net]["h"][i - 1], ws[net]["dz"][i - 1]
+        return dict(A=d_cur.data_ptr(), B=self._matrix(self.flat, L).data_ptr(), D=dz.data_ptr(), M=ws["m"], N=L.fan_in, K=L.rows,
+                    lda=d_cur.stride(0), ldb=L.ld, ldd=dz.stride(0), b_mn_major=1, epilogue=HB_EPI_ELU_BWD, H=h_prev.data_ptr(),
+                    ldh=h_prev.stride(0)), dz
+
+    # ------------------------------------------------------------------ one network at a time
+    def _mlp_forward(self, net: str, x: torch.Tensor, ws: dict):
+        """x: [m, ld] with ld % 4 == 0 (only the first fan_in columns are read).  Returns out [m,16]."""
+        lib, st = self._lib, torch.cuda.current_stream(self.device).cuda_stream
+        a = x
+        for i in range(4):
+            kw, a = self._fwd_desc(net, i, a, ws)
+            gemm(lib, st, self._scratch_for(net), **kw)
+        return a
+
+    def _mlp_backward(self, net: str, x: torch.Tensor, ws: dict):
+        """Gradients of every packed matrix of `net` from d_out (filled by the loss head); accumulates into
+        self.grad with split-K atomics (the buffer is zero on entry: Adam zeroes it).  Per layer, top down: the weight
+        gradient, then the data gradient that feeds the layer below."""
+        lib, st = self._lib, torch.cuda.current_stream(self.device).cuda_stream
+        d_cur = ws[net]["d_out"]
+        for i in (3, 2, 1, 0):
+            gemm(lib, st, self._scratch_for(net), **self._wgrad_desc(net, i, d_cur, x, ws))
+            if i > 0:
+                kw, d_cur = self._dgrad_desc(net, i, d_cur, ws)
+                gemm(lib, st, self._scratch_for(net), **kw)
+
+    # ------------------------------------------------------------------ both networks, layer by layer, grouped launches
     def forward_both(self, xa: torch.Tensor, xc: torch.Tensor, ws: dict):
         """The three hidden layers of the actor (on xa) and the critic (on xc): three grouped launches instead of six.
         Returns the last hidden activations (h3_actor, h3_critic)."""
         lib, st = self._lib, torch.cuda.current_stream(self.device).cuda_stream
-        m = xa.shape[0]
-        a, c = (xa, xa.stride(0)), (xc, xc.stride(0))
+        a, c = xa, xc
         for i in range(3):
-            kwa, da = self._fwd_kw("actor", i, a[0], a[1], m, ws)
-            kwc, dc = self._fwd_kw("critic", i, c[0], c[1], m, ws)
+            kwa, a = self._fwd_desc("actor", i, a, ws)
+            kwc, c = self._fwd_desc("critic", i, c, ws)
             gemm2(lib, st, self._scratch_for("critic"), kwc, self._scratch_for("actor"), kwa)      # the larger problem first
-            a, c = (da, da.stride(0)), (dc, dc.stride(0))
-        return ws["actor"]["h"][-1], ws["critic"]["h"][-1]
+        return a, c
 
     def backward_both(self, xa: torch.Tensor, xc: torch.Tensor, ws: dict):
         """Gradients of the three hidden layers of both networks from dz3 (left in ws by hb_ppo_head_fused): per layer one
         grouped data-gradient launch (critical path first) and one grouped weight-gradient launch - five launches for ten
         GEMMs."""
         lib, st = self._lib, torch.cuda.current_stream(self.device).cuda_stream
-        m = xa.shape[0]
-        nets = {"actor": xa, "critic": xc}
-        cur = {net: (ws[net]["dz"][-1], ws[net]["dz"][-1].stride(0)) for net in nets}
+        da, dc = ws["actor"]["dz"][-1], ws["critic"]["dz"][-1]
         for i in (2, 1, 0):
-            kw_w, kw_d, nxt = {}, {}, {}
-            for net, x in nets.items():
-                L = [L for L in self.layers if L.net == net][i]
-                G, P = self._matrix(self.grad, L), self._matrix(self.flat, L)
-                d_cur, ld_cur = cur[net]
-                act_in = x if i == 0 else ws[net]["h"][i - 1]
-                kw_w[net] = dict(A=d_cur.data_ptr(), B=act_in.data_ptr(), D=G.data_ptr(), M=L.rows, N=L.fan_in + 1, K=m, lda=ld_cur,
-                                 ldb=act_in.stride(0), ldd=L.ld, a_mn_major=1, b_mn_major=1, epilogue=HB_EPI_ATOMIC_ADD, split_k=0)
-                if i > 0:
-                    h_prev, dz = ws[net]["h"][i - 1], ws[net]["dz"][i - 1]
-                    kw_d[net] = dict(A=d_cur.data_ptr(), B=P.data_ptr(), D=dz.data_ptr(), M=m, N=L.fan_in, K=L.rows, lda=ld_cur,
-                                     ldb=L.ld, ldd=dz.stride(0), b_mn_major=1, epilogue=HB_EPI_ELU_BWD, H=h_prev.data_ptr(),
-                                     ldh=h_prev.stride(0))
-                    nxt[net] = (dz, dz.stride(0))
+            wa, wc = self._wgrad_desc("actor", i, da, xa, ws), self._wgrad_desc("critic", i, dc, xc, ws)
             if i > 0:
-                gemm2(lib, st, self._scratch_for("critic"), kw_d["critic"], self._scratch_for("actor"), kw_d["actor"])
-            gemm2(lib, st, self._scratch_for("critic"), kw_w["critic"], self._scratch_for("actor"), kw_w["actor"])
-            cur = nxt
-
-    def _mlp_backward(self, net: str, x: torch.Tensor, ws: dict, from_hidden: bool = False):
-        """Gradients of every packed matrix of `net` from d_out (filled by the loss head); accumulates into
-        self.grad with split-K atomics (the buffer is zero on entry: Adam zeroes it).  With from_hidden the
-        output layer has been handled by hb_ppo_head_fused, which left dz of the last hidden layer in ws."""
-        lib, st = self._lib, torch.cuda.current_stream(self.device).cuda_stream
-        Ls = [L for L in self.layers if L.net == net]
-        m = x.shape[0]
-        d_cur, ld_cur = ws[net]["d_out"], ws[net]["d_out"].stride(0)               # gradient w.r.t. the layer's pre-activation output
-        if from_hidden:
-            d_cur, ld_cur = ws[net]["dz"][-1], ws[net]["dz"][-1].stride(0)
-        for i in reversed(range(3 if from_hidden else 4)):
-            L = Ls[i]
-            G = self._matrix(self.grad, L)
-            act_in = x if i == 0 else ws[net]["h"][i - 1]      # [m, fan_in (+ ones column)]
-            n_w = L.fan_in + 1
-            # weight gradient: G[rows, fan_in + 1] += d_cur^T [rows, m] * [act_in | 1] [m, fan_in + 1]
-            gemm(lib, st, self._scratch_for(net), A=d_cur.data_ptr(), B=act_in.data_ptr(), D=G.data_ptr(), M=L.rows, N=n_w, K=m, lda=ld_cur,
-                 ldb=act_in.stride(0), ldd=L.ld, a_mn_major=1, b_mn_major=1, epilogue=HB_EPI_ATOMIC_ADD, split_k=0)
-            if i == 0:
-                break
-            # data gradient through the previous ELU: dz_prev = (d_cur * W) . elu'(h_prev)
-            P = self._matrix(self.flat, L)
-            h_prev, dz = ws[net]["h"][i - 1], ws[net]["dz"][i - 1]
-            gemm(lib, st, self._scratch_for(net), A=d_cur.data_ptr(), B=P.data_ptr(), D=dz.data_ptr(), M=m, N=L.fan_in, K=L.rows, lda=ld_cur,
-                 ldb=L.ld, ldd=dz.stride(0), b_mn_major=1, epilogue=HB_EPI_ELU_BWD, H=h_prev.data_ptr(),
-                 ldh=h_prev.stride(0))
-            d_cur, ld_cur = dz, dz.stride(0)
+                (kwa, da), (kwc, dc) = self._dgrad_desc("actor", i, da, ws), self._dgrad_desc("critic", i, dc, ws)
+                gemm2(lib, st, self._scratch_for("critic"), kwc, self._scratch_for("actor"), kwa)
+            gemm2(lib, st, self._scratch_for("critic"), wc, self._scratch_for("actor"), wa)
 
     def _as_operand(self, x: torch.Tensor, width: int) -> torch.Tensor:
         """TMA needs 16-byte aligned rows: use x in place when its row stride allows, else stage a padded copy."""

@@ -34,14 +34,8 @@ class _AdamState:
         self.param_groups = [{"lr": ppo._lr_host, "betas": (0.9, 0.999), "eps": 1e-8, "weight_decay": 0,
                               "amsgrad": False, "params": list(range(17))}]
 
-    def _views(self, flat):
-        ac = self._ppo.actor_critic
-        saved = ac.flat
-        try:
-            ac.flat = flat
-            return [v for _, v in ac.named_parameters()]
-        finally:
-            ac.flat = saved
+    def _views(self, buf):
+        return [v for _, v in self._ppo.actor_critic.named_views(buf)]
 
     def state_dict(self):
         p = self._ppo
@@ -105,7 +99,9 @@ class PPO:
         self.injected_eps = None            # parity: the Normal.sample() draw of the next act()
         self.injected_perm = None           # parity: the randperm of the next update()
         self._recorded_slot = None          # rollout slot already filled by the fast path of act()
-        self._side_stream = torch.cuda.Stream(self.device) if self.device.type == "cuda" else None
+        self._env = None                    # env that writes its observations straight into the rollout slots (attach_env)
+        self._slots = None                  # (storage, {k: views and addresses of rollout slot k}), see _slot
+        self._xa = self._xc = self._rec = None      # minibatch-ordered gathers of prepare_minibatches
         self.graph_rollout = True           # PPO.act: replay the hidden-layer GEMMs from a CUDA graph for small shards
         self.graph_rollout_max_envs = 16384
         self._act_graphs, self._act_stages = {}, {}
@@ -202,7 +198,7 @@ class PPO:
     def _slot(self, k):
         """Views and addresses of rollout slot k, built once per storage (tensor indexing costs microseconds)."""
         s = self.storage
-        cache = self.__dict__.get("_slots")
+        cache = self._slots
         if cache is None or cache[0] is not s:
             cache = self._slots = (s, {})
         e = cache[1].get(k)
@@ -216,9 +212,13 @@ class PPO:
             e.next_ptrs = (e.next[0].data_ptr(), e.next[1].data_ptr())
         return e
 
-    def _launch_act_head(self, e, h3a, h3c, eps, n, st):
+    def _act_fused(self, e, n, ws, st, eps):
+        """The fast path's launches for slot e, eagerly or under graph capture: the three grouped hidden-layer GEMMs reading
+        the slot's observations in place, then the fused output layers / sample / log-prob / value kernel writing into the
+        slot.  Callers draw eps in the argument list, so the draw is issued before the first GEMM."""
         ac = self.actor_critic
-        La, Lc = [L for L in ac.layers if L.last]
+        h3a, h3c = ac.forward_both(e.xa, e.xc, ws)
+        La, Lc = ac.output_layers
         _lib.check(self._lib.hb_ppo_act_fused(h3a.data_ptr(), h3a.stride(0), h3c.data_ptr(), h3c.stride(0),
                                               ac._matrix(ac.flat, La).data_ptr(), ac._matrix(ac.flat, Lc).data_ptr(), La.ld,
                                               ac.std.data_ptr(), eps.data_ptr(), n, ac.num_actions, e.actions.data_ptr(),
@@ -250,18 +250,13 @@ class PPO:
                 ws = ac.workspace(n)
                 st = torch.cuda.current_stream(self.device).cuda_stream
                 eps = self.injected_eps.contiguous() if self.injected_eps is not None else self._draw_eps(n, st)
-                if ac.grouped:
-                    h3a, h3c = ac.forward_both(e.xa, e.xc, ws)
-                else:
-                    h3a = ac._mlp_forward("actor", e.xa, ws, hidden_only=True)
-                    h3c = ac._mlp_forward("critic", e.xc, ws, hidden_only=True)
-                self._launch_act_head(e, h3a, h3c, eps, n, st)
+                self._act_fused(e, n, ws, st, eps)
                 self.injected_eps = None
             t.actions, t.values, t.actions_log_prob = e.actions, e.values, e.logp
             t.action_mean, t.action_sigma = e.mu, e.sigma
             t.observations, t.critic_observations = obs, critic_obs
             self._recorded_slot = k
-            env = self.__dict__.get("_env")
+            env = self._env
             if env is not None and env.num_envs == n:
                 # slot T exists: it takes the observations after the last transition
                 if e.next_ptrs[0] != obs.data_ptr() and e.next_ptrs[1] != critic_obs.data_ptr():
@@ -286,33 +281,17 @@ class PPO:
         return t.actions
 
     def _replay_act_graph(self, k, e, n):
-        """Capture (once per rollout slot, hb_graph_*) and replay: the three hidden-layer GEMMs of each network on two
-        branches, reading the slot's observations in place, the N(0,1) draw of the sample, and the fused output
-        layers / sample / log-prob / value kernel writing into the slot - library launches only."""
+        """Capture (once per rollout slot, hb_graph_*) and replay: the N(0,1) draw of the sample, the three grouped
+        hidden-layer GEMMs reading the slot's observations in place, and the fused output layers / sample / log-prob /
+        value kernel writing into the slot - library launches only."""
         entry = self._act_graphs.get(e.xa_ptr)
         if entry is None:
             ac, s, dev = self.actor_critic, self.storage, self.device
             ws = ac.workspace(n)
             if len(self._act_graphs) >= 4 * (s.num_transitions_per_env + 1):     # new storage: drop the stale graphs
                 self._act_graphs.clear()
-            side = self._side_stream
-
-            def launches(st):
-                main = torch.cuda.current_stream(dev)       # the capture stream
-                if ac.grouped:
-                    eps = self._draw_eps(n, st)
-                    h3a, h3c = ac.forward_both(e.xa, e.xc, ws)
-                else:
-                    side.wait_stream(main)
-                    h3a = ac._mlp_forward("actor", e.xa, ws, hidden_only=True)
-                    eps = self._draw_eps(n, st)
-                    with torch.cuda.stream(side):
-                        h3c = ac._mlp_forward("critic", e.xc, ws, hidden_only=True)
-                    main.wait_stream(side)
-                self._launch_act_head(e, h3a, h3c, eps, n, st)
-
             self._eps_stage(n)          # allocated before capture (and without consuming a draw)
-            g = _lib.LaunchGraph(dev).record(launches)
+            g = _lib.LaunchGraph(dev).record(lambda st: self._act_fused(e, n, ws, st, self._draw_eps(n, st)))
             entry = self._act_graphs[e.xa_ptr] = (g, e, ws)       # keeps the slot views and the workspace alive
         entry[0].replay(torch.cuda.current_stream(self.device).cuda_stream)
 
@@ -320,7 +299,7 @@ class PPO:
         """ppo.py:103-113.  After the fast path of act() only rewards (with the time-out bootstrap) and dones are
         left to record: one kernel."""
         t, s = self.transition, self.storage
-        k = getattr(self, "_recorded_slot", None)
+        k = self._recorded_slot
         if k is not None and k == s.step and rewards.is_cuda and rewards.dtype == torch.float32:
             rewards, dones = rewards.contiguous(), dones.contiguous()
             if dones.dtype not in (torch.bool, torch.uint8):
@@ -363,34 +342,16 @@ class PPO:
         xa, xc, rec = self._xa[i * mb:(i + 1) * mb], self._xc[i * mb:(i + 1) * mb], self._rec[i * mb:(i + 1) * mb]
         # self._stats is zero here: update() zeroes it once, the optimizer step's epilogue kernel re-arms it
         if ac.fused_head:
-            # The actor and critic chains are independent: the critic's GEMMs run on a second stream, so one network's
-            # persistent CTAs fill the SMs the other one leaves idle in its last round of tiles.
-            main = torch.cuda.current_stream(self.device)
-            side = self._side_stream
-            if ac.grouped:          # both networks layer by layer, one launch per layer
-                h3a, h3c = ac.forward_both(xa, xc, ws)
-            else:
-                side.wait_stream(main)
-                h3a = ac._mlp_forward("actor", xa, ws, hidden_only=True)
-                with torch.cuda.stream(side):
-                    h3c = ac._mlp_forward("critic", xc, ws, hidden_only=True)
-                main.wait_stream(side)
-            La, Lc = [L for L in ac.layers if L.last]
+            h3a, h3c = ac.forward_both(xa, xc, ws)
+            La, Lc = ac.output_layers
             dza, dzc = ws["actor"]["dz"][-1], ws["critic"]["dz"][-1]
             _lib.check(lib.hb_ppo_head_fused(
                 h3a.data_ptr(), h3a.stride(0), h3c.data_ptr(), h3c.stride(0),
                 ac._matrix(ac.flat, La).data_ptr(), ac._matrix(ac.flat, Lc).data_ptr(), La.ld, ac.std.data_ptr(),
                 rec.data_ptr(), mb, mb * self.world_size, C.byref(self._lp), dza.data_ptr(), dzc.data_ptr(), dza.stride(0),
                 ac._matrix(ac.grad, La).data_ptr(), ac._matrix(ac.grad, Lc).data_ptr(),
-                ac.grad[ac._std_offset:].data_ptr(), self._stats.data_ptr(), main.cuda_stream), "hb_ppo_head_fused")
-            if ac.grouped:
-                ac.backward_both(xa, xc, ws)
-            else:
-                side.wait_stream(main)
-                ac._mlp_backward("actor", xa, ws, from_hidden=True)
-                with torch.cuda.stream(side):
-                    ac._mlp_backward("critic", xc, ws, from_hidden=True)
-                main.wait_stream(side)
+                ac.grad[ac._std_offset:].data_ptr(), self._stats.data_ptr(), st), "hb_ppo_head_fused")
+            ac.backward_both(xa, xc, ws)
         else:
             mu16 = ac._mlp_forward("actor", xa, ws)
             v16 = ac._mlp_forward("critic", xc, ws)
@@ -421,12 +382,12 @@ class PPO:
         self._step += 1
 
     def _update_graph(self, i: int, adaptive: int):
-        """The launches of minibatch i's step as one CUDA graph (hb_graph_*): 6 forward GEMMs on two branches, the fused
-        head, 10 backward GEMMs on two branches, the optimizer step.  Every buffer address and every by-value argument
-        is the same for all epochs and updates (the step's scalars live in hb_optim_state), so it is captured once."""
+        """The launches of minibatch i's step as one CUDA graph (hb_graph_*): 3 grouped forward launches, the fused head,
+        5 grouped backward launches, the optimizer step.  Every buffer address and every by-value argument is the same for
+        all epochs and updates (the step's scalars live in hb_optim_state), so it is captured once."""
         key = (i, self._mb, self._xa.data_ptr(), self._xc.data_ptr(), self._rec.data_ptr(), adaptive, self.clip_param,
                self.value_loss_coef, self.entropy_coef, self.use_clipped_value_loss, self.max_grad_norm, self.desired_kl,
-               self.actor_critic.precision, self.actor_critic.grouped)
+               self.actor_critic.precision)
         g = self._update_graphs.get(key)
         if g is None:
             if len(self._update_graphs) >= 4 * self.num_mini_batches:
@@ -455,7 +416,7 @@ class PPO:
             perm = torch.randperm(used, device=dev)
         perm = perm.to(dev, dtype=torch.int64).contiguous()
         ld_a, ld_c = pitch(ac.num_actor_obs + 1), pitch(ac.num_critic_obs + 1)      # 128-byte rows for the layer-1 GEMMs
-        if getattr(self, "_xa", None) is None or self._xa.shape[0] != used:
+        if self._xa is None or self._xa.shape[0] != used:
             self._xa = torch.zeros(used, ld_a, device=dev)
             self._xc = torch.zeros(used, ld_c, device=dev)
             self._rec = torch.zeros(used, ppo_rec(ac.num_actions), device=dev)
@@ -474,8 +435,6 @@ class PPO:
     def update(self):
         perm, self.injected_perm = self.injected_perm, None
         mb = self.prepare_minibatches(perm)
-        self._mb, self._lp = mb, PpoLossParams(self.clip_param, self.value_loss_coef, self.entropy_coef,
-                                                int(self.use_clipped_value_loss), self.actor_critic.num_actions)
         adaptive = int(self.desired_kl is not None and self.schedule == "adaptive")
         self._per_update.zero_()                 # gradient norm scratch, minibatch loss sums, running sums
         self._opt_i64[OPT_STEPS_IN_UPDATE:OPT_STEPS_IN_UPDATE + 2].zero_()     # trace cursor, barrier ticket

@@ -13,10 +13,7 @@ from typing import Optional
 import torch
 
 from .. import _lib
-
-
-def _pitch(n: int) -> int:
-    return (n + 31) // 32 * 32          # whole 128-byte rows (actor_critic.pitch)
+from .actor_critic import pitch
 
 
 _FUSED_SCRATCH = {}
@@ -90,11 +87,11 @@ class RolloutStorage:
         # observations that follow the last transition when the env writes straight into the storage
         # (PPO.attach_env; they become slot 0 of the next rollout)
         # (pitch = ceil32(width + 1): there is always room for the constant ones column the weight-gradient GEMM reads)
-        self.obs_ld = _pitch(obs_shape[0] + 1)
+        self.obs_ld = pitch(obs_shape[0] + 1)
         self._observations = z(T + 1, N, self.obs_ld)
         self.observations = self._observations[:T, :, :obs_shape[0]]
         if privileged_obs_shape[0] is not None:
-            self.priv_ld = _pitch(privileged_obs_shape[0] + 1)
+            self.priv_ld = pitch(privileged_obs_shape[0] + 1)
             self._privileged_observations = z(T + 1, N, self.priv_ld)
             self.privileged_observations = self._privileged_observations[:T, :, :privileged_obs_shape[0]]
         else:

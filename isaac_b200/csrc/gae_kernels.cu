@@ -200,12 +200,6 @@ gae_serial_kernel(const float *__restrict__ rewards, const float *__restrict__ v
 // once.  Against memset + scan + normalise this drops two launches and the write + re-read of the raw advantages
 // (17 instead of 25 bytes per sample).  scratch = {sum, sum sq, ticket, -}: zero on entry, re-armed by the last block.
 // ------------------------------------------------------------------------------------------
-__device__ __forceinline__ unsigned long long ld_acquire_u64(const unsigned long long *p) {
-    unsigned long long v;
-    asm volatile("ld.acquire.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-    return v;
-}
-
 
 // The grid agrees on (sum, sum of squares): every block adds its pair to one of GAE_SLOTS slot pairs (blocks spread over the
 // slots, so that hundreds of fp64 atomics do not queue on one address), takes a ticket, spins until all blocks have (every
@@ -220,7 +214,7 @@ __device__ __forceinline__ void grid_statistics(double *__restrict__ scratch, do
     atomicAdd(scratch + GAE_SLOTS + slot, q);
     __threadfence();
     atomicAdd(ticket, 1ull);
-    while (ld_acquire_u64(ticket) < (unsigned long long)gridDim.x) { }           // ---- grid barrier ----
+    while (hb::ld_acquire_u64(ticket) < (unsigned long long)gridDim.x) { }       // ---- grid barrier ----
     const volatile double *sv = scratch;
     double s1 = 0.0, s2 = 0.0;
 #pragma unroll
@@ -351,13 +345,8 @@ int launch_gae_fused(const float *rewards, const float *values, const uint8_t *d
     const int grid = (N + THREADS - 1) / THREADS;
     *fits = grid <= per_sm * hb::sm_count();                 // the blocks wait for one another: all must be resident
     if (!*fits) return HB_OK;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(grid), cfg.blockDim = dim3(THREADS), cfg.dynamicSmemBytes = smem, cfg.stream = st;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeCooperative;
-    at[0].val.cooperative = hb::g_coop_launch ? 1 : 0;
-    cfg.attrs = at, cfg.numAttrs = 1;
-    HB_CUDA(cudaLaunchKernelEx(&cfg, kern, rewards, values, dones, last_values, returns, advantages, scratch, T, N, gamma, lam));
+    HB_CUDA(hb::launch_coop(kern, dim3(grid), dim3(THREADS), smem, st, rewards, values, dones, last_values, returns, advantages,
+                            scratch, T, N, gamma, lam));
     HB_CHECK_LAUNCH("gae_fused_kernel");
     return HB_OK;
 }

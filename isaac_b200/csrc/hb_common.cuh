@@ -74,6 +74,19 @@ inline cudaError_t launch_pdl(bool pdl, void (*kernel)(KArgs...), dim3 grid, dim
     cfg.attrs = at, cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
+
+// <<<grid, block, smem, stream>>> of a kernel whose blocks wait on one another at a grid barrier: the caller sizes the grid
+// to be co-resident, and the "coop_launch" option adds the cooperative attribute (g_coop_launch).
+template <typename... KArgs, typename... Args>
+inline cudaError_t launch_coop(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args &&...args) {
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = grid, cfg.blockDim = block, cfg.dynamicSmemBytes = smem, cfg.stream = st;
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeCooperative;
+    at[0].val.cooperative = g_coop_launch ? 1 : 0;
+    cfg.attrs = at, cfg.numAttrs = 1;
+    return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
+}
 #endif
 
 // ---- device helpers -------------------------------------------------------------------------
@@ -141,6 +154,13 @@ __device__ __forceinline__ void bulk_wait() {
 // predecessor grid has completed and its writes are visible).  pdl_trigger() lets the NEXT kernel start early.
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+
+// acquire load of a grid-barrier ticket or flag written by other blocks
+__device__ __forceinline__ unsigned long long ld_acquire_u64(const unsigned long long *p) {
+    unsigned long long v;
+    asm volatile("ld.acquire.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
+    return v;
+}
 
 // streaming loads / stores (data touched once per step: keep it out of L1)
 __device__ __forceinline__ float4 ld_stream4(const float4 *p) {

@@ -19,6 +19,16 @@ namespace {
             hb::set_error("num_actions = %d: built for 10 (hector), 12 (XBot-L), 18 (hector_full)", (int)(na)); \
             return HB_ERR_UNSUPPORTED;                                                    \
     }
+// The fused heads put one lane pair on each output, so they take at most 15 actions: HB_PPO_FUSED_DISPATCH builds 10 and 12
+// only; `msg` (printf format, one %d for the width) reports any other width.
+#define HB_PPO_FUSED_DISPATCH(na, CALL, msg)                                              \
+    switch (na) {                                                                         \
+        case 10: { constexpr int NA = 10; CALL; break; }                                  \
+        case 12: { constexpr int NA = 12; CALL; break; }                                  \
+        default:                                                                          \
+            hb::set_error(msg, (int)(na));                                                \
+            return HB_ERR_UNSUPPORTED;                                                    \
+    }
 constexpr float HALF_LOG_2PI = 0.91893853320467274178f;     // log(sqrt(2*pi))
 
 __global__ void __launch_bounds__(256)
@@ -491,12 +501,6 @@ act_head_kernel(const float *__restrict__ mu, int ld_mu, const float *__restrict
 constexpr int OPT_THREADS = 256;
 constexpr int OPT_REGV = 8;          // float4 gradient vectors a thread carries from phase 1 to phase 2
 
-__device__ __forceinline__ unsigned long long ld_acquire_u64(const unsigned long long *p) {
-    unsigned long long v;
-    asm volatile("ld.acquire.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-    return v;
-}
-
 __global__ void __launch_bounds__(OPT_THREADS)
 optimizer_step_kernel(float *__restrict__ p, float *__restrict__ g, float *__restrict__ m, float *__restrict__ v, long long n,
                       const hb_adam_params ap, hb_optim_state *__restrict__ st) {
@@ -530,7 +534,7 @@ optimizer_step_kernel(float *__restrict__ p, float *__restrict__ g, float *__res
         atomicAdd(&st->grad_sumsq, t);
         __threadfence();
         atomicAdd(ticket, 1ull);
-        while (ld_acquire_u64(ticket) < (unsigned long long)gridDim.x) { }      // ---- grid barrier ----
+        while (hb::ld_acquire_u64(ticket) < (unsigned long long)gridDim.x) { }  // ---- grid barrier ----
         const volatile hb_optim_state *sv = st;
         double lr = sv->lr;
         const double kl = sv->stats[2] / (double)ap.kl_count;
@@ -683,7 +687,7 @@ dp_optimizer_step_kernel(const __grid_constant__ hb_dp_comm c, float *__restrict
         }
     }
     if (threadIdx.x == 0) {
-        const bool ok = spin_until([&] { return ld_acquire_u64(go) >= 3ull * epoch + 1ull; });
+        const bool ok = spin_until([&] { return hb::ld_acquire_u64(go) >= 3ull * epoch + 1ull; });
         if (!ok) st->reserved = 2;
     }
     __syncthreads();
@@ -776,7 +780,7 @@ dp_optimizer_step_kernel(const __grid_constant__ hb_dp_comm c, float *__restrict
         }
     }
     if (threadIdx.x == 0) {
-        const bool ok = spin_until([&] { return ld_acquire_u64(go) >= 3ull * epoch + 2ull; });
+        const bool ok = spin_until([&] { return hb::ld_acquire_u64(go) >= 3ull * epoch + 2ull; });
         if (!ok) st->reserved = 4;
         const volatile float *bc = st->bcast;
         s_scal[0] = bc[0], s_scal[1] = bc[1], s_scal[2] = bc[2];
@@ -998,20 +1002,10 @@ int hb_ppo_head_fused(const float *h3_actor, int32_t ld_ha, const float *h3_crit
     const unsigned grid = (unsigned)(blocks < cap ? blocks : cap);
     const double inv_b = 1.0 / (double)mb_global;
     const float ent_scale = (float)((double)mb / (double)mb_global);
-    switch (lp->num_actions) {          // one lane pair per output: at most 15 actions
-        case 10:
-            head_fused_kernel<10><<<grid, HEAD_THREADS, 0, (cudaStream_t)stream>>>(h3_actor, ld_ha, h3_critic, ld_hc, w4_actor, w4_critic, ld_w, std,
-                records, mb, inv_b, ent_scale, *lp, dz3_actor, dz3_critic, ld_dz, g4_actor, g4_critic, d_std, stats);
-            break;
-        case 12:
-            head_fused_kernel<12><<<grid, HEAD_THREADS, 0, (cudaStream_t)stream>>>(h3_actor, ld_ha, h3_critic, ld_hc, w4_actor, w4_critic, ld_w, std,
-                records, mb, inv_b, ent_scale, *lp, dz3_actor, dz3_critic, ld_dz, g4_actor, g4_critic, d_std, stats);
-            break;
-        default:
-            hb::set_error("hb_ppo_head_fused: num_actions = %d (built for 10 and 12; wider heads use hb_gemm_tf32 + hb_ppo_loss_head)",
-                          lp->num_actions);
-            return HB_ERR_UNSUPPORTED;
-    }
+    HB_PPO_FUSED_DISPATCH(lp->num_actions, (head_fused_kernel<NA><<<grid, HEAD_THREADS, 0, (cudaStream_t)stream>>>(
+        h3_actor, ld_ha, h3_critic, ld_hc, w4_actor, w4_critic, ld_w, std, records, mb, inv_b, ent_scale, *lp, dz3_actor, dz3_critic,
+        ld_dz, g4_actor, g4_critic, d_std, stats)),
+        "hb_ppo_head_fused: num_actions = %d (built for 10 and 12; wider heads use hb_gemm_tf32 + hb_ppo_loss_head)");
     HB_CHECK_LAUNCH("head_fused_kernel");
     return HB_OK;
 }
@@ -1047,19 +1041,9 @@ int hb_ppo_act_fused(const float *h3_actor, int32_t ld_ha, const float *h3_criti
     long long blocks = (n + 7) / 8;
     const long long cap = 8ll * hb::sm_count();
     const unsigned grid = (unsigned)(blocks < cap ? blocks : cap);
-    switch (num_actions) {
-        case 10:
-            act_fused_kernel<10><<<grid, 256, 0, (cudaStream_t)stream>>>(h3_actor, ld_ha, h3_critic, ld_hc, w4_actor, w4_critic, ld_w, std, eps, n,
-                                                                          actions, log_prob, mu_out, sigma_out, values);
-            break;
-        case 12:
-            act_fused_kernel<12><<<grid, 256, 0, (cudaStream_t)stream>>>(h3_actor, ld_ha, h3_critic, ld_hc, w4_actor, w4_critic, ld_w, std, eps, n,
-                                                                          actions, log_prob, mu_out, sigma_out, values);
-            break;
-        default:
-            hb::set_error("hb_ppo_act_fused: num_actions = %d (built for 10 and 12)", num_actions);
-            return HB_ERR_UNSUPPORTED;
-    }
+    HB_PPO_FUSED_DISPATCH(num_actions, (act_fused_kernel<NA><<<grid, 256, 0, (cudaStream_t)stream>>>(
+        h3_actor, ld_ha, h3_critic, ld_hc, w4_actor, w4_critic, ld_w, std, eps, n, actions, log_prob, mu_out, sigma_out, values)),
+        "hb_ppo_act_fused: num_actions = %d (built for 10 and 12)");
     HB_CHECK_LAUNCH("act_fused_kernel");
     return HB_OK;
 }
@@ -1083,13 +1067,8 @@ int hb_optimizer_step(float *params, float *grads, float *exp_avg, float *exp_av
     const long long want = ((n >> 2) + OPT_THREADS - 1) / OPT_THREADS;
     const long long cap = 2ll * hb::sm_count();
     const unsigned grid = (unsigned)(want < 1 ? 1 : (want < cap ? want : cap));
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(grid), cfg.blockDim = dim3(OPT_THREADS), cfg.dynamicSmemBytes = 0, cfg.stream = (cudaStream_t)stream;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeCooperative;
-    at[0].val.cooperative = hb::g_coop_launch ? 1 : 0;
-    cfg.attrs = at, cfg.numAttrs = 1;
-    HB_CUDA(cudaLaunchKernelEx(&cfg, optimizer_step_kernel, params, grads, exp_avg, exp_avg_sq, (long long)n, *ap, state));
+    HB_CUDA(hb::launch_coop(optimizer_step_kernel, dim3(grid), dim3(OPT_THREADS), 0, (cudaStream_t)stream, params, grads, exp_avg,
+                            exp_avg_sq, (long long)n, *ap, state));
     HB_CHECK_LAUNCH("optimizer_step_kernel");
     return HB_OK;
 }
@@ -1119,13 +1098,8 @@ int hb_dp_optimizer_step(const hb_dp_comm *comm, float *exp_avg, float *exp_avg_
     const long long want = (per + DP_THREADS - 1) / DP_THREADS;
     const long long cap = hb::sm_count();                  // blocks wait on one another and on the peers: one per SM, all resident
     const unsigned grid = (unsigned)(want < 1 ? 1 : (want < cap ? want : cap));
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(grid), cfg.blockDim = dim3(DP_THREADS), cfg.stream = (cudaStream_t)stream;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeCooperative;
-    at[0].val.cooperative = hb::g_coop_launch ? 1 : 0;
-    cfg.attrs = at, cfg.numAttrs = 1;
-    HB_CUDA(cudaLaunchKernelEx(&cfg, dp_optimizer_step_kernel, *comm, exp_avg, exp_avg_sq, (long long)n, *ap, state));
+    HB_CUDA(hb::launch_coop(dp_optimizer_step_kernel, dim3(grid), dim3(DP_THREADS), 0, (cudaStream_t)stream, *comm, exp_avg,
+                            exp_avg_sq, (long long)n, *ap, state));
     HB_CHECK_LAUNCH("dp_optimizer_step_kernel");
     return HB_OK;
 }
