@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define HB_ABI_VERSION 5
+#define HB_ABI_VERSION 6
 
 typedef enum hb_status {
     HB_OK = 0,
@@ -366,9 +366,31 @@ int hb_gae_fused(const float *rewards, const float *values, const uint8_t *dones
 enum hb_gemm_epilogue {
     HB_EPI_STORE = 0,      /* D = acc */
     HB_EPI_BIAS = 1,       /* D = acc + bias[n]                       nn.Linear (actor_critic.py:62,74) */
-    HB_EPI_BIAS_ELU = 2,   /* D = elu(acc + bias[n])                  nn.Linear + nn.ELU (:56-60) */
-    HB_EPI_ELU_BWD = 3,    /* D = acc * elu'(z) with H = elu(z)       autograd of the above */
-    HB_EPI_ATOMIC_ADD = 4  /* D += acc (split-K weight gradients; D must be zeroed by the caller) */
+    HB_EPI_BIAS_ACT = 2,   /* D = f(acc + bias[n])                    nn.Linear + activation f (:56-60) */
+    HB_EPI_ACT_BWD = 3,    /* D = acc * f'(z) with H = f(z)           autograd of the above */
+    HB_EPI_ATOMIC_ADD = 4, /* D += acc (split-K weight gradients; D must be zeroed by the caller) */
+    HB_EPI_BIAS_ELU = HB_EPI_BIAS_ACT,     /* the names from before the activation became a descriptor field */
+    HB_EPI_ELU_BWD = HB_EPI_ACT_BWD
+};
+/* The activation f of HB_EPI_BIAS_ACT / HB_EPI_ACT_BWD: the set of get_activation in algo/ppo/actor_critic.py, with
+ * torch's definitions.  Every f' is written in the forward output h = f(z), which is what the data-gradient epilogue reads:
+ *   HB_ACT_ELU      z > 0 ? z : exp(z) - 1                       h > 0 ? 1 : h + 1
+ *   HB_ACT_SELU     s * (z > 0 ? z : a * (exp(z) - 1))           h > 0 ? s : h + s * a     (a = 1.6732632, s = 1.0507010)
+ *   HB_ACT_RELU     max(z, 0)                                    h > 0 ? 1 : 0              ("crelu" maps here too)
+ *   HB_ACT_LRELU    z > 0 ? z : 0.01 z                           h > 0 ? 1 : 0.01
+ *   HB_ACT_TANH     tanh(z)                                      1 - h * h
+ *   HB_ACT_SIGMOID  1 / (1 + exp(-z))                            (1 - h) * h
+ * In HB_GEMM_TF32 mode the non-ELU activations are built for the layouts these epilogues have in an MLP: HB_EPI_BIAS_ACT
+ * with A and B K-major, HB_EPI_ACT_BWD with A K-major and B MN-major (HB_ERR_UNSUPPORTED otherwise); ELU takes every
+ * layout.  An unknown value is HB_ERR_BAD_ARG. */
+enum hb_activation {
+    HB_ACT_ELU = 0,
+    HB_ACT_SELU = 1,
+    HB_ACT_RELU = 2,
+    HB_ACT_LRELU = 3,
+    HB_ACT_TANH = 4,
+    HB_ACT_SIGMOID = 5,
+    HB_ACT_COUNT = 6
 };
 /* A, B (and, for every epilogue but HB_EPI_ATOMIC_ADD, D and H) are moved by TMA: 16-byte aligned bases, leading dimensions
  * that are multiples of 4 floats (HB_ERR_BAD_ARG otherwise).  Ragged M / N are clipped by the tensor maps. */
@@ -389,6 +411,7 @@ typedef struct hb_gemm_desc {
     int32_t precision;           /* hb_gemm_precision */
     float *workspace;            /* HB_GEMM_3XTF32: scratch for the split operands, 16-byte aligned, */
     int64_t workspace_floats;    /*   at least hb_gemm_workspace_floats(desc) floats */
+    int32_t activation;          /* hb_activation of HB_EPI_BIAS_ACT / HB_EPI_ACT_BWD; 0 = ELU */
 } hb_gemm_desc;
 /* Arithmetic of the products.  HB_GEMM_TF32: operands truncated to TF32 by the tensor core (10-bit mantissa), fp32
  * accumulation - the fast path.  HB_GEMM_3XTF32: every operand is split x = hi + lo (hi = x rounded to TF32, lo = x - hi)
@@ -425,6 +448,7 @@ typedef struct hb_ppo_loss_params {
     float clip_param, value_loss_coef, entropy_coef;
     int32_t use_clipped_value_loss;
     int32_t num_actions;          /* 10 / 12 / 18 */
+    int32_t activation;           /* hb_activation of the hidden layers (hb_ppo_head_fused's f'); 0 = ELU */
 } hb_ppo_loss_params;
 /* Loss head and its analytic backward for one minibatch (ppo.py:130-168): Gaussian log-prob, ratio,
  * clipped surrogate, clipped value loss, entropy bonus, KL to the behaviour policy.
@@ -437,7 +461,7 @@ int hb_ppo_loss_head(const float *mu, int32_t ld_mu, const float *value, int32_t
 
 /* Update path, output layers fused with the loss head: for hidden width 128 (hector_config.py:207-210) the last
  * nn.Linear of both MLPs (actor_critic.py:62,74) is evaluated with fp32 FMAs inside the loss kernel, together with
- * its data gradient (into dz3 = d loss / d pre-activation of the last hidden layer, ELU' applied) and its weight /
+ * its data gradient (into dz3 = d loss / d pre-activation of the last hidden layer, f' of lp->activation applied) and its weight /
  * bias gradients (accumulated into g4_actor [>=10 rows, ld_w] and g4_critic [>=1 row, ld_w], packed [W | b]).
  * h3_* [mb, ld_h]: last hidden activations; w4_* packed [W | b] with leading dimension ld_w; records, std, lp,
  * d_std, stats as in hb_ppo_loss_head. */

@@ -10,7 +10,7 @@ import ctypes as C
 import os
 from typing import Optional
 
-HB_ABI_VERSION = 5
+HB_ABI_VERSION = 6
 HB_MAX_DOF = 24
 HB_MAX_OBS = 80
 HB_NUM_REWARDS = 22
@@ -84,7 +84,9 @@ class EnvNoise(C.Structure):
     _fields_ = [(name, _fp) for name in _NOISE_FIELDS] + [("rng_counter", _fp)]
 
 
-HB_EPI_STORE, HB_EPI_BIAS, HB_EPI_BIAS_ELU, HB_EPI_ELU_BWD, HB_EPI_ATOMIC_ADD = range(5)
+HB_EPI_STORE, HB_EPI_BIAS, HB_EPI_BIAS_ACT, HB_EPI_ACT_BWD, HB_EPI_ATOMIC_ADD = range(5)
+HB_EPI_BIAS_ELU, HB_EPI_ELU_BWD = HB_EPI_BIAS_ACT, HB_EPI_ACT_BWD
+HB_ACT_ELU, HB_ACT_SELU, HB_ACT_RELU, HB_ACT_LRELU, HB_ACT_TANH, HB_ACT_SIGMOID = range(6)      # hb_activation
 PPO_NUM_ACTIONS = (10, 12, 18)          # instantiations of the PPO head kernels (hector, XBot-L, hector_full)
 
 
@@ -100,7 +102,7 @@ class GemmDesc(C.Structure):
     _fields_ = [("A", _fp), ("B", _fp), ("D", _fp), ("M", _i), ("N", _i), ("K", _i), ("lda", _i), ("ldb", _i),
                 ("ldd", _i), ("a_mn_major", _i), ("b_mn_major", _i), ("epilogue", _i), ("bias", _fp),
                 ("bias_stride", _i), ("H", _fp), ("ldh", _i), ("split_k", _i), ("tile_n", _i), ("precision", _i),
-                ("workspace", _fp), ("workspace_floats", C.c_int64)]
+                ("workspace", _fp), ("workspace_floats", C.c_int64), ("activation", _i)]
 
 
 HB_GEMM_TF32, HB_GEMM_3XTF32 = 0, 1
@@ -108,7 +110,7 @@ HB_GEMM_TF32, HB_GEMM_3XTF32 = 0, 1
 
 class PpoLossParams(C.Structure):
     _fields_ = [("clip_param", _f), ("value_loss_coef", _f), ("entropy_coef", _f), ("use_clipped_value_loss", _i),
-                ("num_actions", _i)]
+                ("num_actions", _i), ("activation", _i)]
 
 
 class AdamParams(C.Structure):

@@ -6,8 +6,10 @@ passes.  Each `nn.Linear` is a packed matrix `P[out_pad, ld]` = `[W | b | 0-pad]
   * the weight-gradient GEMM multiplies by the activations extended with a constant ones column, so the bias
     gradient is simply column `in` of the packed gradient — no separate reduction kernel;
   * rows are 16-byte aligned (615*4 and 1050*4 are not, SURVEY.md §7 hard part 2).
-`state_dict()` / `load_state_dict()` use the reference's keys (`actor.{0,2,4,6}.{weight,bias}`,
-`critic.{0,2,4,6}.{weight,bias}`, `std`), so checkpoints interchange.
+Like the reference, each network has one or more hidden layers of its own widths and the activation `get_activation`
+names (ELU, SELU, ReLU, LeakyReLU, Tanh, Sigmoid), evaluated in the GEMM epilogues.  `state_dict()` / `load_state_dict()`
+use the reference's `nn.Sequential` keys (`actor.{0,2,...,2d}.{weight,bias}` for d hidden layers, `critic.…`, `std`), so
+checkpoints interchange.
 """
 from __future__ import annotations
 
@@ -18,8 +20,12 @@ from typing import Dict, List, Optional
 import torch
 
 from .. import _lib
-from .._lib import (GemmDesc, HB_EPI_ATOMIC_ADD, HB_EPI_BIAS, HB_EPI_BIAS_ELU, HB_EPI_ELU_BWD, HB_GEMM_3XTF32, HB_GEMM_TF32,
-                    PPO_NUM_ACTIONS)
+from .._lib import (GemmDesc, HB_ACT_ELU, HB_ACT_LRELU, HB_ACT_RELU, HB_ACT_SELU, HB_ACT_SIGMOID, HB_ACT_TANH, HB_EPI_ACT_BWD,
+                    HB_EPI_ATOMIC_ADD, HB_EPI_BIAS, HB_EPI_BIAS_ACT, HB_GEMM_3XTF32, HB_GEMM_TF32, PPO_NUM_ACTIONS)
+
+# the names get_activation resolves (algo/ppo/actor_critic.py), "crelu" being nn.ReLU there too
+ACTIVATIONS = {"elu": HB_ACT_ELU, "selu": HB_ACT_SELU, "relu": HB_ACT_RELU, "crelu": HB_ACT_RELU, "lrelu": HB_ACT_LRELU,
+               "tanh": HB_ACT_TANH, "sigmoid": HB_ACT_SIGMOID}
 
 
 def pitch(n: int) -> int:
@@ -83,17 +89,27 @@ class ActorCritic:
             print("ActorCritic.__init__ got unexpected arguments, which will be ignored: " + str(list(kwargs)))
         if num_actions not in PPO_NUM_ACTIONS:
             raise ValueError(f"the loss-head kernels are built for {PPO_NUM_ACTIONS} actions (hector, XBot-L, hector_full)")
-        if len(actor_hidden_dims) != 3 or len(critic_hidden_dims) != 3:
-            raise ValueError("three hidden layers per network (hector_config.py:207-210)")
+        activation = "elu" if activation is None else activation
+        if activation not in ACTIVATIONS:
+            raise ValueError(f"unknown activation {activation!r}: one of {sorted(ACTIVATIONS)}")
+        for name, dims in (("actor_hidden_dims", actor_hidden_dims), ("critic_hidden_dims", critic_hidden_dims)):
+            if len(dims) == 0:
+                raise ValueError(f"{name} is empty: each network needs at least one hidden layer")
+            if min(dims) <= 64:
+                raise ValueError(f"{name} = {list(dims)}: hidden widths must exceed 64 - the data-gradient GEMM into a hidden "
+                                 "layer reads the weights as an MN-major B operand with N = that layer's width, and an "
+                                 "MN-major B operand needs N > 64")
         self._lib = _lib.load()
+        self.activation = activation
+        self.hb_activation = ACTIVATIONS[activation]        # hb_activation of every GEMM epilogue and of the fused head
         self.device = torch.device(device)
         self.num_actor_obs, self.num_critic_obs, self.num_actions = num_actor_obs, num_critic_obs, num_actions
         self.layers: List[_Layer] = []
         off = 0
         for net, dims in (("actor", (num_actor_obs, *actor_hidden_dims, num_actions)),
                           ("critic", (num_critic_obs, *critic_hidden_dims, 1))):
-            for i in range(4):
-                L = _Layer(net, 2 * i, dims[i], dims[i + 1], i == 3, off)
+            for i in range(len(dims) - 1):
+                L = _Layer(net, 2 * i, dims[i], dims[i + 1], i == len(dims) - 2, off)
                 self.layers.append(L)
                 off += L.numel
         self.net_layers = {net: tuple(L for L in self.layers if L.net == net) for net in ("actor", "critic")}
@@ -215,13 +231,13 @@ class ActorCritic:
 
     def _fwd_desc(self, net: str, i: int, a: torch.Tensor, ws: dict):
         """Forward GEMM of layer i of `net` on a [m, ld] (ld % 4 == 0, only the first fan_in columns are read), bias and (hidden
-        layers) ELU in the epilogue.  Returns the kwargs of gemm / gemm2 and the output the GEMM writes."""
+        layers) the activation in the epilogue.  Returns the kwargs of gemm / gemm2 and the output the GEMM writes."""
         L = self.net_layers[net][i]
         P = self._matrix(self.flat, L)
         d = ws[net]["out"] if L.last else ws[net]["h"][i]
         return dict(A=a.data_ptr(), B=P.data_ptr(), D=d.data_ptr(), M=ws["m"], N=L.rows if L.last else L.fan_out, K=L.fan_in,
-                    lda=a.stride(0), ldb=L.ld, ldd=d.stride(0), epilogue=HB_EPI_BIAS if L.last else HB_EPI_BIAS_ELU,
-                    bias=P.data_ptr() + L.fan_in * 4, bias_stride=L.ld), d
+                    lda=a.stride(0), ldb=L.ld, ldd=d.stride(0), epilogue=HB_EPI_BIAS if L.last else HB_EPI_BIAS_ACT,
+                    bias=P.data_ptr() + L.fan_in * 4, bias_stride=L.ld, activation=self.hb_activation), d
 
     def _wgrad_desc(self, net: str, i: int, d_cur: torch.Tensor, x: torch.Tensor, ws: dict):
         """Weight gradient of layer i from d_cur, the gradient w.r.t. the layer's pre-activation output (x: the network's
@@ -230,23 +246,23 @@ class ActorCritic:
         act_in = x if i == 0 else ws[net]["h"][i - 1]      # [m, fan_in (+ ones column)]
         return dict(A=d_cur.data_ptr(), B=act_in.data_ptr(), D=self._matrix(self.grad, L).data_ptr(), M=L.rows, N=L.fan_in + 1,
                     K=ws["m"], lda=d_cur.stride(0), ldb=act_in.stride(0), ldd=L.ld, a_mn_major=1, b_mn_major=1,
-                    epilogue=HB_EPI_ATOMIC_ADD, split_k=0)
+                    epilogue=HB_EPI_ATOMIC_ADD, split_k=0, activation=self.hb_activation)
 
     def _dgrad_desc(self, net: str, i: int, d_cur: torch.Tensor, ws: dict):
-        """Data gradient of layer i > 0 through the previous ELU: dz_prev = (d_cur * W) . elu'(h_prev).  Returns the kwargs
-        and dz_prev, the d_cur of layer i - 1."""
+        """Data gradient of layer i > 0 through the previous activation f: dz_prev = (d_cur * W) . f'(h_prev).  Returns the
+        kwargs and dz_prev, the d_cur of layer i - 1."""
         L = self.net_layers[net][i]
         h_prev, dz = ws[net]["h"][i - 1], ws[net]["dz"][i - 1]
         return dict(A=d_cur.data_ptr(), B=self._matrix(self.flat, L).data_ptr(), D=dz.data_ptr(), M=ws["m"], N=L.fan_in, K=L.rows,
-                    lda=d_cur.stride(0), ldb=L.ld, ldd=dz.stride(0), b_mn_major=1, epilogue=HB_EPI_ELU_BWD, H=h_prev.data_ptr(),
-                    ldh=h_prev.stride(0)), dz
+                    lda=d_cur.stride(0), ldb=L.ld, ldd=dz.stride(0), b_mn_major=1, epilogue=HB_EPI_ACT_BWD, H=h_prev.data_ptr(),
+                    ldh=h_prev.stride(0), activation=self.hb_activation), dz
 
     # ------------------------------------------------------------------ one network at a time
     def _mlp_forward(self, net: str, x: torch.Tensor, ws: dict):
         """x: [m, ld] with ld % 4 == 0 (only the first fan_in columns are read).  Returns out [m,16]."""
         lib, st = self._lib, torch.cuda.current_stream(self.device).cuda_stream
         a = x
-        for i in range(4):
+        for i in range(len(self.net_layers[net])):
             kw, a = self._fwd_desc(net, i, a, ws)
             gemm(lib, st, self._scratch_for(net), **kw)
         return a
@@ -257,36 +273,60 @@ class ActorCritic:
         gradient, then the data gradient that feeds the layer below."""
         lib, st = self._lib, torch.cuda.current_stream(self.device).cuda_stream
         d_cur = ws[net]["d_out"]
-        for i in (3, 2, 1, 0):
+        for i in reversed(range(len(self.net_layers[net]))):
             gemm(lib, st, self._scratch_for(net), **self._wgrad_desc(net, i, d_cur, x, ws))
             if i > 0:
                 kw, d_cur = self._dgrad_desc(net, i, d_cur, ws)
                 gemm(lib, st, self._scratch_for(net), **kw)
 
     # ------------------------------------------------------------------ both networks, layer by layer, grouped launches
-    def forward_both(self, xa: torch.Tensor, xc: torch.Tensor, ws: dict):
-        """The three hidden layers of the actor (on xa) and the critic (on xc): three grouped launches instead of six.
-        Returns the last hidden activations (h3_actor, h3_critic)."""
+    def _hidden_depths(self):
+        return len(self.net_layers["actor"]) - 1, len(self.net_layers["critic"]) - 1
+
+    def _gemm_both(self, kwc, kwa):
+        """Layer i's GEMM of both networks in one grouped launch (the critic's, the larger problem, first) when both have a
+        hidden layer i; otherwise one launch of the network that has it (the other's kwargs are None)."""
         lib, st = self._lib, torch.cuda.current_stream(self.device).cuda_stream
+        if kwc is not None and kwa is not None:
+            gemm2(lib, st, self._scratch_for("critic"), kwc, self._scratch_for("actor"), kwa)
+        elif kwc is not None:
+            gemm(lib, st, self._scratch_for("critic"), **kwc)
+        else:
+            gemm(lib, st, self._scratch_for("actor"), **kwa)
+
+    def forward_both(self, xa: torch.Tensor, xc: torch.Tensor, ws: dict):
+        """The hidden layers of the actor (on xa) and the critic (on xc), input side first: one grouped launch per layer
+        index both networks have, then single launches for the deeper network's remaining layers (hector: three grouped
+        launches instead of six).  Returns the last hidden activations (h_actor, h_critic)."""
+        na, nc = self._hidden_depths()
         a, c = xa, xc
-        for i in range(3):
-            kwa, a = self._fwd_desc("actor", i, a, ws)
-            kwc, c = self._fwd_desc("critic", i, c, ws)
-            gemm2(lib, st, self._scratch_for("critic"), kwc, self._scratch_for("actor"), kwa)      # the larger problem first
+        for i in range(max(na, nc)):
+            kwa = kwc = None
+            if i < na:
+                kwa, a = self._fwd_desc("actor", i, a, ws)
+            if i < nc:
+                kwc, c = self._fwd_desc("critic", i, c, ws)
+            self._gemm_both(kwc, kwa)
         return a, c
 
     def backward_both(self, xa: torch.Tensor, xc: torch.Tensor, ws: dict):
-        """Gradients of the three hidden layers of both networks from dz3 (left in ws by hb_ppo_head_fused): per layer one
-        grouped data-gradient launch (critical path first) and one grouped weight-gradient launch - five launches for ten
-        GEMMs."""
-        lib, st = self._lib, torch.cuda.current_stream(self.device).cuda_stream
+        """Gradients of the hidden layers of both networks from the gradients w.r.t. the last hidden pre-activations (left in
+        ws by hb_ppo_head_fused), top layer index first: per layer index one data-gradient launch (critical path first) and
+        one weight-gradient launch, grouped where both networks have that hidden layer (hector: five launches for ten
+        GEMMs)."""
+        na, nc = self._hidden_depths()
         da, dc = ws["actor"]["dz"][-1], ws["critic"]["dz"][-1]
-        for i in (2, 1, 0):
-            wa, wc = self._wgrad_desc("actor", i, da, xa, ws), self._wgrad_desc("critic", i, dc, xc, ws)
+        for i in reversed(range(max(na, nc))):
+            wa = self._wgrad_desc("actor", i, da, xa, ws) if i < na else None
+            wc = self._wgrad_desc("critic", i, dc, xc, ws) if i < nc else None
             if i > 0:
-                (kwa, da), (kwc, dc) = self._dgrad_desc("actor", i, da, ws), self._dgrad_desc("critic", i, dc, ws)
-                gemm2(lib, st, self._scratch_for("critic"), kwc, self._scratch_for("actor"), kwa)
-            gemm2(lib, st, self._scratch_for("critic"), wc, self._scratch_for("actor"), wa)
+                kwa = kwc = None
+                if i < na:
+                    kwa, da = self._dgrad_desc("actor", i, da, ws)
+                if i < nc:
+                    kwc, dc = self._dgrad_desc("critic", i, dc, ws)
+                self._gemm_both(kwc, kwa)
+            self._gemm_both(wc, wa)
 
     def _as_operand(self, x: torch.Tensor, width: int) -> torch.Tensor:
         """TMA needs 16-byte aligned rows: use x in place when its row stride allows, else stage a padded copy."""

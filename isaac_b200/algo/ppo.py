@@ -3,9 +3,9 @@
     act / process_env_step / compute_returns / update       same signatures and semantics
     actor_critic, optimizer.state_dict(), learning_rate, storage, transition   same attributes
 
-Per minibatch step: 6 forward GEMMs (tcgen05, TF32 operands, fused bias+ELU), one fused kernel for the two
+Per minibatch step (hector's networks): 6 forward GEMMs (tcgen05, TF32 operands, fused bias + activation), one fused kernel for the two
 output layers + the loss head (log-prob, clipped surrogate, clipped value loss, entropy, KL, their analytic
-gradients, and the output layers' data / weight gradients), 4 data-gradient GEMMs (fused ELU'), 6 split-K
+gradients, and the output layers' data / weight gradients), 4 data-gradient GEMMs (fused activation derivative), 6 split-K
 weight-gradient GEMMs (bias gradients ride along as one more column), one gradient-norm reduction and one fused clip + Adam kernel that also applies the adaptive-KL learning-rate rule
 on the device (no `.item()` sync per minibatch; the reference needs ~22, SURVEY.md §3.4).  The minibatch
 permutation is drawn once per update and reused by every epoch (rollout_storage.py:149), so the index gathers
@@ -32,7 +32,7 @@ class _AdamState:
     def __init__(self, ppo: "PPO"):
         self._ppo = ppo
         self.param_groups = [{"lr": ppo._lr_host, "betas": (0.9, 0.999), "eps": 1e-8, "weight_decay": 0,
-                              "amsgrad": False, "params": list(range(17))}]
+                              "amsgrad": False, "params": list(range(len(self._views(ppo.actor_critic.flat))))}]
 
     def _views(self, buf):
         return [v for _, v in self._ppo.actor_critic.named_views(buf)]
@@ -429,7 +429,8 @@ class PPO:
                                            s.returns.data_ptr(), s.actions_log_prob.data_ptr(), ac.num_actions, self._rec.data_ptr(), st),
                    "hb_ppo_pack_samples")
         self._mb = mb
-        self._lp = PpoLossParams(self.clip_param, self.value_loss_coef, self.entropy_coef, int(self.use_clipped_value_loss), ac.num_actions)
+        self._lp = PpoLossParams(self.clip_param, self.value_loss_coef, self.entropy_coef, int(self.use_clipped_value_loss), ac.num_actions,
+                                 ac.hb_activation)
         return mb
 
     def update(self):

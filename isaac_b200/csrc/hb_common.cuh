@@ -40,6 +40,22 @@ void count_launch(int n = 1);
         }                                                                             \
     } while (0)
 
+// Runs CALL with `constexpr int ACT` = the hb_activation value `act` (the kernels take the activation as a template
+// parameter); an unknown value is HB_ERR_BAD_ARG.
+#define HB_ACT_CASE(A, CALL) case A: { constexpr int ACT = A; CALL; break; }
+#define HB_ACT_DISPATCH(act, CALL)                                                        \
+    switch (act) {                                                                        \
+        HB_ACT_CASE(HB_ACT_ELU, CALL)                                                     \
+        HB_ACT_CASE(HB_ACT_SELU, CALL)                                                    \
+        HB_ACT_CASE(HB_ACT_RELU, CALL)                                                    \
+        HB_ACT_CASE(HB_ACT_LRELU, CALL)                                                   \
+        HB_ACT_CASE(HB_ACT_TANH, CALL)                                                    \
+        HB_ACT_CASE(HB_ACT_SIGMOID, CALL)                                                 \
+        default:                                                                          \
+            hb::set_error("unknown activation %d (hb_activation)", (int)(act));          \
+            return HB_ERR_BAD_ARG;                                                        \
+    }
+
 inline bool aligned16(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
 int sm_count();   // cached cudaDevAttrMultiProcessorCount of the current device
@@ -191,6 +207,30 @@ __device__ __forceinline__ void st_stream4(float4 *p, const float4 &v) {
     asm volatile("st.global.L1::no_allocate.v4.f32 [%0], {%1,%2,%3,%4};" ::"l"(p), "f"(v.x), "f"(v.y), "f"(v.z),
                  "f"(v.w)
                  : "memory");
+}
+
+// Hidden-layer activations of the MLPs (hb_activation, torch's definitions: include/hector_b200.h).  act_fwd with
+// ACCURATE = true uses libm's expm1f / expf (fp32-grade, the 3xTF32 epilogue pass); otherwise the exponentials are __expf,
+// whose error is far below the TF32 operand rounding of the GEMM in front of it.  act_grad(h) is f'(z) written in the
+// forward output h = f(z).
+constexpr float SELU_ALPHA = 1.6732632423543772848170429916717f, SELU_SCALE = 1.0507009873554804934193349852946f;
+template <int ACT, bool ACCURATE>
+__device__ __forceinline__ float act_fwd(float z) {
+    if constexpr (ACT == HB_ACT_ELU) return z > 0.0f ? z : (ACCURATE ? expm1f(z) : __expf(z) - 1.0f);
+    else if constexpr (ACT == HB_ACT_SELU) return z > 0.0f ? SELU_SCALE * z : (SELU_SCALE * SELU_ALPHA) * (ACCURATE ? expm1f(z) : __expf(z) - 1.0f);
+    else if constexpr (ACT == HB_ACT_RELU) return z > 0.0f ? z : 0.0f;
+    else if constexpr (ACT == HB_ACT_LRELU) return z > 0.0f ? z : 0.01f * z;
+    else if constexpr (ACT == HB_ACT_TANH) return tanhf(z);
+    else return 1.0f / (1.0f + (ACCURATE ? expf(-z) : __expf(-z)));
+}
+template <int ACT>
+__device__ __forceinline__ float act_grad(float h) {
+    if constexpr (ACT == HB_ACT_ELU) return h > 0.0f ? 1.0f : h + 1.0f;
+    else if constexpr (ACT == HB_ACT_SELU) return h > 0.0f ? SELU_SCALE : h + SELU_SCALE * SELU_ALPHA;
+    else if constexpr (ACT == HB_ACT_RELU) return h > 0.0f ? 1.0f : 0.0f;
+    else if constexpr (ACT == HB_ACT_LRELU) return h > 0.0f ? 1.0f : 0.01f;
+    else if constexpr (ACT == HB_ACT_TANH) return 1.0f - h * h;
+    else return (1.0f - h) * h;
 }
 
 // Philox4x32-10 (counter c0..c3, key k0 k1): the library's device generator (env noise, PPO action sample)

@@ -7,8 +7,8 @@
 //   warp 9      allocates TMEM (two accumulators) and issues tcgen05.mma.cta_group::1.kind::tf32 (one elected
 //               lane); tcgen05.commit releases smem stages and hands finished accumulators to the epilogue
 //   warps 0-7   epilogue: tcgen05.ld the accumulator quarter / column half that belongs to the warp
-//               (lane = row), apply the fused tail in registers - bias + ELU (forward), ELU' (dgrad: the forward
-//               activations arrive by TMA, one 32 x 32 block ahead) - write the block into a 128-byte-swizzled
+//               (lane = row), apply the fused tail in registers - bias + activation f (forward), f' (dgrad: the
+//               forward activations arrive by TMA, one 32 x 32 block ahead) - write the block into a 128-byte-swizzled
 //               shared-memory tile and hand it to a TMA store; split-K wgrad tiles leave as vector red.add instead
 // The kernel is persistent: one CTA per SM walks a static tile list, so barrier / TMEM setup is paid once and
 // the epilogue of one tile overlaps the main loop of the next.
@@ -32,7 +32,7 @@ constexpr int EPI_WARPS = 8;          // two warps per TMEM lane quarter, each t
 constexpr int PRODUCER_WARP = EPI_WARPS, MMA_WARP = EPI_WARPS + 1;
 constexpr int GEMM_THREADS = (EPI_WARPS + 2) * 32;
 
-enum Epilogue { EPI_STORE = 0, EPI_BIAS = 1, EPI_BIAS_ELU = 2, EPI_ELU_BWD = 3, EPI_ATOMIC = 4 };
+enum Epilogue { EPI_STORE = 0, EPI_BIAS = 1, EPI_BIAS_ACT = 2, EPI_ACT_BWD = 3, EPI_ATOMIC = 4 };
 
 struct GemmArgs {
     int M, N, K;                  // logical sizes (K = contraction length)
@@ -42,7 +42,7 @@ struct GemmArgs {
     int ldd;
     const float *bias;            // bias[n * bias_stride] (weights and bias share one packed matrix)
     int bias_stride;
-    const float *H;               // EPI_ELU_BWD: forward activations [M, ldh]
+    const float *H;               // EPI_ACT_BWD: forward activations [M, ldh]
     int ldh;
     int snake;                    // rounds of the tile list dealt in alternating direction (problem 0's value counts)
 };
@@ -195,10 +195,10 @@ __host__ __device__ constexpr uint32_t make_idesc(int n, bool a_mn, bool b_mn, i
 // its own 128 rows of A but only HALF of the B tile (the tensor core reads the other half from the peer's shared
 // memory).  These TF32 GEMMs are bound by operand delivery (L2 -> SMEM, ~12 TB/s chip-wide), not by the tensor
 // pipe: per CTA and k-block a pair moves 32 KB instead of 48 KB for the same 128 x 256 x 32 MACs.
-constexpr int H_TILE_BYTES = 4096;                // ELU' epilogue: per warp, one TMA-loaded 32 x 32 block of forward activations
+constexpr int H_TILE_BYTES = 4096;                // f' epilogue: per warp, one TMA-loaded 32 x 32 block of forward activations
 template <int BN, bool PAIR, int EPI = 0>
 __host__ __device__ constexpr int stages_for() {
-    // the ELU' kernels give one stage to the epilogue warps' activation tiles (their K is a layer width: few k-blocks)
+    // the f' kernels give one stage to the epilogue warps' activation tiles (their K is a layer width: few k-blocks)
     return (PAIR ? 6 : (BN >= 256 ? 4 : (BN >= 128 ? 6 : 8))) - (EPI != 3 ? 0 : (BN >= 128 ? 1 : (BN >= 64 ? 2 : 0)));
 }
 
@@ -210,7 +210,7 @@ __host__ __device__ constexpr size_t smem_bytes_for() {
 }
 static_assert(smem_bytes_for<256, true, 3>() <= 227 * 1024 && smem_bytes_for<256, false, 3>() <= 227 * 1024 &&
                   smem_bytes_for<128, false, 3>() <= 227 * 1024 && smem_bytes_for<64, false, 3>() <= 227 * 1024,
-              "ELU' kernels: stages + output tiles + activation tiles must fit in shared memory");
+              "f' kernels: stages + output tiles + activation tiles must fit in shared memory");
 static_assert((EPI_WARPS * EPI_TILE_FLOATS * 4) % 1024 == 0, "the activation tiles behind the output tiles stay 1024-byte aligned");
 
 // Persistent, warp-specialised: one CTA per SM walks a static list of output tiles
@@ -221,7 +221,8 @@ static_assert((EPI_WARPS * EPI_TILE_FLOATS * 4) % 1024 == 0, "the activation til
 // GROUPED: one launch may carry TWO problems of the same kind (the actor's and the critic's GEMM of one layer): the tile
 // list is problem 0's tiles followed by problem 1's, dealt round-robin to the persistent CTAs, so both networks share
 // every wave of tiles and the pipeline set-up / drain of a launch is paid once per layer instead of once per network.
-template <int BN, bool A_MN, bool B_MN, int EPI, bool PAIR>
+// ACT: the hb_activation of EPI_BIAS_ACT / EPI_ACT_BWD (HB_ACT_ELU for the other epilogues).
+template <int BN, bool A_MN, bool B_MN, int EPI, bool PAIR, int ACT>
 __global__ void __launch_bounds__(GEMM_THREADS, 1)
 gemm_tf32_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_constant__ CUtensorMap map_b0,
                  const __grid_constant__ GemmArgs g0, const __grid_constant__ CUtensorMap map_a1,
@@ -262,11 +263,11 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_consta
     if (warp == PRODUCER_WARP && lane == 0) {
         prefetch_tmap(&map_a0), prefetch_tmap(&map_b0);
         if (EPI != EPI_ATOMIC) prefetch_tmap(&map_d0);
-        if (EPI == EPI_ELU_BWD) prefetch_tmap(&map_h0);
+        if (EPI == EPI_ACT_BWD) prefetch_tmap(&map_h0);
         if (g1.total_tiles > 0) {
             prefetch_tmap(&map_a1), prefetch_tmap(&map_b1);
             if (EPI != EPI_ATOMIC) prefetch_tmap(&map_d1);
-            if (EPI == EPI_ELU_BWD) prefetch_tmap(&map_h1);
+            if (EPI == EPI_ACT_BWD) prefetch_tmap(&map_h1);
         }
     }
     if (warp == MMA_WARP) {
@@ -394,7 +395,7 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_consta
         // Warp w reads TMEM lanes 32*(w%4) .. +31 (the hardware's lane-quarter rule) and the column half w/4.
         // The accumulator arrives with lane = row.  Global traffic wants lane = column (128-byte rows), so
         // every 32 x 32 block goes through a padded shared-memory tile private to the warp: activations for
-        // ELU' come in coalesced, results leave coalesced.
+        // f' come in coalesced, results leave coalesced.
         const int quarter = warp & 3, half = warp >> 2;
         constexpr int HALF_COLS = BN >= 64 ? BN / 2 : BN;          // narrow tiles: the second warp of a quarter idles
         const int c_begin = BN >= 64 ? half * HALF_COLS : 0;
@@ -410,7 +411,7 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_consta
             tile_coords(second ? t - g0.total_tiles : t, g, m0, n0, kb_begin, nkb);
             const uint32_t a = acc_it & 1, aph = (acc_it >> 1) & 1;
             const int mw = m0 + quarter * 32;                  // first row of this warp
-            // ELU': the warp's 32 x 32 blocks of the forward activations arrive by TMA in its second tile, one block ahead
+            // f': the warp's 32 x 32 blocks of the forward activations arrive by TMA in its second tile, one block ahead
             // of their use (the first while the accumulator is still being computed), with the same 128-byte swizzle
             uint8_t *htile = reinterpret_cast<uint8_t *>(epi_smem) + EPI_WARPS * EPI_TILE_FLOATS * 4 + warp * H_TILE_BYTES;
             const CUtensorMap *pmap_h = second ? &map_h1 : &map_h0;
@@ -420,7 +421,7 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_consta
                     tma_load_2d(htile, pmap_h, n0 + c, mw, &h_bar[warp]);
                 }
             };
-            if (EPI == EPI_ELU_BWD && c_begin < c_end && n0 + c_begin < g.N && mw < g.M) {
+            if (EPI == EPI_ACT_BWD && c_begin < c_end && n0 + c_begin < g.N && mw < g.M) {
                 if (g.N - (n0 + c_begin) > 32 && c_begin + 32 < c_end) {       // pull the blocks after the first towards L2 meanwhile
                     const int row = mw + lane, n_lo = n0 + c_begin + 32;
                     if (row < g.M) {
@@ -435,7 +436,7 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_consta
             tc_fence_after();
             const uint32_t tmem_acc = tmem_base + a * ACC_COLS + ((uint32_t)(quarter * 32) << 16);
             if constexpr (EPI != EPI_ATOMIC) {
-                // Plain / bias / ELU / ELU' results leave through the TMA: the warp applies the tail in registers (lane = row,
+                // Plain / bias / f / f' results leave through the TMA: the warp applies the tail in registers (lane = row,
                 // as TMEM delivers it), writes its 32 x 32 block into a 128-byte-swizzled 4 KB tile with eight conflict-free
                 // 16-byte stores per lane and hands the tile to one cp.async.bulk.tensor store - no transposing read-back, no
                 // per-lane global stores, ragged edges clipped by the tensor map.
@@ -447,7 +448,7 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_consta
                     const int n = n0 + c;
                     if (n >= g.N || mw >= g.M) break;
                     float4 h4[8];
-                    if (EPI == EPI_ELU_BWD) {                    // this lane's row of the block, chunk j at j ^ (lane % 8)
+                    if (EPI == EPI_ACT_BWD) {                    // this lane's row of the block, chunk j at j ^ (lane % 8)
                         hb::mbar_wait(&h_bar[warp], h_phase);
                         h_phase ^= 1u;
 #pragma unroll
@@ -459,7 +460,7 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_consta
                         }
                     }
                     float bias_l = 0.0f;
-                    if (EPI == EPI_BIAS || EPI == EPI_BIAS_ELU) bias_l = (n + lane < g.N) ? __ldg(g.bias + (size_t)(n + lane) * g.bias_stride) : 0.0f;
+                    if (EPI == EPI_BIAS || EPI == EPI_BIAS_ACT) bias_l = (n + lane < g.N) ? __ldg(g.bias + (size_t)(n + lane) * g.bias_stride) : 0.0f;
                     float v[32];
                     if (BN > 16) {
                         tmem_ld32(tmem_acc + (uint32_t)c, v);
@@ -476,19 +477,19 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_consta
                         }
                         handed_back = true;
                     }
-                    if (EPI == EPI_BIAS || EPI == EPI_BIAS_ELU) {
+                    if (EPI == EPI_BIAS || EPI == EPI_BIAS_ACT) {
 #pragma unroll
                         for (int i = 0; i < 32; ++i) {
                             float x = v[i] + __shfl_sync(0xffffffffu, bias_l, i);
-                            if (EPI == EPI_BIAS_ELU) x = x > 0.0f ? x : __expf(x) - 1.0f;       // nn.ELU(alpha=1)
+                            if (EPI == EPI_BIAS_ACT) x = hb::act_fwd<ACT, false>(x);
                             v[i] = x;
                         }
-                    } else if (EPI == EPI_ELU_BWD) {            // h = elu(z): elu'(z) = z > 0 ? 1 : h + 1
+                    } else if (EPI == EPI_ACT_BWD) {            // h = f(z): f'(z) from h
 #pragma unroll
                         for (int j = 0; j < 8; ++j) {
                             const float h[4] = {h4[j].x, h4[j].y, h4[j].z, h4[j].w};
 #pragma unroll
-                            for (int k = 0; k < 4; ++k) v[4 * j + k] *= (h[k] > 0.0f ? 1.0f : h[k] + 1.0f);
+                            for (int k = 0; k < 4; ++k) v[4 * j + k] *= hb::act_grad<ACT>(h[k]);
                         }
                     }
                     if (lane == 0) tma_store_wait_read();        // the previous block's store has read the tile
@@ -519,11 +520,11 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_consta
                 // readout mapping: 8 lanes x float4 per row, 4 rows per instruction (128-byte row segments)
                 const int rr = lane >> 3, c4 = (lane & 7) * 4;
                 const bool fast = (ncols == 32) && ((g.ldd & 3) == 0) && ((reinterpret_cast<uintptr_t>(g.D) & 15u) == 0) &&
-                                  (EPI != EPI_ELU_BWD || (((g.ldh & 3) == 0) && ((reinterpret_cast<uintptr_t>(g.H) & 15u) == 0)));
-                float4 h4[8];                                  // ELU': forward activations, all loads in flight early
+                                  (EPI != EPI_ACT_BWD || (((g.ldh & 3) == 0) && ((reinterpret_cast<uintptr_t>(g.H) & 15u) == 0)));
+                float4 h4[8];                                  // f': forward activations, all loads in flight early
                 float b4[4] = {0.f, 0.f, 0.f, 0.f};           // forward: this lane's four biases
                 if (fast) {
-                    if (EPI == EPI_ELU_BWD) {
+                    if (EPI == EPI_ACT_BWD) {
 #pragma unroll
                         for (int it = 0; it < 8; ++it) {
                             const int r = it * 4 + rr;
@@ -531,7 +532,7 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_consta
                                                  : make_float4(0.f, 0.f, 0.f, 0.f);
                         }
                     }
-                    if (EPI == EPI_BIAS || EPI == EPI_BIAS_ELU) {
+                    if (EPI == EPI_BIAS || EPI == EPI_BIAS_ACT) {
 #pragma unroll
                         for (int k = 0; k < 4; ++k) b4[k] = __ldg(g.bias + (size_t)(n + c4 + k) * g.bias_stride);
                     }
@@ -550,16 +551,16 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_consta
                         if (r < nrows) {
                             const float *tt = tile + r * 33 + c4;
                             float x[4] = {tt[0], tt[1], tt[2], tt[3]};
-                            if (EPI == EPI_BIAS || EPI == EPI_BIAS_ELU) {
+                            if (EPI == EPI_BIAS || EPI == EPI_BIAS_ACT) {
 #pragma unroll
                                 for (int k = 0; k < 4; ++k) {
                                     x[k] += b4[k];
-                                    if (EPI == EPI_BIAS_ELU) x[k] = x[k] > 0.0f ? x[k] : __expf(x[k]) - 1.0f;   // nn.ELU(alpha=1)
+                                    if (EPI == EPI_BIAS_ACT) x[k] = hb::act_fwd<ACT, false>(x[k]);
                                 }
-                            } else if (EPI == EPI_ELU_BWD) {    // h = elu(z): elu'(z) = z > 0 ? 1 : h + 1
+                            } else if (EPI == EPI_ACT_BWD) {
                                 const float h[4] = {h4[it].x, h4[it].y, h4[it].z, h4[it].w};
 #pragma unroll
-                                for (int k = 0; k < 4; ++k) x[k] *= (h[k] > 0.0f ? 1.0f : h[k] + 1.0f);
+                                for (int k = 0; k < 4; ++k) x[k] *= hb::act_grad<ACT>(h[k]);
                             }
                             float *dst = g.D + (size_t)(mw + r) * g.ldd + n + c4;
                             if (EPI == EPI_ATOMIC) {      // one 16-byte vector reduction per lane (sm_90+)
@@ -572,15 +573,14 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_consta
                         }
                     }
                 } else if (col_ok) {                           // ragged edge / unaligned: one column per lane
-                    const float bias = (EPI == EPI_BIAS || EPI == EPI_BIAS_ELU) ? __ldg(g.bias + (size_t)(n + lane) * g.bias_stride) : 0.0f;
+                    const float bias = (EPI == EPI_BIAS || EPI == EPI_BIAS_ACT) ? __ldg(g.bias + (size_t)(n + lane) * g.bias_stride) : 0.0f;
                     for (int r = 0; r < nrows; ++r) {
                         float x = tile[r * 33 + lane];
-                        if (EPI == EPI_BIAS || EPI == EPI_BIAS_ELU) {
+                        if (EPI == EPI_BIAS || EPI == EPI_BIAS_ACT) {
                             x += bias;
-                            if (EPI == EPI_BIAS_ELU) x = x > 0.0f ? x : __expf(x) - 1.0f;
-                        } else if (EPI == EPI_ELU_BWD) {
-                            const float h = __ldg(g.H + (size_t)(mw + r) * g.ldh + n + lane);
-                            x *= (h > 0.0f ? 1.0f : h + 1.0f);
+                            if (EPI == EPI_BIAS_ACT) x = hb::act_fwd<ACT, false>(x);
+                        } else if (EPI == EPI_ACT_BWD) {
+                            x *= hb::act_grad<ACT>(__ldg(g.H + (size_t)(mw + r) * g.ldh + n + lane));
                         }
                         float *dst = g.D + (size_t)(mw + r) * g.ldd + n + lane;
                         if (EPI == EPI_ATOMIC) atomicAdd(dst, x);
@@ -664,7 +664,7 @@ int setup_problem(const hb_gemm_desc *d, CUtensorMap *ma, CUtensorMap *mb, CUten
     constexpr int BN_CTA = PAIR ? BN / 2 : BN;
     int rc;
     *mh = CUtensorMap{};
-    if (EPI == EPI_ELU_BWD) {     // forward activations, read in the same 32 x 32 boxes as the output is written
+    if (EPI == EPI_ACT_BWD) {     // forward activations, read in the same 32 x 32 boxes as the output is written
         rc = make_map(mh, d->H, d->M, d->N, d->ldh, 32, 32, false);
         if (rc) return rc;
     }
@@ -697,11 +697,11 @@ int setup_problem(const hb_gemm_desc *d, CUtensorMap *ma, CUtensorMap *mb, CUten
 }
 
 // d1 may be null (one problem)
-template <int BN, bool A_MN, bool B_MN, int EPI, bool PAIR>
+template <int BN, bool A_MN, bool B_MN, int EPI, bool PAIR, int ACT>
 int launch(const hb_gemm_desc *d, const hb_gemm_desc *d1, cudaStream_t st) {
     constexpr size_t SMEM = smem_bytes_for<BN, PAIR, EPI>();
     static bool attr = false;
-    auto kern = gemm_tf32_kernel<BN, A_MN, B_MN, EPI, PAIR>;
+    auto kern = gemm_tf32_kernel<BN, A_MN, B_MN, EPI, PAIR, ACT>;
     if (!attr) {
         HB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM));
         attr = true;
@@ -760,12 +760,12 @@ int launch(const hb_gemm_desc *d, const hb_gemm_desc *d1, cudaStream_t st) {
 
 int g_gemm_pair = 1;          // "gemm_pair" option: 0 disables the 2-CTA kernels
 
-template <int BN, bool A_MN, bool B_MN, int EPI>
+template <int BN, bool A_MN, bool B_MN, int EPI, int ACT = HB_ACT_ELU>
 int launch_auto(const hb_gemm_desc *d, const hb_gemm_desc *d1, cudaStream_t st) {
     if constexpr (BN == 256) {
-        if (g_gemm_pair && d->M > BM && (!d1 || d1->M > BM)) return launch<BN, A_MN, B_MN, EPI, true>(d, d1, st);
+        if (g_gemm_pair && d->M > BM && (!d1 || d1->M > BM)) return launch<BN, A_MN, B_MN, EPI, true, ACT>(d, d1, st);
     }
-    return launch<BN, A_MN, B_MN, EPI, false>(d, d1, st);
+    return launch<BN, A_MN, B_MN, EPI, false, ACT>(d, d1, st);
 }
 
 template <int BN, int EPI>
@@ -777,13 +777,33 @@ int dispatch_major(const hb_gemm_desc *d, const hb_gemm_desc *d1, cudaStream_t s
     return HB_ERR_UNSUPPORTED;
 }
 
+// The activation epilogues: ELU in every layout, the other activations in the layout of their GEMM in an MLP - the forward
+// pass (A and B K-major) and the data gradient (A K-major, B = the weights MN-major).  An MN-major B has N > 64
+// (check_desc), so the data gradient never runs on tiles narrower than 128.
+template <int BN, int EPI>
+int dispatch_act(const hb_gemm_desc *d, const hb_gemm_desc *d1, cudaStream_t st) {
+    if (d->activation == HB_ACT_ELU) return dispatch_major<BN, EPI>(d, d1, st);
+    constexpr bool B_MN = EPI == EPI_ACT_BWD;
+    if (d->a_mn_major || (d->b_mn_major != 0) != B_MN) {
+        hb::set_error("hb_gemm_tf32: activation %d is built for %s only", d->activation,
+                      B_MN ? "A K-major with B MN-major (data gradient)" : "A and B K-major (forward)");
+        return HB_ERR_UNSUPPORTED;
+    }
+    if constexpr (B_MN && BN < 128) {
+        hb::set_error("hb_gemm_tf32: MN-major B needs N > 64");
+        return HB_ERR_BAD_ARG;
+    } else {
+        HB_ACT_DISPATCH(d->activation, return (launch_auto<BN, false, B_MN, EPI, ACT>(d, d1, st)));
+    }
+}
+
 template <int BN>
 int dispatch_epi(const hb_gemm_desc *d, const hb_gemm_desc *d1, cudaStream_t st) {
     switch (d->epilogue) {
         case HB_EPI_STORE: return dispatch_major<BN, EPI_STORE>(d, d1, st);
         case HB_EPI_BIAS: return dispatch_major<BN, EPI_BIAS>(d, d1, st);
-        case HB_EPI_BIAS_ELU: return dispatch_major<BN, EPI_BIAS_ELU>(d, d1, st);
-        case HB_EPI_ELU_BWD: return dispatch_major<BN, EPI_ELU_BWD>(d, d1, st);
+        case HB_EPI_BIAS_ACT: return dispatch_act<BN, EPI_BIAS_ACT>(d, d1, st);
+        case HB_EPI_ACT_BWD: return dispatch_act<BN, EPI_ACT_BWD>(d, d1, st);
         case HB_EPI_ATOMIC_ADD: return dispatch_major<BN, EPI_ATOMIC>(d, d1, st);
     }
     hb::set_error("hb_gemm_tf32: unknown epilogue %d", d->epilogue);
@@ -846,9 +866,10 @@ int gemm_tf32_dispatch(const hb_gemm_desc *d, cudaStream_t st);
 // 3e-8 relative per step (measured: 1.2e-5 over the ~400 steps of a K' = 3 * 1052 contraction, where exact accumulation of
 // the same split operands gives 5e-7).  The fp32-grade mode therefore keeps accumulation chains SHORT: the contraction
 // is cut into splits of CHAIN_KB k-blocks (16 accumulation steps), every split adds its partial tile to D with
-// round-to-nearest fp32 reductions (red.global.add), and bias / ELU / ELU' run as a separate pass over D.
+// round-to-nearest fp32 reductions (red.global.add), and bias / f / f' run as a separate pass over D (libm accuracy).
 constexpr int CHAIN_KB = 4;
 
+template <int ACT>
 __global__ void __launch_bounds__(256)
 epilogue_inplace_kernel(float *__restrict__ D, int ldd, long long M, int N, int epi, const float *__restrict__ bias, int bias_stride,
                         const float *__restrict__ H, int ldh) {
@@ -857,12 +878,11 @@ epilogue_inplace_kernel(float *__restrict__ D, int ldd, long long M, int N, int 
     const long long m = i / N;
     const int n = (int)(i - m * N);
     float x = D[(size_t)m * ldd + n];
-    if (epi == EPI_BIAS || epi == EPI_BIAS_ELU) {
+    if (epi == EPI_BIAS || epi == EPI_BIAS_ACT) {
         x += __ldg(bias + (size_t)n * bias_stride);
-        if (epi == EPI_BIAS_ELU) x = x > 0.0f ? x : expm1f(x);                   // nn.ELU(alpha=1)
-    } else if (epi == EPI_ELU_BWD) {
-        const float h = __ldg(H + (size_t)m * ldh + n);
-        x *= (h > 0.0f ? 1.0f : h + 1.0f);
+        if (epi == EPI_BIAS_ACT) x = hb::act_fwd<ACT, true>(x);
+    } else if (epi == EPI_ACT_BWD) {
+        x *= hb::act_grad<ACT>(__ldg(H + (size_t)m * ldh + n));
     }
     D[(size_t)m * ldd + n] = x;
 }
@@ -900,10 +920,10 @@ int gemm_3xtf32(const hb_gemm_desc *d, cudaStream_t st) {
     if (d->epilogue != HB_EPI_ATOMIC_ADD)                               // D = ..., not D += ...: start from zero
         HB_CUDA(cudaMemset2DAsync(d->D, (size_t)d->ldd * 4, 0, (size_t)d->N * 4, (size_t)d->M, st));
     if (int rc = gemm_tf32_dispatch(&e, st)) return rc;
-    if (d->epilogue == HB_EPI_BIAS || d->epilogue == HB_EPI_BIAS_ELU || d->epilogue == HB_EPI_ELU_BWD) {
+    if (d->epilogue == HB_EPI_BIAS || d->epilogue == HB_EPI_BIAS_ACT || d->epilogue == HB_EPI_ACT_BWD) {
         const long long total = (long long)d->M * d->N;
-        epilogue_inplace_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(d->D, d->ldd, d->M, d->N, d->epilogue, d->bias,
-                                                                              d->bias_stride, d->H, d->ldh);
+        HB_ACT_DISPATCH(d->activation, (epilogue_inplace_kernel<ACT><<<(unsigned)((total + 255) / 256), 256, 0, st>>>(
+            d->D, d->ldd, d->M, d->N, d->epilogue, d->bias, d->bias_stride, d->H, d->ldh)));
         HB_CHECK_LAUNCH("epilogue_inplace_kernel");
     }
     return HB_OK;
@@ -920,8 +940,9 @@ namespace {
 static int check_desc(const hb_gemm_desc *d) {
     HB_REQUIRE(d && d->A && d->B && d->D, "hb_gemm_tf32: null descriptor/operand");
     HB_REQUIRE(d->M > 0 && d->N > 0 && d->K > 0, "hb_gemm_tf32: empty problem %dx%dx%d", d->M, d->N, d->K);
-    HB_REQUIRE((d->epilogue != HB_EPI_BIAS && d->epilogue != HB_EPI_BIAS_ELU) || d->bias, "hb_gemm_tf32: bias epilogue without bias");
-    HB_REQUIRE(d->epilogue != HB_EPI_ELU_BWD || d->H, "hb_gemm_tf32: ELU backward epilogue without activations");
+    HB_REQUIRE((d->epilogue != HB_EPI_BIAS && d->epilogue != HB_EPI_BIAS_ACT) || d->bias, "hb_gemm_tf32: bias epilogue without bias");
+    HB_REQUIRE(d->epilogue != HB_EPI_ACT_BWD || d->H, "hb_gemm_tf32: activation backward epilogue without activations");
+    HB_REQUIRE(d->activation >= 0 && d->activation < HB_ACT_COUNT, "hb_gemm_tf32: unknown activation %d (hb_activation)", d->activation);
     HB_REQUIRE(d->split_k <= 1 || d->epilogue == HB_EPI_ATOMIC_ADD, "hb_gemm_tf32: split-K needs the atomic epilogue");
     HB_REQUIRE(!d->b_mn_major || d->N > 64, "hb_gemm_tf32: MN-major B needs N > 64 (32-wide TMA boxes per 128-byte swizzle row)");
     return HB_OK;
@@ -967,7 +988,8 @@ int gemm_tf32_dispatch(const hb_gemm_desc *d, cudaStream_t st) {
 int gemm_tf32_dispatch_grouped(const hb_gemm_desc *d0, const hb_gemm_desc *d1, cudaStream_t st) {
     if (int rc = check_desc(d0)) return rc;
     if (int rc = check_desc(d1)) return rc;
-    HB_REQUIRE(d0->epilogue == d1->epilogue && d0->a_mn_major == d1->a_mn_major && d0->b_mn_major == d1->b_mn_major,
+    HB_REQUIRE(d0->epilogue == d1->epilogue && d0->activation == d1->activation && d0->a_mn_major == d1->a_mn_major &&
+                   d0->b_mn_major == d1->b_mn_major,
                "hb_gemm_tf32_grouped: both problems must share epilogue and operand layouts");
     // one tile width for both: with two problems in flight there are enough tiles for the wide one whenever both are wide
     int bn0 = pick_tile_n(d0), bn1 = pick_tile_n(d1);
@@ -1000,6 +1022,8 @@ extern "C" int hb_gemm_tf32(const hb_gemm_desc *d, void *stream) {
     HB_REQUIRE(d->precision == HB_GEMM_TF32 || d->precision == HB_GEMM_3XTF32, "hb_gemm_tf32: unknown precision %d", d->precision);
     if (d->precision == HB_GEMM_3XTF32) {
         HB_REQUIRE(d->A && d->B && d->D && d->M > 0 && d->N > 0 && d->K > 0, "hb_gemm_tf32: null operand / empty problem");
+        HB_REQUIRE(d->activation >= 0 && d->activation < HB_ACT_COUNT, "hb_gemm_tf32: unknown activation %d (hb_activation)",
+                   d->activation);
         return gemm_3xtf32(d, (cudaStream_t)stream);
     }
     return gemm_tf32_dispatch(d, (cudaStream_t)stream);

@@ -93,12 +93,22 @@ __device__ __forceinline__ float warp_sum(float v) {
     return v;
 }
 
+// The loss coefficients as the kernels take them by value: hb_ppo_loss_params without its activation field, which picks
+// the instantiation of head_fused_kernel instead; a field added to the header struct does not move the kernels' parameters.
+struct LossCoefs {
+    float clip_param, value_loss_coef, entropy_coef;
+    int32_t use_clipped_value_loss, num_actions;
+};
+inline LossCoefs loss_coefs(const hb_ppo_loss_params &p) {
+    return {p.clip_param, p.value_loss_coef, p.entropy_coef, p.use_clipped_value_loss, p.num_actions};
+}
+
 // ppo.py:130-168 and its gradient w.r.t. mu, value and std.  One thread per sample.
 template <int NA>
 __global__ void __launch_bounds__(256)
 loss_head_kernel(const float *__restrict__ mu, int ld_mu, const float *__restrict__ value, int ld_v,
                  const float *__restrict__ stdp, const float *__restrict__ rec, long long mb, double inv_b,
-                 float ent_scale, hb_ppo_loss_params lp, float *__restrict__ d_mu, float *__restrict__ d_value,
+                 float ent_scale, LossCoefs lp, float *__restrict__ d_mu, float *__restrict__ d_value,
                  float *__restrict__ d_std, double *__restrict__ stats) {
     __shared__ float s_dstd[8][NA];
     __shared__ double s_stat[8][4];
@@ -191,7 +201,7 @@ loss_head_kernel(const float *__restrict__ mu, int ld_mu, const float *__restric
 // activations and the loss.  One pass over the minibatch does, per sample (one warp per row, lane = 4 features):
 //   mu = H3a W4a^T + b, v = H3c W4c^T + b          actor_critic.py:62,74 (fp32 FMAs, not TF32)
 //   loss head and its gradient (ppo.py:130-168)     same arithmetic as loss_head_kernel
-//   dz3 = (d_out W4) * elu'(H3)                     data gradient into the last hidden layer
+//   dz3 = (d_out W4) * f'(H3)                       data gradient into the last hidden layer (f: ACT, hb_activation)
 //   G4 += d_out^T [H3 | 1]                          weight + bias gradients, reduced per CTA, then atomics
 // so H3 is read once and mu / value / d_out never touch HBM.
 // ------------------------------------------------------------------------------------------------------------
@@ -218,11 +228,11 @@ __device__ __forceinline__ float warp_reduce16(float (&v)[16], int lane) {
     return v[0] + __shfl_xor_sync(0xffffffffu, v[0], 1);
 }
 
-template <int NA>
+template <int NA, int ACT>
 __global__ void __launch_bounds__(HEAD_THREADS, 1)
 head_fused_kernel(const float *__restrict__ h3a, int ld_ha, const float *__restrict__ h3c, int ld_hc,
                   const float *__restrict__ w4a, const float *__restrict__ w4c, int ld_w, const float *__restrict__ stdp,
-                  const float *__restrict__ rec, long long mb, double inv_b, float ent_scale, hb_ppo_loss_params lp,
+                  const float *__restrict__ rec, long long mb, double inv_b, float ent_scale, LossCoefs lp,
                   float *__restrict__ dz3a, float *__restrict__ dz3c, int ld_dz, float *__restrict__ g4a,
                   float *__restrict__ g4c, float *__restrict__ d_std, double *__restrict__ stats) {
     constexpr int HEAD_OUT = NA + 1;         // NA action means + 1 value: one lane pair each (NA <= 15)
@@ -339,7 +349,7 @@ head_fused_kernel(const float *__restrict__ h3a, int ld_ha, const float *__restr
         if (own_action && even) gstd += g_lp * ((diff * diff) * inv_var_sg - inv_sg);
         if (even) gb += g_out;
         stf[0] += fmaxf(s1, s2), stf[1] += st_v, stf[2] += kl, stf[3] += ent;       // a warp sees a few dozen rows: fp32 is enough here
-        // ---- data gradient through the last ELU (elu'(z) = z > 0 ? 1 : elu(z) + 1) and weight gradients ----
+        // ---- data gradient through the last activation (f'(z) from h = f(z)) and weight gradients ----
         float da[4] = {0.f, 0.f, 0.f, 0.f};
 #pragma unroll
         for (int j = 0; j < NA; ++j) {
@@ -354,8 +364,8 @@ head_fused_kernel(const float *__restrict__ h3a, int ld_ha, const float *__restr
         float dc[4];
 #pragma unroll
         for (int i = 0; i < 4; ++i) {
-            da[i] *= (ha[i] > 0.0f ? 1.0f : ha[i] + 1.0f);
-            dc[i] = (g_v * wcv[i]) * (hc[i] > 0.0f ? 1.0f : hc[i] + 1.0f);
+            da[i] *= hb::act_grad<ACT>(ha[i]);
+            dc[i] = (g_v * wcv[i]) * hb::act_grad<ACT>(hc[i]);
             gc[i] += g_v * hc[i];
         }
         hb::st_stream4(reinterpret_cast<float4 *>(dz3a + (size_t)row * ld_dz) + lane, make_float4(da[0], da[1], da[2], da[3]));
@@ -979,7 +989,7 @@ int hb_ppo_loss_head(const float *mu, int32_t ld_mu, const float *value, int32_t
     HB_REQUIRE(mu && value && std && records && lp && d_mu && d_value && d_std && stats, "hb_ppo_loss_head: null buffer");
     HB_REQUIRE(mb > 0 && mb_global >= mb && ld_mu >= lp->num_actions && ld_v >= 1, "hb_ppo_loss_head: bad sizes");
     HB_PPO_DISPATCH(lp->num_actions, (loss_head_kernel<NA><<<(unsigned)((mb + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
-        mu, ld_mu, value, ld_v, std, records, mb, 1.0 / (double)mb_global, (float)((double)mb / (double)mb_global), *lp, d_mu,
+        mu, ld_mu, value, ld_v, std, records, mb, 1.0 / (double)mb_global, (float)((double)mb / (double)mb_global), loss_coefs(*lp), d_mu,
         d_value, d_std, stats)));
     HB_CHECK_LAUNCH("loss_head_kernel");
     return HB_OK;
@@ -1002,9 +1012,10 @@ int hb_ppo_head_fused(const float *h3_actor, int32_t ld_ha, const float *h3_crit
     const unsigned grid = (unsigned)(blocks < cap ? blocks : cap);
     const double inv_b = 1.0 / (double)mb_global;
     const float ent_scale = (float)((double)mb / (double)mb_global);
-    HB_PPO_FUSED_DISPATCH(lp->num_actions, (head_fused_kernel<NA><<<grid, HEAD_THREADS, 0, (cudaStream_t)stream>>>(
-        h3_actor, ld_ha, h3_critic, ld_hc, w4_actor, w4_critic, ld_w, std, records, mb, inv_b, ent_scale, *lp, dz3_actor, dz3_critic,
-        ld_dz, g4_actor, g4_critic, d_std, stats)),
+    const LossCoefs coefs = loss_coefs(*lp);
+    HB_PPO_FUSED_DISPATCH(lp->num_actions, HB_ACT_DISPATCH(lp->activation, (head_fused_kernel<NA, ACT><<<grid, HEAD_THREADS, 0,
+        (cudaStream_t)stream>>>(h3_actor, ld_ha, h3_critic, ld_hc, w4_actor, w4_critic, ld_w, std, records, mb, inv_b, ent_scale,
+        coefs, dz3_actor, dz3_critic, ld_dz, g4_actor, g4_critic, d_std, stats))),
         "hb_ppo_head_fused: num_actions = %d (built for 10 and 12; wider heads use hb_gemm_tf32 + hb_ppo_loss_head)");
     HB_CHECK_LAUNCH("head_fused_kernel");
     return HB_OK;
