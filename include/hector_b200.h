@@ -438,7 +438,9 @@ int hb_ppo_gather_rows(const float *src, int32_t ld_src, float *dst, int32_t ld_
                        int64_t rows, int32_t cols, int32_t ones_col, void *stream);
 
 /* Per-sample record, gathered in minibatch order: actions[A] old_mu[A] old_sigma[A] old_value advantage
- * return old_log_prob 0 0 = HB_PPO_REC(A) floats; A = num_actions: 10 (hector), 12 (XBot-L), 18 (hector_full). */
+ * return old_log_prob 0 0 = HB_PPO_REC(A) floats; A = num_actions, 1 to 64 (hb_ppo_pack_samples, hb_ppo_loss_head
+ * and hb_ppo_act_head) or 1 to 15 (hb_ppo_head_fused, hb_ppo_act_fused).  A count below 1 is HB_ERR_BAD_ARG, one above
+ * the entry point's limit HB_ERR_UNSUPPORTED; either is refused before any launch. */
 #define HB_PPO_REC(num_actions) (3 * (num_actions) + 6)
 int hb_ppo_pack_samples(const int64_t *perm, int64_t rows, const float *actions, const float *mu, const float *sigma,
                         const float *values, const float *advantages, const float *returns, const float *log_prob,
@@ -447,13 +449,13 @@ int hb_ppo_pack_samples(const int64_t *perm, int64_t rows, const float *actions,
 typedef struct hb_ppo_loss_params {
     float clip_param, value_loss_coef, entropy_coef;
     int32_t use_clipped_value_loss;
-    int32_t num_actions;          /* 10 / 12 / 18 */
+    int32_t num_actions;          /* 1 to 64 (hb_ppo_loss_head), 1 to 15 (hb_ppo_head_fused) */
     int32_t activation;           /* hb_activation of the hidden layers (hb_ppo_head_fused's f'); 0 = ELU */
 } hb_ppo_loss_params;
 /* Loss head and its analytic backward for one minibatch (ppo.py:130-168): Gaussian log-prob, ratio,
  * clipped surrogate, clipped value loss, entropy bonus, KL to the behaviour policy.
- * mu [mb, ld_mu] (first 10 columns), value [mb, ld_v] (first column), std[10], records [mb, HB_PPO_REC].
- * Writes d_mu [mb, ld_mu] and d_value [mb, ld_v] (padding columns zeroed), accumulates d_std[10] and
+ * mu [mb, ld_mu] (first A = num_actions columns), value [mb, ld_v] (first column), std[A], records [mb, HB_PPO_REC(A)].
+ * Writes d_mu [mb, ld_mu] and d_value [mb, ld_v] (padding columns zeroed), accumulates d_std[A] and
  * stats[4] = {sum surrogate, sum value loss, sum kl, sum entropy} (fp64; caller zeroes both). */
 int hb_ppo_loss_head(const float *mu, int32_t ld_mu, const float *value, int32_t ld_v, const float *std,
                      const float *records, int64_t mb, int64_t mb_global, const hb_ppo_loss_params *lp, float *d_mu,
@@ -462,9 +464,10 @@ int hb_ppo_loss_head(const float *mu, int32_t ld_mu, const float *value, int32_t
 /* Update path, output layers fused with the loss head: for hidden width 128 (hector_config.py:207-210) the last
  * nn.Linear of both MLPs (actor_critic.py:62,74) is evaluated with fp32 FMAs inside the loss kernel, together with
  * its data gradient (into dz3 = d loss / d pre-activation of the last hidden layer, f' of lp->activation applied) and its weight /
- * bias gradients (accumulated into g4_actor [>=10 rows, ld_w] and g4_critic [>=1 row, ld_w], packed [W | b]).
+ * bias gradients (accumulated into g4_actor [>=A rows, ld_w] and g4_critic [>=1 row, ld_w], packed [W | b]).
  * h3_* [mb, ld_h]: last hidden activations; w4_* packed [W | b] with leading dimension ld_w; records, std, lp,
- * d_std, stats as in hb_ppo_loss_head. */
+ * d_std, stats as in hb_ppo_loss_head.  A = lp->num_actions, 1 to 15: one lane pair per action and one for the value
+ * (wider heads: hb_gemm_tf32 + hb_ppo_loss_head). */
 int hb_ppo_head_fused(const float *h3_actor, int32_t ld_ha, const float *h3_critic, int32_t ld_hc, const float *w4_actor,
                       const float *w4_critic, int32_t ld_w, const float *std, const float *records, int64_t mb,
                       int64_t mb_global, const hb_ppo_loss_params *lp, float *dz3_actor, float *dz3_critic, int32_t ld_dz,
@@ -476,14 +479,16 @@ int hb_ppo_head_fused(const float *h3_actor, int32_t ld_ha, const float *h3_crit
  * (write the key, zero the counter). */
 int hb_ppo_draw_normal(float *out, int64_t count, uint64_t *state, void *stream);
 
-/* PPO.act head (ppo.py:91-101, actor_critic.py:111-120): a = mu + sigma*eps, log-prob, copies of mu/sigma. */
+/* PPO.act head (ppo.py:91-101, actor_critic.py:111-120): a = mu + sigma*eps, log-prob, copies of mu/sigma; 1 to 64
+ * actions. */
 int hb_ppo_act_head(const float *mu, int32_t ld_mu, const float *std, const float *eps, int64_t n, int32_t num_actions,
                     float *actions, float *log_prob, float *mu_out, float *sigma_out, void *stream);
 
 /* Rollout side.  hb_ppo_act_fused: the output layers of both MLPs (hidden width 128) + PPO.act's sampling head
  * (ppo.py:91-101, actor_critic.py:111-120): a = mu + sigma * eps, log-prob, mu, sigma and the value, written to
  * caller-chosen destinations - normally the rollout-storage slot of the step (rollout_storage.py:87-100), so
- * add_transitions' copies of these tensors disappear.  actions/mu_out/sigma_out [n,10], log_prob/values [n].
+ * add_transitions' copies of these tensors disappear.  actions/mu_out/sigma_out [n, num_actions] with 1 to 15 actions,
+ * log_prob/values [n].
  * hb_ppo_record_step: PPO.process_env_step's record (ppo.py:103-113): rewards_out = rewards + gamma * values *
  * time_outs (time_outs may be NULL), dones_out = dones as uint8. */
 int hb_ppo_act_fused(const float *h3_actor, int32_t ld_ha, const float *h3_critic, int32_t ld_hc, const float *w4_actor,

@@ -87,7 +87,8 @@ class EnvNoise(C.Structure):
 HB_EPI_STORE, HB_EPI_BIAS, HB_EPI_BIAS_ACT, HB_EPI_ACT_BWD, HB_EPI_ATOMIC_ADD = range(5)
 HB_EPI_BIAS_ELU, HB_EPI_ELU_BWD = HB_EPI_BIAS_ACT, HB_EPI_ACT_BWD
 HB_ACT_ELU, HB_ACT_SELU, HB_ACT_RELU, HB_ACT_LRELU, HB_ACT_TANH, HB_ACT_SIGMOID = range(6)      # hb_activation
-PPO_NUM_ACTIONS = (10, 12, 18)          # instantiations of the PPO head kernels (hector, XBot-L, hector_full)
+PPO_MAX_ACTIONS = 64                    # hb_ppo_pack_samples / _loss_head / _act_head take 1 to 64 actions
+PPO_MAX_FUSED_ACTIONS = 15              # hb_ppo_head_fused / _act_fused take 1 to 15 (one lane pair per output)
 
 
 def ppo_rec(num_actions: int) -> int:

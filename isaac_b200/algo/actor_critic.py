@@ -21,7 +21,8 @@ import torch
 
 from .. import _lib
 from .._lib import (GemmDesc, HB_ACT_ELU, HB_ACT_LRELU, HB_ACT_RELU, HB_ACT_SELU, HB_ACT_SIGMOID, HB_ACT_TANH, HB_EPI_ACT_BWD,
-                    HB_EPI_ATOMIC_ADD, HB_EPI_BIAS, HB_EPI_BIAS_ACT, HB_GEMM_3XTF32, HB_GEMM_TF32, PPO_NUM_ACTIONS)
+                    HB_EPI_ATOMIC_ADD, HB_EPI_BIAS, HB_EPI_BIAS_ACT, HB_GEMM_3XTF32, HB_GEMM_TF32, PPO_MAX_ACTIONS,
+                    PPO_MAX_FUSED_ACTIONS)
 
 # the names get_activation resolves (algo/ppo/actor_critic.py), "crelu" being nn.ReLU there too
 ACTIVATIONS = {"elu": HB_ACT_ELU, "selu": HB_ACT_SELU, "relu": HB_ACT_RELU, "crelu": HB_ACT_RELU, "lrelu": HB_ACT_LRELU,
@@ -87,8 +88,8 @@ class ActorCritic:
             raise ValueError("precision must be 'tf32' or '3xtf32'")
         if kwargs:
             print("ActorCritic.__init__ got unexpected arguments, which will be ignored: " + str(list(kwargs)))
-        if num_actions not in PPO_NUM_ACTIONS:
-            raise ValueError(f"the loss-head kernels are built for {PPO_NUM_ACTIONS} actions (hector, XBot-L, hector_full)")
+        if not 1 <= num_actions <= PPO_MAX_ACTIONS:
+            raise ValueError(f"num_actions = {num_actions}: the PPO head kernels take 1 to {PPO_MAX_ACTIONS} actions")
         activation = "elu" if activation is None else activation
         if activation not in ACTIVATIONS:
             raise ValueError(f"unknown activation {activation!r}: one of {sorted(ACTIVATIONS)}")
@@ -227,7 +228,7 @@ class ActorCritic:
     def fused_head(self) -> bool:
         """Both last hidden layers are 128 wide (and at most 15 actions): the update path evaluates the output layers inside
         the loss kernel (hb_ppo_head_fused) instead of as 128-row tensor-core tiles with 10 / 1 useful columns."""
-        return all(L.fan_in == 128 for L in self.output_layers) and self.num_actions <= 15
+        return all(L.fan_in == 128 for L in self.output_layers) and self.num_actions <= PPO_MAX_FUSED_ACTIONS
 
     def _fwd_desc(self, net: str, i: int, a: torch.Tensor, ws: dict):
         """Forward GEMM of layer i of `net` on a [m, ld] (ld % 4 == 0, only the first fan_in columns are read), bias and (hidden

@@ -8,26 +8,32 @@
 
 namespace {
 
-// The kernels below are templated on the number of actions NA: 10 (hector), 12 (XBot-L), 18 (hector_full); a sample's
-// record is 3 NA + 6 floats.  HB_PPO_DISPATCH picks the instantiation.
-#define HB_PPO_DISPATCH(na, CALL)                                                        \
+// The PPO head kernels are templated on the number of actions NA.  10 (hector), 12 (XBot-L) and 18 (hector_full) are
+// compiled for their count; every other count runs the NA_RUNTIME instantiation, which takes it as a kernel argument
+// (loss_head_kernel: LossCoefs::num_actions).  A sample's record is 3 NA + 6 floats.  HB_PPO_DISPATCH picks the
+// instantiation, HB_PPO_FUSED_DISPATCH that of the fused heads.  Each entry point first checks 1 <= na <= max with
+// HB_PPO_CHECK_ACTIONS: below 1 is HB_ERR_BAD_ARG, above the limit HB_ERR_UNSUPPORTED, and `msg` (printf format, one %d
+// for the count) names the range.
+constexpr int NA_RUNTIME = 0;
+constexpr int MAX_ACTIONS = 64;
+constexpr int MAX_FUSED_ACTIONS = 15;       // one lane pair per action and one for the value in a 16-value butterfly
+#define HB_PPO_CHECK_ACTIONS(na, max, msg)                                                \
+    if ((na) < 1 || (na) > (max)) {                                                       \
+        hb::set_error(msg, (int)(na));                                                    \
+        return (na) < 1 ? HB_ERR_BAD_ARG : HB_ERR_UNSUPPORTED;                            \
+    }
+#define HB_PPO_DISPATCH(na, CALL)                                                         \
     switch (na) {                                                                         \
         case 10: { constexpr int NA = 10; CALL; break; }                                  \
         case 12: { constexpr int NA = 12; CALL; break; }                                  \
         case 18: { constexpr int NA = 18; CALL; break; }                                  \
-        default:                                                                          \
-            hb::set_error("num_actions = %d: built for 10 (hector), 12 (XBot-L), 18 (hector_full)", (int)(na)); \
-            return HB_ERR_UNSUPPORTED;                                                    \
+        default: { constexpr int NA = NA_RUNTIME; CALL; break; }                          \
     }
-// The fused heads put one lane pair on each output, so they take at most 15 actions: HB_PPO_FUSED_DISPATCH builds 10 and 12
-// only; `msg` (printf format, one %d for the width) reports any other width.
-#define HB_PPO_FUSED_DISPATCH(na, CALL, msg)                                              \
+#define HB_PPO_FUSED_DISPATCH(na, CALL)                                                   \
     switch (na) {                                                                         \
         case 10: { constexpr int NA = 10; CALL; break; }                                  \
         case 12: { constexpr int NA = 12; CALL; break; }                                  \
-        default:                                                                          \
-            hb::set_error(msg, (int)(na));                                                \
-            return HB_ERR_UNSUPPORTED;                                                    \
+        default: { constexpr int NA = NA_RUNTIME; CALL; break; }                          \
     }
 constexpr float HALF_LOG_2PI = 0.91893853320467274178f;     // log(sqrt(2*pi))
 
@@ -66,20 +72,21 @@ __global__ void __launch_bounds__(256)
 pack_samples_kernel(const int64_t *__restrict__ perm, long long rows, const float *__restrict__ actions,
                     const float *__restrict__ mu, const float *__restrict__ sigma, const float *__restrict__ values,
                     const float *__restrict__ adv, const float *__restrict__ ret, const float *__restrict__ logp,
-                    float *__restrict__ rec) {
+                    float *__restrict__ rec, int num_actions) {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= rows) return;
-    constexpr int REC = 3 * NA + 6;
+    const int na = NA != NA_RUNTIME ? NA : num_actions;
+    const int REC = 3 * na + 6;
     const long long j = perm[i];
     float *r = rec + i * REC;
 #pragma unroll
-    for (int k = 0; k < NA; ++k) {
-        r[k] = actions[j * NA + k];
-        r[NA + k] = mu[j * NA + k];
-        r[2 * NA + k] = sigma[j * NA + k];
+    for (int k = 0; k < na; ++k) {
+        r[k] = actions[j * na + k];
+        r[na + k] = mu[j * na + k];
+        r[2 * na + k] = sigma[j * na + k];
     }
-    r[3 * NA] = values[j], r[3 * NA + 1] = adv[j], r[3 * NA + 2] = ret[j], r[3 * NA + 3] = logp[j];
-    r[3 * NA + 4] = 0.0f, r[3 * NA + 5] = 0.0f;
+    r[3 * na] = values[j], r[3 * na + 1] = adv[j], r[3 * na + 2] = ret[j], r[3 * na + 3] = logp[j];
+    r[3 * na + 4] = 0.0f, r[3 * na + 5] = 0.0f;
 }
 
 __device__ __forceinline__ double warp_sum(double v) {
@@ -195,6 +202,100 @@ loss_head_kernel(const float *__restrict__ mu, int ld_mu, const float *__restric
     }
 }
 
+// The same loss head for any count up to MAX_ACTIONS (lp.num_actions).  The three per-action arrays of the template
+// above would take 3 x 64 registers a thread at 64 actions, so nothing is kept per action here: sigma sits in shared
+// memory, the second pass re-reads the record and mu for (action - mu), and each action's std gradient is summed over
+// the warp as soon as it is formed.  Same arithmetic, summed over the actions in the same order.
+template <>
+__global__ void __launch_bounds__(256)
+loss_head_kernel<NA_RUNTIME>(const float *__restrict__ mu, int ld_mu, const float *__restrict__ value, int ld_v,
+                             const float *__restrict__ stdp, const float *__restrict__ rec, long long mb, double inv_b,
+                             float ent_scale, LossCoefs lp, float *__restrict__ d_mu, float *__restrict__ d_value,
+                             float *__restrict__ d_std, double *__restrict__ stats) {
+    __shared__ float s_sig[MAX_ACTIONS];
+    __shared__ float s_dstd[8][MAX_ACTIONS];
+    __shared__ double s_stat[8][4];
+    const int na = lp.num_actions;
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    if (threadIdx.x < na) s_sig[threadIdx.x] = stdp[threadIdx.x];
+    __syncthreads();
+    const bool live = i < mb;
+    const float *r = rec + i * (3 * na + 6);
+    const float *m = mu + i * ld_mu;
+    float g_lp = 0.0f;
+    double st_s = 0.0, st_v = 0.0, st_k = 0.0, st_e = 0.0;
+    if (live) {
+        float lp_new = 0.0f, kl = 0.0f, ent = 0.0f;
+        for (int j = 0; j < na; ++j) {
+            const float sg = s_sig[j], var = sg * sg;
+            const float diff = r[j] - m[j];
+            lp_new += (-(diff * diff) / (2.0f * var) - logf(sg)) - HALF_LOG_2PI;                    // Normal.log_prob
+            const float so = r[2 * na + j], dm = r[na + j] - m[j];
+            kl += (logf(sg / so + 1.e-5f) + (so * so + dm * dm) / (2.0f * var)) - 0.5f;            // ppo.py:138-139
+            ent += (0.5f + HALF_LOG_2PI) + logf(sg);                                                // Normal.entropy
+        }
+        const float v_old = r[3 * na], adv = r[3 * na + 1], ret = r[3 * na + 2], lp_old = r[3 * na + 3];
+        // clipped surrogate (ppo.py:152-156); torch.max splits the gradient evenly on ties
+        const float ratio = expf(lp_new - lp_old);
+        const float lo = 1.0f - lp.clip_param, hi = 1.0f + lp.clip_param;
+        const float s1 = -adv * ratio, s2 = -adv * fminf(fmaxf(ratio, lo), hi);
+        const float inr = (ratio >= lo && ratio <= hi) ? 1.0f : 0.0f;
+        const float w1 = s1 > s2 ? 1.0f : (s1 == s2 ? 0.5f : 0.0f);
+        const float g_ratio = -adv * (w1 + (1.0f - w1) * inr);
+        g_lp = (float)((double)(g_ratio * ratio) * inv_b);
+        st_s = (double)fmaxf(s1, s2);
+        // value loss (ppo.py:158-166)
+        const float v = value[i * ld_v];
+        float g_v;
+        if (lp.use_clipped_value_loss) {
+            const float dv = v - v_old;
+            const float vc = v_old + fminf(fmaxf(dv, -lp.clip_param), lp.clip_param);
+            const float l1 = (v - ret) * (v - ret), l2 = (vc - ret) * (vc - ret);
+            const float inv = (dv >= -lp.clip_param && dv <= lp.clip_param) ? 1.0f : 0.0f;
+            const float u1 = l1 > l2 ? 1.0f : (l1 == l2 ? 0.5f : 0.0f);
+            g_v = 2.0f * (v - ret) * u1 + 2.0f * (vc - ret) * inv * (1.0f - u1);
+            st_v = (double)fmaxf(l1, l2);
+        } else {
+            g_v = -2.0f * (ret - v);
+            st_v = (double)((ret - v) * (ret - v));
+        }
+        st_k = (double)kl, st_e = (double)ent;
+        float *dv_out = d_value + i * ld_v;
+        dv_out[0] = (float)((double)(lp.value_loss_coef * g_v) * inv_b);
+        for (int j = 1; j < ld_v; ++j) dv_out[j] = 0.0f;
+    }
+    float *dm_out = d_mu + i * ld_mu;
+    for (int j = 0; j < na; ++j) {                  // every lane takes part in the warp sums, rows past mb with 0
+        float g_std = 0.0f;
+        if (live) {
+            const float sg = s_sig[j], var = sg * sg;
+            const float diff = r[j] - m[j];
+            dm_out[j] = g_lp * (diff / var);
+            g_std = g_lp * ((diff * diff) / (var * sg) - 1.0f / sg);
+        }
+        g_std = warp_sum(g_std);
+        if (lane == 0) s_dstd[warp][j] = g_std;
+    }
+    if (live)
+        for (int j = na; j < ld_mu; ++j) dm_out[j] = 0.0f;
+    st_s = warp_sum(st_s), st_v = warp_sum(st_v), st_k = warp_sum(st_k), st_e = warp_sum(st_e);
+    if (lane == 0) s_stat[warp][0] = st_s, s_stat[warp][1] = st_v, s_stat[warp][2] = st_k, s_stat[warp][3] = st_e;
+    __syncthreads();
+    if (threadIdx.x < na) {
+        float s = 0.0f;
+        for (int w = 0; w < 8; ++w) s += s_dstd[w][threadIdx.x];
+        // entropy bonus, added once by block 0 (see loss_head_kernel)
+        if (blockIdx.x == 0) s += ent_scale * (-lp.entropy_coef / s_sig[threadIdx.x]);
+        atomicAdd(d_std + threadIdx.x, s);
+    } else if (threadIdx.x >= MAX_ACTIONS && threadIdx.x < MAX_ACTIONS + 4) {
+        const int k = threadIdx.x - MAX_ACTIONS;
+        double s = 0.0;
+        for (int w = 0; w < 8; ++w) s += s_stat[w][k];
+        atomicAdd(stats + k, s);
+    }
+}
+
 // ------------------------------------------------------------------------------------------------------------
 // Fused output layers + loss head (update path).  The last nn.Linear of both MLPs is 128 -> 10 / 128 -> 1:
 // 1 290 + 129 MACs per sample, far too thin for a 128-row tensor-core tile, and it sits between the last hidden
@@ -235,32 +336,34 @@ head_fused_kernel(const float *__restrict__ h3a, int ld_ha, const float *__restr
                   const float *__restrict__ rec, long long mb, double inv_b, float ent_scale, LossCoefs lp,
                   float *__restrict__ dz3a, float *__restrict__ dz3c, int ld_dz, float *__restrict__ g4a,
                   float *__restrict__ g4c, float *__restrict__ d_std, double *__restrict__ stats) {
-    constexpr int HEAD_OUT = NA + 1;         // NA action means + 1 value: one lane pair each (NA <= 15)
-    static_assert(HEAD_OUT <= 16, "the 16-value butterfly holds at most 15 actions and the value");
-    __shared__ __align__(16) float s_w[HEAD_OUT * HID];    // output-layer weights, row j = action j, row NA = value
-    __shared__ float s_g[HEAD_OUT * (HID + 1)];            // CTA-level weight/bias gradient accumulators
-    __shared__ float s_dstd[NA];
+    constexpr int NB = NA != NA_RUNTIME ? NA : MAX_FUSED_ACTIONS;     // bound of the per-action arrays and loops
+    static_assert(NB + 1 <= 16, "the 16-value butterfly holds at most 15 actions and the value");
+    const int na = NA != NA_RUNTIME ? NA : lp.num_actions;         // na action means + 1 value: one lane pair each
+    __shared__ __align__(16) float s_w[(NB + 1) * HID];    // output-layer weights, row j = action j, row na = value
+    __shared__ float s_g[(NB + 1) * (HID + 1)];            // CTA-level weight/bias gradient accumulators
+    __shared__ float s_dstd[NB];
     __shared__ double s_stat[4];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    for (int i = threadIdx.x; i < HEAD_OUT * HID; i += HEAD_THREADS) {
+    for (int i = threadIdx.x; i < (na + 1) * HID; i += HEAD_THREADS) {
         const int j = i / HID, k = i - j * HID;
-        s_w[i] = (j < NA) ? w4a[(size_t)j * ld_w + k] : w4c[k];
+        s_w[i] = (j < na) ? w4a[(size_t)j * ld_w + k] : w4c[k];
     }
-    for (int i = threadIdx.x; i < HEAD_OUT * (HID + 1); i += HEAD_THREADS) s_g[i] = 0.0f;
-    if (threadIdx.x < NA) s_dstd[threadIdx.x] = 0.0f;
+    for (int i = threadIdx.x; i < (na + 1) * (HID + 1); i += HEAD_THREADS) s_g[i] = 0.0f;
+    if (threadIdx.x < na) s_dstd[threadIdx.x] = 0.0f;
     if (threadIdx.x < 4) s_stat[threadIdx.x] = 0.0;
-    // After the butterfly, output `o` of a row lives on lanes 2o, 2o+1: lane pair o < 10 owns action o, pair 10 the value.
+    // After the butterfly, output `o` of a row lives on lanes 2o, 2o+1: lane pair o < na owns action o, pair na the value,
+    // and the pairs past it idle.
     const int o = lane >> 1;
-    const bool own_action = o < NA, even = (lane & 1) == 0;
-    const float bias = (o < NA) ? w4a[(size_t)o * ld_w + HID] : (o == NA ? w4c[HID] : 0.0f);
+    const bool own_action = o < na, even = (lane & 1) == 0;
+    const float bias = (o < na) ? w4a[(size_t)o * ld_w + HID] : (o == na ? w4c[HID] : 0.0f);
     // row-invariant pieces of the loss for this lane's action (ppo.py:130-168)
     const float sg = own_action ? stdp[o] : 1.0f;
     const float var = sg * sg, log_sg = logf(sg);
     const float inv_2var = 1.0f / (2.0f * var), inv_var = 1.0f / var, inv_var_sg = 1.0f / (var * sg), inv_sg = 1.0f / sg;
     const float inv_bf = (float)inv_b;
-    float ga[NA][4], gc[4], gb = 0.0f, gstd = 0.0f;        // weight grads of this lane's 4 columns; bias / std grad of output o
+    float ga[NB][4], gc[4], gb = 0.0f, gstd = 0.0f;        // weight grads of this lane's 4 columns; bias / std grad of output o
 #pragma unroll
-    for (int j = 0; j < NA; ++j) ga[j][0] = ga[j][1] = ga[j][2] = ga[j][3] = 0.0f;
+    for (int j = 0; j < NB; ++j) ga[j][0] = ga[j][1] = ga[j][2] = ga[j][3] = 0.0f;
     gc[0] = gc[1] = gc[2] = gc[3] = 0.0f;
     float stf[4] = {0.0f, 0.0f, 0.0f, 0.0f};
     __syncthreads();
@@ -277,10 +380,10 @@ head_fused_kernel(const float *__restrict__ h3a, int ld_ha, const float *__restr
         RowIn in;
         in.ha = hb::ld_stream4(reinterpret_cast<const float4 *>(h3a + (size_t)rw * ld_ha) + lane);
         in.hc = hb::ld_stream4(reinterpret_cast<const float4 *>(h3c + (size_t)rw * ld_hc) + lane);
-        const float *r = rec + rw * (3 * NA + 6);
-        in.act = own_action ? __ldg(r + o) : 0.0f, in.mu = own_action ? __ldg(r + NA + o) : 0.0f;
-        in.sig = own_action ? __ldg(r + 2 * NA + o) : 1.0f;
-        in.v_old = __ldg(r + 3 * NA), in.adv = __ldg(r + 3 * NA + 1), in.ret = __ldg(r + 3 * NA + 2), in.lp_old = __ldg(r + 3 * NA + 3);
+        const float *r = rec + rw * (3 * na + 6);
+        in.act = own_action ? __ldg(r + o) : 0.0f, in.mu = own_action ? __ldg(r + na + o) : 0.0f;
+        in.sig = own_action ? __ldg(r + 2 * na + o) : 1.0f;
+        in.v_old = __ldg(r + 3 * na), in.adv = __ldg(r + 3 * na + 1), in.ret = __ldg(r + 3 * na + 2), in.lp_old = __ldg(r + 3 * na + 3);
         return in;
     };
     RowIn nxt_in = {};
@@ -294,18 +397,19 @@ head_fused_kernel(const float *__restrict__ h3a, int ld_ha, const float *__restr
         // ---- output layers: partial dot products over this lane's 4 features, then the 16-shuffle reduction ----
         float part[16];
 #pragma unroll
-        for (int j = 0; j < NA; ++j) {
-            const float4 w = w4[j * (HID / 4) + lane];
-            part[j] = ((ha[0] * w.x + ha[1] * w.y) + ha[2] * w.z) + ha[3] * w.w;
+        for (int j = 0; j < 16; ++j) {
+            if (j < na) {
+                const float4 w = w4[j * (HID / 4) + lane];
+                part[j] = ((ha[0] * w.x + ha[1] * w.y) + ha[2] * w.z) + ha[3] * w.w;
+            } else if (j == na) {
+                const float4 w = w4[j * (HID / 4) + lane];
+                part[j] = ((hc[0] * w.x + hc[1] * w.y) + hc[2] * w.z) + hc[3] * w.w;
+            } else {
+                part[j] = 0.0f;
+            }
         }
-        {
-            const float4 w = w4[NA * (HID / 4) + lane];
-            part[NA] = ((hc[0] * w.x + hc[1] * w.y) + hc[2] * w.z) + hc[3] * w.w;
-        }
-#pragma unroll
-        for (int j = HEAD_OUT; j < 16; ++j) part[j] = 0.0f;
-        const float out = warp_reduce16(part, lane) + bias;               // mu_o on pair o < 10, value on pair 10
-        const float v = __shfl_sync(0xffffffffu, out, 2 * NA);
+        const float out = warp_reduce16(part, lane) + bias;               // mu_o on pair o < na, value on pair na
+        const float v = __shfl_sync(0xffffffffu, out, 2 * na);
         // ---- loss head (same arithmetic as loss_head_kernel), the per-action part on the lane pair of the action ----
         const float diff = r_act - out, dm = r_mu - out;
         float lp_j = 0.0f, kl_j = 0.0f, ent_j = 0.0f;
@@ -315,10 +419,11 @@ head_fused_kernel(const float *__restrict__ h3a, int ld_ha, const float *__restr
             kl_j = (logf(sg / r_sig + 1.e-5f) + (r_sig * r_sig + dm * dm) * inv_2var) - 0.5f;               // ppo.py:138-139
             ent_j = (0.5f + HALF_LOG_2PI) + log_sg;                                                           // Normal.entropy
         }
-        // sum over the actions in the reference's order (j = 0..9) so that the result matches loss_head_kernel
+        // sum over the actions in the reference's order (j = 0..na-1) so that the result matches loss_head_kernel; the
+        // idle pairs past na (NB > na) add exact zeros
         float lp_new = 0.0f, kl = 0.0f, ent = 0.0f;
 #pragma unroll
-        for (int j = 0; j < NA; ++j) {
+        for (int j = 0; j < NB; ++j) {
             lp_new += __shfl_sync(0xffffffffu, lp_j, 2 * j);
             kl += __shfl_sync(0xffffffffu, kl_j, 2 * j);
             ent += __shfl_sync(0xffffffffu, ent_j, 2 * j);
@@ -344,22 +449,24 @@ head_fused_kernel(const float *__restrict__ h3a, int ld_ha, const float *__restr
             st_v = (ret - v) * (ret - v);
         }
         g_v = (lp.value_loss_coef * g_v) * inv_bf;
-        // gradient w.r.t. this lane's output: d_mu_o on the action pairs, d_value on pair 10
-        const float g_out = own_action ? g_lp * (diff * inv_var) : (o == NA ? g_v : 0.0f);
+        // gradient w.r.t. this lane's output: d_mu_o on the action pairs, d_value on pair na
+        const float g_out = own_action ? g_lp * (diff * inv_var) : (o == na ? g_v : 0.0f);
         if (own_action && even) gstd += g_lp * ((diff * diff) * inv_var_sg - inv_sg);
         if (even) gb += g_out;
         stf[0] += fmaxf(s1, s2), stf[1] += st_v, stf[2] += kl, stf[3] += ent;       // a warp sees a few dozen rows: fp32 is enough here
         // ---- data gradient through the last activation (f'(z) from h = f(z)) and weight gradients ----
         float da[4] = {0.f, 0.f, 0.f, 0.f};
 #pragma unroll
-        for (int j = 0; j < NA; ++j) {
-            const float gm = __shfl_sync(0xffffffffu, g_out, 2 * j);
-            const float4 w = w4[j * (HID / 4) + lane];
-            da[0] += gm * w.x, da[1] += gm * w.y, da[2] += gm * w.z, da[3] += gm * w.w;
+        for (int j = 0; j < NB; ++j) {
+            if (j < na) {
+                const float gm = __shfl_sync(0xffffffffu, g_out, 2 * j);
+                const float4 w = w4[j * (HID / 4) + lane];
+                da[0] += gm * w.x, da[1] += gm * w.y, da[2] += gm * w.z, da[3] += gm * w.w;
 #pragma unroll
-            for (int i = 0; i < 4; ++i) ga[j][i] += gm * ha[i];
+                for (int i = 0; i < 4; ++i) ga[j][i] += gm * ha[i];
+            }
         }
-        const float4 wc = w4[NA * (HID / 4) + lane];
+        const float4 wc = w4[na * (HID / 4) + lane];
         const float wcv[4] = {wc.x, wc.y, wc.z, wc.w};
         float dc[4];
 #pragma unroll
@@ -373,24 +480,25 @@ head_fused_kernel(const float *__restrict__ h3a, int ld_ha, const float *__restr
     }
     // CTA reduction in shared memory, then one atomic per parameter and CTA
 #pragma unroll
-    for (int j = 0; j < NA; ++j)
+    for (int j = 0; j < NB; ++j)
+        if (j < na)
 #pragma unroll
-        for (int i = 0; i < 4; ++i) atomicAdd(&s_g[j * (HID + 1) + lane * 4 + i], ga[j][i]);
+            for (int i = 0; i < 4; ++i) atomicAdd(&s_g[j * (HID + 1) + lane * 4 + i], ga[j][i]);
 #pragma unroll
-    for (int i = 0; i < 4; ++i) atomicAdd(&s_g[NA * (HID + 1) + lane * 4 + i], gc[i]);
-    if (even && o <= NA) atomicAdd(&s_g[o * (HID + 1) + HID], gb);
+    for (int i = 0; i < 4; ++i) atomicAdd(&s_g[na * (HID + 1) + lane * 4 + i], gc[i]);
+    if (even && o <= na) atomicAdd(&s_g[o * (HID + 1) + HID], gb);
     if (even && own_action) atomicAdd(&s_dstd[o], gstd);
     if (lane == 0) {
 #pragma unroll
         for (int k = 0; k < 4; ++k) atomicAdd(&s_stat[k], (double)stf[k]);
     }
     __syncthreads();
-    for (int i = threadIdx.x; i < HEAD_OUT * (HID + 1); i += HEAD_THREADS) {
+    for (int i = threadIdx.x; i < (na + 1) * (HID + 1); i += HEAD_THREADS) {
         const int j = i / (HID + 1), k = i - j * (HID + 1);
-        float *dst = (j < NA) ? g4a + (size_t)j * ld_w + k : g4c + k;
+        float *dst = (j < na) ? g4a + (size_t)j * ld_w + k : g4c + k;
         atomicAdd(dst, s_g[i]);
     }
-    if (threadIdx.x < NA) {
+    if (threadIdx.x < na) {
         float sacc = s_dstd[threadIdx.x];
         // entropy bonus: -entropy_coef * mean(entropy) -> d/dsigma_j = -coef / sigma_j (added once, by block 0)
         if (blockIdx.x == 0) sacc += ent_scale * (-lp.entropy_coef / stdp[threadIdx.x]);
@@ -411,18 +519,19 @@ __global__ void __launch_bounds__(256)
 act_fused_kernel(const float *__restrict__ h3a, int ld_ha, const float *__restrict__ h3c, int ld_hc,
                  const float *__restrict__ w4a, const float *__restrict__ w4c, int ld_w, const float *__restrict__ stdp,
                  const float *__restrict__ eps, long long n, float *__restrict__ actions, float *__restrict__ logp,
-                 float *__restrict__ mu_out, float *__restrict__ sigma_out, float *__restrict__ values) {
-    constexpr int HEAD_OUT = NA + 1;
-    static_assert(HEAD_OUT <= 16, "the 16-value butterfly holds at most 15 actions and the value");
-    __shared__ __align__(16) float s_w[HEAD_OUT * HID];
+                 float *__restrict__ mu_out, float *__restrict__ sigma_out, float *__restrict__ values, int num_actions) {
+    constexpr int NB = NA != NA_RUNTIME ? NA : MAX_FUSED_ACTIONS;
+    static_assert(NB + 1 <= 16, "the 16-value butterfly holds at most 15 actions and the value");
+    const int na = NA != NA_RUNTIME ? NA : num_actions;
+    __shared__ __align__(16) float s_w[(NB + 1) * HID];
     const int lane = threadIdx.x & 31;
-    for (int i = threadIdx.x; i < HEAD_OUT * HID; i += blockDim.x) {
+    for (int i = threadIdx.x; i < (na + 1) * HID; i += blockDim.x) {
         const int j = i / HID, k = i - j * HID;
-        s_w[i] = (j < NA) ? w4a[(size_t)j * ld_w + k] : w4c[k];
+        s_w[i] = (j < na) ? w4a[(size_t)j * ld_w + k] : w4c[k];
     }
     const int o = lane >> 1;
-    const bool own_action = o < NA;
-    const float bias = (o < NA) ? w4a[(size_t)o * ld_w + HID] : (o == NA ? w4c[HID] : 0.0f);
+    const bool own_action = o < na;
+    const float bias = (o < na) ? w4a[(size_t)o * ld_w + HID] : (o == na ? w4c[HID] : 0.0f);
     const float sg = own_action ? stdp[o] : 1.0f;
     __syncthreads();
     const float4 *w4 = reinterpret_cast<const float4 *>(s_w);
@@ -430,19 +539,20 @@ act_fused_kernel(const float *__restrict__ h3a, int ld_ha, const float *__restri
     for (long long row = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); row < n; row += warps) {
         const float4 ha = hb::ld_stream4(reinterpret_cast<const float4 *>(h3a + (size_t)row * ld_ha) + lane);
         const float4 hc = hb::ld_stream4(reinterpret_cast<const float4 *>(h3c + (size_t)row * ld_hc) + lane);
-        const float e = own_action ? __ldg(eps + row * NA + o) : 0.0f;
+        const float e = own_action ? __ldg(eps + row * na + o) : 0.0f;
         float part[16];
 #pragma unroll
-        for (int j = 0; j < NA; ++j) {
-            const float4 w = w4[j * (HID / 4) + lane];
-            part[j] = ((ha.x * w.x + ha.y * w.y) + ha.z * w.z) + ha.w * w.w;
+        for (int j = 0; j < 16; ++j) {
+            if (j < na) {
+                const float4 w = w4[j * (HID / 4) + lane];
+                part[j] = ((ha.x * w.x + ha.y * w.y) + ha.z * w.z) + ha.w * w.w;
+            } else if (j == na) {
+                const float4 w = w4[j * (HID / 4) + lane];
+                part[j] = ((hc.x * w.x + hc.y * w.y) + hc.z * w.z) + hc.w * w.w;
+            } else {
+                part[j] = 0.0f;
+            }
         }
-        {
-            const float4 w = w4[NA * (HID / 4) + lane];
-            part[NA] = ((hc.x * w.x + hc.y * w.y) + hc.z * w.z) + hc.w * w.w;
-        }
-#pragma unroll
-        for (int j = HEAD_OUT; j < 16; ++j) part[j] = 0.0f;
         const float out = warp_reduce16(part, lane) + bias;
         const float sgm = out * 0.0f + sg;                              // actor_critic.py:113
         const float act = out + sgm * e;                                // Normal.sample with the draw supplied
@@ -450,11 +560,11 @@ act_fused_kernel(const float *__restrict__ h3a, int ld_ha, const float *__restri
         const float lp_j = own_action ? (-(d * d) / (2.0f * (sgm * sgm)) - logf(sgm)) - HALF_LOG_2PI : 0.0f;
         float lp = 0.0f;
 #pragma unroll
-        for (int j = 0; j < NA; ++j) lp += __shfl_sync(0xffffffffu, lp_j, 2 * j);
+        for (int j = 0; j < NB; ++j) lp += __shfl_sync(0xffffffffu, lp_j, 2 * j);      // pairs past na add exact zeros
         if ((lane & 1) == 0) {
             if (own_action) {
-                actions[row * NA + o] = act, mu_out[row * NA + o] = out, sigma_out[row * NA + o] = sgm;
-            } else if (o == NA) {
+                actions[row * na + o] = act, mu_out[row * na + o] = out, sigma_out[row * na + o] = sgm;
+            } else if (o == na) {
                 values[row] = out;
             }
         }
@@ -480,18 +590,19 @@ template <int NA>
 __global__ void __launch_bounds__(256)
 act_head_kernel(const float *__restrict__ mu, int ld_mu, const float *__restrict__ stdp, const float *__restrict__ eps,
                 long long n, float *__restrict__ actions, float *__restrict__ logp, float *__restrict__ mu_out,
-                float *__restrict__ sigma_out) {
+                float *__restrict__ sigma_out, int num_actions) {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
+    const int na = NA != NA_RUNTIME ? NA : num_actions;
     float lp = 0.0f;
 #pragma unroll
-    for (int j = 0; j < NA; ++j) {
+    for (int j = 0; j < na; ++j) {
         const float m = mu[i * ld_mu + j];
         const float s = m * 0.0f + stdp[j];                         // actor_critic.py:113
-        const float a = m + s * eps[i * NA + j];                    // Normal.sample with the draw supplied
+        const float a = m + s * eps[i * na + j];                    // Normal.sample with the draw supplied
         const float d = a - m;
         lp += (-(d * d) / (2.0f * (s * s)) - logf(s)) - HALF_LOG_2PI;
-        actions[i * NA + j] = a, mu_out[i * NA + j] = m, sigma_out[i * NA + j] = s;
+        actions[i * na + j] = a, mu_out[i * na + j] = m, sigma_out[i * na + j] = s;
     }
     logp[i] = lp;
 }
@@ -977,8 +1088,9 @@ int hb_ppo_pack_samples(const int64_t *perm, int64_t rows, const float *actions,
                         int32_t num_actions, float *records, void *stream) {
     HB_REQUIRE(perm && actions && mu && sigma && values && advantages && returns && log_prob && records && rows > 0,
                "hb_ppo_pack_samples: bad arguments");
+    HB_PPO_CHECK_ACTIONS(num_actions, MAX_ACTIONS, "hb_ppo_pack_samples: num_actions = %d (1 to 64)");
     HB_PPO_DISPATCH(num_actions, (pack_samples_kernel<NA><<<(unsigned)((rows + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
-        perm, rows, actions, mu, sigma, values, advantages, returns, log_prob, records)));
+        perm, rows, actions, mu, sigma, values, advantages, returns, log_prob, records, num_actions)));
     HB_CHECK_LAUNCH("pack_samples_kernel");
     return HB_OK;
 }
@@ -987,6 +1099,7 @@ int hb_ppo_loss_head(const float *mu, int32_t ld_mu, const float *value, int32_t
                      const float *records, int64_t mb, int64_t mb_global, const hb_ppo_loss_params *lp, float *d_mu,
                      float *d_value, float *d_std, double *stats, void *stream) {
     HB_REQUIRE(mu && value && std && records && lp && d_mu && d_value && d_std && stats, "hb_ppo_loss_head: null buffer");
+    HB_PPO_CHECK_ACTIONS(lp->num_actions, MAX_ACTIONS, "hb_ppo_loss_head: num_actions = %d (1 to 64)");
     HB_REQUIRE(mb > 0 && mb_global >= mb && ld_mu >= lp->num_actions && ld_v >= 1, "hb_ppo_loss_head: bad sizes");
     HB_PPO_DISPATCH(lp->num_actions, (loss_head_kernel<NA><<<(unsigned)((mb + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
         mu, ld_mu, value, ld_v, std, records, mb, 1.0 / (double)mb_global, (float)((double)mb / (double)mb_global), loss_coefs(*lp), d_mu,
@@ -1001,6 +1114,8 @@ int hb_ppo_head_fused(const float *h3_actor, int32_t ld_ha, const float *h3_crit
                       float *g4_actor, float *g4_critic, float *d_std, double *stats, void *stream) {
     HB_REQUIRE(h3_actor && h3_critic && w4_actor && w4_critic && std && records && lp && dz3_actor && dz3_critic &&
                    g4_actor && g4_critic && d_std && stats, "hb_ppo_head_fused: null buffer");
+    HB_PPO_CHECK_ACTIONS(lp->num_actions, MAX_FUSED_ACTIONS,
+                         "hb_ppo_head_fused: num_actions = %d (1 to 15; wider heads use hb_gemm_tf32 + hb_ppo_loss_head)");
     HB_REQUIRE(mb > 0 && mb_global >= mb, "hb_ppo_head_fused: bad sizes");
     HB_REQUIRE(ld_ha >= HID + 1 && ld_hc >= HID + 1 && ld_w >= HID + 1 && ld_dz >= HID && ld_ha % 4 == 0 && ld_hc % 4 == 0 &&
                    ld_w % 4 == 0 && ld_dz % 4 == 0,
@@ -1015,8 +1130,7 @@ int hb_ppo_head_fused(const float *h3_actor, int32_t ld_ha, const float *h3_crit
     const LossCoefs coefs = loss_coefs(*lp);
     HB_PPO_FUSED_DISPATCH(lp->num_actions, HB_ACT_DISPATCH(lp->activation, (head_fused_kernel<NA, ACT><<<grid, HEAD_THREADS, 0,
         (cudaStream_t)stream>>>(h3_actor, ld_ha, h3_critic, ld_hc, w4_actor, w4_critic, ld_w, std, records, mb, inv_b, ent_scale,
-        coefs, dz3_actor, dz3_critic, ld_dz, g4_actor, g4_critic, d_std, stats))),
-        "hb_ppo_head_fused: num_actions = %d (built for 10 and 12; wider heads use hb_gemm_tf32 + hb_ppo_loss_head)");
+        coefs, dz3_actor, dz3_critic, ld_dz, g4_actor, g4_critic, d_std, stats))));
     HB_CHECK_LAUNCH("head_fused_kernel");
     return HB_OK;
 }
@@ -1032,10 +1146,11 @@ int hb_ppo_draw_normal(float *out, int64_t count, uint64_t *state, void *stream)
 
 int hb_ppo_act_head(const float *mu, int32_t ld_mu, const float *std, const float *eps, int64_t n, int32_t num_actions,
                     float *actions, float *log_prob, float *mu_out, float *sigma_out, void *stream) {
+    HB_PPO_CHECK_ACTIONS(num_actions, MAX_ACTIONS, "hb_ppo_act_head: num_actions = %d (1 to 64)");
     HB_REQUIRE(mu && std && eps && actions && log_prob && mu_out && sigma_out && n > 0 && ld_mu >= num_actions,
                "hb_ppo_act_head: bad arguments");
     HB_PPO_DISPATCH(num_actions, (act_head_kernel<NA><<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
-        mu, ld_mu, std, eps, n, actions, log_prob, mu_out, sigma_out)));
+        mu, ld_mu, std, eps, n, actions, log_prob, mu_out, sigma_out, num_actions)));
     HB_CHECK_LAUNCH("act_head_kernel");
     return HB_OK;
 }
@@ -1045,6 +1160,8 @@ int hb_ppo_act_fused(const float *h3_actor, int32_t ld_ha, const float *h3_criti
                      float *actions, float *log_prob, float *mu_out, float *sigma_out, float *values, void *stream) {
     HB_REQUIRE(h3_actor && h3_critic && w4_actor && w4_critic && std && eps && actions && log_prob && mu_out && sigma_out &&
                    values && n > 0, "hb_ppo_act_fused: bad arguments");
+    HB_PPO_CHECK_ACTIONS(num_actions, MAX_FUSED_ACTIONS,
+                         "hb_ppo_act_fused: num_actions = %d (1 to 15; wider heads use hb_gemm_tf32 + hb_ppo_act_head)");
     HB_REQUIRE(ld_ha >= HID && ld_hc >= HID && ld_w >= HID + 1 && ld_ha % 4 == 0 && ld_hc % 4 == 0 && ld_w % 4 == 0,
                "hb_ppo_act_fused: rows of %d features, leading dimensions multiples of 4", HID);
     HB_REQUIRE(hb::aligned16(h3_actor) && hb::aligned16(h3_critic) && hb::aligned16(w4_actor) && hb::aligned16(w4_critic),
@@ -1053,8 +1170,8 @@ int hb_ppo_act_fused(const float *h3_actor, int32_t ld_ha, const float *h3_criti
     const long long cap = 8ll * hb::sm_count();
     const unsigned grid = (unsigned)(blocks < cap ? blocks : cap);
     HB_PPO_FUSED_DISPATCH(num_actions, (act_fused_kernel<NA><<<grid, 256, 0, (cudaStream_t)stream>>>(
-        h3_actor, ld_ha, h3_critic, ld_hc, w4_actor, w4_critic, ld_w, std, eps, n, actions, log_prob, mu_out, sigma_out, values)),
-        "hb_ppo_act_fused: num_actions = %d (built for 10 and 12)");
+        h3_actor, ld_ha, h3_critic, ld_hc, w4_actor, w4_critic, ld_w, std, eps, n, actions, log_prob, mu_out, sigma_out, values,
+        num_actions)));
     HB_CHECK_LAUNCH("act_fused_kernel");
     return HB_OK;
 }
