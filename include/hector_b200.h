@@ -221,7 +221,9 @@ void hb_launch_count_reset(void);
  * tail of its predecessor; griddepcontrol.wait guards the dependent data): 1 = all kernels, 0 = none, 2 or -1
  * (default) = only the PD-torque launches (measured on one box, 4096 envs: 52.0 us per step with the default, 52.7
  * with none, 60.4 with all; PD launches only: +5.6 % at 16384 envs, +2 % at 65536; all kernels: -13 % at 65536);
- * "gae_serial_min_envs" (default 8192): shards at least this wide run GAE one thread per env. */
+ * "gae_serial_min_envs" (default 8192): shards at least this wide run GAE one thread per env;
+ * "env_runtime_task" 0 (default) / 1: the built robots too run post-physics on the kernel that reads the layout at run
+ * time (for tests and A/B measurements). */
 /* "coop_launch" 0 (default) / 1: the two kernels that contain a grid barrier (hb_optimizer_step, hb_gae_fused) size their
  * grid to what the device holds at once; with 1 they are also launched with the cooperative attribute (the driver then
  * guarantees co-residency but serialises the launch against everything else on the device: measured 24.8 us against
@@ -269,7 +271,11 @@ int hb_env_prologue_torques(const hb_env_params *p, const hb_env_buffers *buf, c
  * last_* copies.  The newest frames are written (noise added, clipped) into the last frame slot of
  * obs_new / priv_new; hb_env_stack_observations fills the other slots.  Shard-wide results of
  * reset_idx (id list, count, episode means) are produced by hb_env_reset_finalize, which must
- * follow every call of this function. */
+ * follow every call of this function.
+ * The three built robots (hector 10 DOF 41/70, hector_full 18 DOF 65/94, XBot-L 12 DOF 47/73 with their joint pairs) run
+ * kernels compiled for their layout; any other layout of either task_kind runs the kernel that reads num_dof, yaw_roll,
+ * arm_pair, ref_left / ref_right from p: 1 to 23 joints (HB_ERR_UNSUPPORTED above), frames 3 num_dof + 11 and
+ * 3 num_dof + 40 (XBot: 4 num_dof + 25), every joint index inside the robot (HB_ERR_BAD_ARG otherwise). */
 int hb_env_post_physics(const hb_env_params *p, const hb_env_buffers *buf, const hb_env_noise *noise,
                         float *obs_new, float *priv_new, int32_t stages, void *stream);
 

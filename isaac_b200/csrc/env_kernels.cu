@@ -25,29 +25,68 @@ namespace {
 //                 friction | mass/30 | stance 2 | contact 2]                                        = 4 N + 25
 // The observation frame is [cmd 5 | q-q0 N | dq N | a N | ang 3 | euler 3] = 3 N + 11 for all of them.
 constexpr int KIND_HECTOR = 0, KIND_XBOT = 1;
+// Any other robot with the same env file runs the same kernel with its joint count and joint pairs read at run time
+// (RuntimeTask), up to MAX_TASK_DOF joints: an observation frame 3 N + 11 <= HB_MAX_OBS, so that its draws stay inside the
+// Philox slots below.
+constexpr int MAX_TASK_DOF = (HB_MAX_OBS - 11) / 3;
+
+// Column offsets of the frames and the joint pairs of default_joint_pos of a task with `ndof` joints
+struct TaskDims {
+    int NDOF, OBS, B0, B1, P_DIFF, P_LIN, P_ANG, P_EUL, P_FEET_POS, P_FEET_VEL, P_ROOT, P_PUSH_F, P_PUSH_T, P_FRICTION, P_MASS,
+        P_STANCE, P_CONTACT, PRIV, U_RESET, YAW_L, YAW_R, ARM_L, ARM_R;
+    bool HAS_ARMS;
+};
+__host__ __device__ constexpr TaskDims task_dims(int ndof, int kind, int yaw_l, int yaw_r, int arm_l, int arm_r) {
+    TaskDims d{};
+    d.NDOF = ndof;
+    d.OBS = 5 + 3 * ndof + 6;
+    d.B0 = 5 + 3 * ndof;                                 // end of the joint columns
+    d.B1 = kind == KIND_XBOT ? d.B0 + ndof : d.B0;       // start of the base-velocity columns
+    d.P_DIFF = d.B0;                                     // KIND_XBOT only
+    d.P_LIN = d.B1, d.P_ANG = d.B1 + 3, d.P_EUL = d.B1 + 6;
+    d.P_FEET_POS = d.B1 + 9, d.P_FEET_VEL = d.B1 + 15, d.P_ROOT = d.B1 + 21;      // KIND_HECTOR only
+    d.P_PUSH_F = kind == KIND_XBOT ? d.B1 + 9 : d.B1 + 24;
+    d.P_PUSH_T = d.P_PUSH_F + 2, d.P_FRICTION = d.P_PUSH_F + 5, d.P_MASS = d.P_PUSH_F + 6, d.P_STANCE = d.P_PUSH_F + 7;
+    d.P_CONTACT = d.P_PUSH_F + 9;
+    d.PRIV = d.P_CONTACT + 2;
+    d.U_RESET = ndof + 5;                                // dof offsets, root xy, command draws (legged_robot.py:366,384,327-330)
+    d.YAW_L = yaw_l, d.YAW_R = yaw_r, d.ARM_L = arm_l, d.ARM_R = arm_r;
+    d.HAS_ARMS = arm_l >= 0;
+    return d;
+}
+
 // OPT_: the optional reward terms (joint_pos with the reference trajectory, vel_mismatch_exp, track_vel_hard, low_speed:
 // zero-scale in hector_config.py) are compiled in.  A config that scales none of them runs the kernel without their code:
 // the four-role kernel is bound by instruction latency and its footprint (6.5 k SASS instructions with them, 5.5 k without).
+// The kernel reads a task's dimensions from `T::dims(p)`: this empty object, whose members are compile-time constants, or
+// RuntimeTask's TaskDims.  CAP sizes the per-lane joint arrays.
 template <int NDOF_, int KIND_, bool OPT_ = true>
 struct Task {
-    static constexpr int NDOF = NDOF_, KIND = KIND_;
+    static constexpr int NDOF = NDOF_, KIND = KIND_, CAP = NDOF_;
     static constexpr bool OPT = OPT_ || KIND_ == 1;                 // XBot-L always maintains the reference trajectory
+    static constexpr bool RUNTIME = false;
     // default_joint_pos (hector_env.py:357-367, hector_w_arm_env.py:371-378, humanoid_env.py:368-369): first joint of each
     // leg's (yaw, roll) pair and, with arms, of each arm's pair - joint-order constants of the three robots
-    static constexpr int YAW_L = 0, YAW_R = NDOF_ / 2;
     static constexpr bool HAS_ARMS = NDOF_ == 18;
-    static constexpr int ARM_L = HAS_ARMS ? 5 : -1, ARM_R = HAS_ARMS ? NDOF_ / 2 + 5 : -1;
-    static constexpr int OBS = 5 + 3 * NDOF + 6;
-    static constexpr int B0 = 5 + 3 * NDOF;                         // end of the joint columns
-    static constexpr int B1 = KIND == KIND_XBOT ? B0 + NDOF : B0;   // start of the base-velocity columns
-    static constexpr int P_DIFF = B0;                               // KIND_XBOT only
-    static constexpr int P_LIN = B1, P_ANG = B1 + 3, P_EUL = B1 + 6;
-    static constexpr int P_FEET_POS = B1 + 9, P_FEET_VEL = B1 + 15, P_ROOT = B1 + 21;       // KIND_HECTOR only
-    static constexpr int P_PUSH_F = KIND == KIND_XBOT ? B1 + 9 : B1 + 24;
-    static constexpr int P_PUSH_T = P_PUSH_F + 2, P_FRICTION = P_PUSH_F + 5, P_MASS = P_PUSH_F + 6, P_STANCE = P_PUSH_F + 7,
-                         P_CONTACT = P_PUSH_F + 9;
-    static constexpr int PRIV = P_CONTACT + 2;
-    static constexpr int U_RESET = NDOF + 5;                        // dof offsets, root xy, command draws (legged_robot.py:366,384,327-330)
+    static constexpr TaskDims d() {
+        return task_dims(NDOF_, KIND_, 0, NDOF_ / 2, HAS_ARMS ? 5 : -1, HAS_ARMS ? NDOF_ / 2 + 5 : -1);
+    }
+    static constexpr int YAW_L = d().YAW_L, YAW_R = d().YAW_R, ARM_L = d().ARM_L, ARM_R = d().ARM_R;
+    static constexpr int OBS = d().OBS, B0 = d().B0, B1 = d().B1, P_DIFF = d().P_DIFF, P_LIN = d().P_LIN, P_ANG = d().P_ANG,
+                         P_EUL = d().P_EUL, P_FEET_POS = d().P_FEET_POS, P_FEET_VEL = d().P_FEET_VEL, P_ROOT = d().P_ROOT,
+                         P_PUSH_F = d().P_PUSH_F, P_PUSH_T = d().P_PUSH_T, P_FRICTION = d().P_FRICTION, P_MASS = d().P_MASS,
+                         P_STANCE = d().P_STANCE, P_CONTACT = d().P_CONTACT, PRIV = d().PRIV, U_RESET = d().U_RESET;
+    __device__ static Task dims(const hb_env_params &) { return Task{}; }
+};
+// Any other robot of a kind: joint count and pairs read from hb_env_params (validated by the launcher), every optional
+// term compiled in
+template <int KIND_>
+struct RuntimeTask {
+    static constexpr int KIND = KIND_, CAP = MAX_TASK_DOF;
+    static constexpr bool OPT = true, RUNTIME = true;
+    __device__ static TaskDims dims(const hb_env_params &p) {
+        return task_dims(p.num_dof, KIND_, p.yaw_roll[0], p.yaw_roll[1], p.arm_pair[0], p.arm_pair[1]);
+    }
 };
 static_assert(Task<10, KIND_HECTOR>::OBS == 41 && Task<10, KIND_HECTOR>::PRIV == 70, "hector (hector_config.py:12-14)");
 static_assert(Task<18, KIND_HECTOR>::OBS == 65 && Task<18, KIND_HECTOR>::PRIV == 94, "hector_full (hector_w_arm_config.py:12-14)");
@@ -279,8 +318,8 @@ struct TileLayout {          // float offsets into the CTA's shared-memory tile
 // The staged inputs are dead once every role has passed barrier 1 (each lane keeps its env's values in
 // registers), so the newest-frame staging tiles so/sp reuse the same bytes: ~19 KB per CTA instead of
 // ~38 KB, which is what bounds the number of resident tiles per SM.
-__host__ __device__ inline TileLayout make_layout(int nbody, bool with_noise, int NDOF, int OBS, int PRIV) {
-    TileLayout L;
+__host__ __device__ constexpr TileLayout make_layout(int nbody, bool with_noise, int NDOF, int OBS, int PRIV) {
+    TileLayout L{};
     int o = 0;
     L.root = o, o += TILE * 13;
     L.dof = o, o += TILE * NDOF * 2;
@@ -304,6 +343,12 @@ __host__ __device__ inline TileLayout make_layout(int nbody, bool with_noise, in
     L.total = o;
     return L;
 }
+// dynamic shared memory the launcher allows post_physics_kernel: enough for the largest task (MAX_TASK_DOF joints, the longer
+// XBot-L privileged frame, 32 bodies, observation noise)
+constexpr int POST_SMEM_MAX = 96 * 1024;
+static_assert(make_layout(32, true, MAX_TASK_DOF, task_dims(MAX_TASK_DOF, KIND_XBOT, 0, 0, 0, 0).OBS,
+                          task_dims(MAX_TASK_DOF, KIND_XBOT, 0, 0, 0, 0).PRIV).total * 4 <= POST_SMEM_MAX,
+              "the largest task's tile fits the dynamic shared memory of post_physics_kernel");
 
 // all four warps of the tile (named barrier 1: the roles meet at different program points)
 __device__ __forceinline__ void tile_barrier() { asm volatile("bar.sync 1, 128;" ::: "memory"); }
@@ -358,11 +403,13 @@ __device__ __forceinline__ unsigned long long gtime() {
 #endif
 
 template <bool kBulk, typename T>
-__global__ void __launch_bounds__(4 * TILE, T::NDOF <= 12 ? 8 : 5)
+__global__ void __launch_bounds__(4 * TILE, T::RUNTIME ? 4 : (T::CAP <= 12 ? 8 : 5))
 post_physics_kernel(const __grid_constant__ hb_env_params p, const __grid_constant__ hb_env_buffers b,
                     const __grid_constant__ hb_env_noise nz, float *__restrict__ obs_new,
                     float *__restrict__ priv_new, int stages) {
-    constexpr int NDOF = T::NDOF, OBS = T::OBS, PRIV = T::PRIV, PRIV_PAD = T::PRIV, KIND = T::KIND, U_RESET = T::U_RESET;
+    constexpr int KIND = T::KIND, CAP = T::CAP;
+    const auto D = T::dims(p);      // (the three robots: every D.X below is a constant expression)
+    const int NDOF = D.NDOF, OBS = D.OBS, PRIV = D.PRIV, PRIV_PAD = D.PRIV, U_RESET = D.U_RESET;
     extern __shared__ __align__(128) float sm[];
     __shared__ __align__(8) uint64_t bar;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -603,7 +650,7 @@ post_physics_kernel(const __grid_constant__ hb_env_params p, const __grid_consta
             for (int k = 0; k < 4; ++k) b.commands[(size_t)env * 4 + k] = cmd[k];
         }
         if (emit_obs) {      // command input, base velocities, euler, root position, push (hector_env.py:186-226)
-            constexpr int B0 = T::B0;
+            const int B0 = D.B0;
             float o[11];
             o[0] = gs, o[1] = gc;
             o[2] = cmd[0] * p.obs_lin_vel, o[3] = cmd[1] * p.obs_lin_vel, o[4] = cmd[2] * p.obs_ang_vel;
@@ -616,20 +663,20 @@ post_physics_kernel(const __grid_constant__ hb_env_params p, const __grid_consta
             }
 #pragma unroll
             for (int k = 0; k < 6; ++k) {
-                sp[lane * PRIV_PAD + T::P_ANG + k] = clampf(o[5 + k], -clip, clip);
+                sp[lane * PRIV_PAD + D.P_ANG + k] = clampf(o[5 + k], -clip, clip);
                 so[lane * OBS + B0 + k] = noisy_clip(o[5 + k], B0 + k);
             }
-            sp[lane * PRIV_PAD + T::P_LIN] = clampf(lin.x * p.obs_lin_vel, -clip, clip);
-            sp[lane * PRIV_PAD + T::P_LIN + 1] = clampf(lin.y * p.obs_lin_vel, -clip, clip);
-            sp[lane * PRIV_PAD + T::P_LIN + 2] = clampf(lin.z * p.obs_lin_vel, -clip, clip);
+            sp[lane * PRIV_PAD + D.P_LIN] = clampf(lin.x * p.obs_lin_vel, -clip, clip);
+            sp[lane * PRIV_PAD + D.P_LIN + 1] = clampf(lin.y * p.obs_lin_vel, -clip, clip);
+            sp[lane * PRIV_PAD + D.P_LIN + 2] = clampf(lin.z * p.obs_lin_vel, -clip, clip);
             if (KIND == KIND_HECTOR) {
 #pragma unroll
-                for (int k = 0; k < 3; ++k) sp[lane * PRIV_PAD + T::P_ROOT + k] = clampf(root[k], -clip, clip);
+                for (int k = 0; k < 3; ++k) sp[lane * PRIV_PAD + D.P_ROOT + k] = clampf(root[k], -clip, clip);
             }
-            sp[lane * PRIV_PAD + T::P_PUSH_F] = clampf(push_f[0], -clip, clip);
-            sp[lane * PRIV_PAD + T::P_PUSH_F + 1] = clampf(push_f[1], -clip, clip);
+            sp[lane * PRIV_PAD + D.P_PUSH_F] = clampf(push_f[0], -clip, clip);
+            sp[lane * PRIV_PAD + D.P_PUSH_F + 1] = clampf(push_f[1], -clip, clip);
 #pragma unroll
-            for (int k = 0; k < 3; ++k) sp[lane * PRIV_PAD + T::P_PUSH_T + k] = clampf(push_t[k], -clip, clip);
+            for (int k = 0; k < 3; ++k) sp[lane * PRIV_PAD + D.P_PUSH_T + k] = clampf(push_t[k], -clip, clip);
         }
     } else if (warp == 1) {
         // ================================ joints ================================
@@ -643,9 +690,10 @@ post_physics_kernel(const __grid_constant__ hb_env_params p, const __grid_consta
         const bool use_ref = T::OPT && (KIND == KIND_XBOT || joint_pos_on) && b.ref_dof_pos != nullptr;
         long long ep_len = 0;
         if (use_ref && valid) ep_len = b.episode_length_buf[env] + (do_prepare ? 1 : 0);
-        float q[NDOF], qd[NDOF], act[NDOF];
+        float q[CAP], qd[CAP], act[CAP];
 #pragma unroll
-        for (int j = 0; j < NDOF; ++j) {
+        for (int j = 0; j < CAP; ++j) {
+            if (T::RUNTIME && j == NDOF) break;
             q[j] = sm[L.dof + ln * NDOF * 2 + 2 * j];
             qd[j] = sm[L.dof + ln * NDOF * 2 + 2 * j + 1];
             act[j] = sm[L.actions + ln * NDOF + j];
@@ -653,9 +701,10 @@ post_physics_kernel(const __grid_constant__ hb_env_params p, const __grid_consta
         if (do_rew || do_last) {
             float t1 = 0.f, t2 = 0.f, t3 = 0.f, ss = 0.f, acc = 0.f, vel = 0.f, tq = 0.f, rr = 0.f;
             float dy0 = 0.f, dy1 = 0.f, dy2 = 0.f, dy3 = 0.f, da0 = 0.f, da1 = 0.f, da2 = 0.f, da3 = 0.f;
-            constexpr int yl = T::YAW_L, yr_ = T::YAW_R, al = T::ARM_L, ar_ = T::ARM_R;      // (checked against p by the launcher)
+            const int yl = D.YAW_L, yr_ = D.YAW_R, al = D.ARM_L, ar_ = D.ARM_R;      // (checked against p by the launcher)
 #pragma unroll
-            for (int j = 0; j < NDOF; ++j) {
+            for (int j = 0; j < CAP; ++j) {
+                if (T::RUNTIME && j == NDOF) break;
                 const float lact = sm[L.last_actions + ln * NDOF + j];
                 const float llact = sm[L.last_last_actions + ln * NDOF + j];
                 const float ldv = sm[L.last_dof_vel + ln * NDOF + j];
@@ -671,7 +720,7 @@ post_physics_kernel(const __grid_constant__ hb_env_params p, const __grid_consta
                 // (j is a compile-time value in the unrolled loop: these are plain register copies)
                 dy0 = (j == yl) ? d : dy0, dy1 = (j == yl + 1) ? d : dy1;
                 dy2 = (j == yr_) ? d : dy2, dy3 = (j == yr_ + 1) ? d : dy3;
-                if (T::HAS_ARMS) {
+                if (D.HAS_ARMS) {
                     da0 = (j == al) ? d : da0, da1 = (j == al + 1) ? d : da1;
                     da2 = (j == ar_) ? d : da2, da3 = (j == ar_ + 1) ? d : da3;
                 }
@@ -695,7 +744,7 @@ post_physics_kernel(const __grid_constant__ hb_env_params p, const __grid_consta
                 float yr = sqrtf(dy0 * dy0 + dy1 * dy1) + sqrtf(dy2 * dy2 + dy3 * dy3);
                 yr = clampf(yr - 0.1f, 0.0f, 50.0f);
                 float djp = expf(-yr * 100.0f);
-                if (T::HAS_ARMS) {
+                if (D.HAS_ARMS) {
                     float ar = sqrtf(da0 * da0 + da1 * da1) + sqrtf(da2 * da2 + da3 * da3);
                     ar = clampf(ar - 0.1f, 0.0f, 25.0f);
                     djp = djp + expf(-ar * 2.0f);
@@ -715,15 +764,19 @@ post_physics_kernel(const __grid_constant__ hb_env_params p, const __grid_consta
         HB_STAMP(3);
         const bool reset = valid && (flags[lane] & 1);
         if (reset) {         // _reset_dofs (legged_robot.py:358-372) + buffer zeroing (:186-191)
-            float u[NDOF];
+            float u[CAP];
             if (nz.u_reset) {
 #pragma unroll
-                for (int j = 0; j < NDOF; ++j) u[j] = nz.u_reset[(size_t)env * U_RESET + j];
+                for (int j = 0; j < CAP; ++j) {
+                    if (T::RUNTIME && j == NDOF) break;
+                    u[j] = nz.u_reset[(size_t)env * U_RESET + j];
+                }
             } else {
                 rng_uniforms(rng, env, SLOT_U_RESET, 0, NDOF, u);
             }
 #pragma unroll
-            for (int j = 0; j < NDOF; ++j) {
+            for (int j = 0; j < CAP; ++j) {
+                if (T::RUNTIME && j == NDOF) break;
                 q[j] = p.default_dof_pos[j] + (p.reset_dof_span * u[j] + p.reset_dof_lo);
                 qd[j] = 0.0f;
                 act[j] = 0.0f;
@@ -744,7 +797,8 @@ post_physics_kernel(const __grid_constant__ hb_env_params p, const __grid_consta
                 if (fabsf(sn) < 0.1f) sl = sr = 0.0f;               // double support
             }
 #pragma unroll
-            for (int j = 0; j < NDOF; ++j) {
+            for (int j = 0; j < CAP; ++j) {
+                if (T::RUNTIME && j == NDOF) break;
                 if (use_ref) {
                     float ref = 0.0f;
 #pragma unroll
@@ -754,7 +808,7 @@ post_physics_kernel(const __grid_constant__ hb_env_params p, const __grid_consta
                         if (j == p.ref_right[k]) ref = sr * sc;
                     }
                     if (valid) b.ref_dof_pos[(size_t)env * NDOF + j] = ref;
-                    if (KIND == KIND_XBOT) sp[lane * PRIV_PAD + T::P_DIFF + j] = clampf(q[j] - ref, -clip, clip);
+                    if (KIND == KIND_XBOT) sp[lane * PRIV_PAD + D.P_DIFF + j] = clampf(q[j] - ref, -clip, clip);
                 }
                 float v0 = (q[j] - p.default_dof_pos[j]) * p.obs_dof_pos, v1 = qd[j] * p.obs_dof_vel;
                 sp[lane * PRIV_PAD + 5 + j] = clampf(v0, -clip, clip);
@@ -901,14 +955,14 @@ post_physics_kernel(const __grid_constant__ hb_env_params p, const __grid_consta
                 for (int f = 0; f < 2; ++f)
 #pragma unroll
                     for (int k = 0; k < 3; ++k) {
-                        sp[lane * PRIV_PAD + T::P_FEET_POS + f * 3 + k] = clampf(foot_pos[f][k], -clip, clip);
-                        sp[lane * PRIV_PAD + T::P_FEET_VEL + f * 3 + k] = clampf(foot_vel[f][k], -clip, clip);
+                        sp[lane * PRIV_PAD + D.P_FEET_POS + f * 3 + k] = clampf(foot_pos[f][k], -clip, clip);
+                        sp[lane * PRIV_PAD + D.P_FEET_VEL + f * 3 + k] = clampf(foot_vel[f][k], -clip, clip);
                     }
             }
-            sp[lane * PRIV_PAD + T::P_FRICTION] = clampf(friction, -clip, clip);
-            sp[lane * PRIV_PAD + T::P_MASS] = clampf(mass / 30.0f, -clip, clip);
-            sp[lane * PRIV_PAD + T::P_STANCE] = st[0], sp[lane * PRIV_PAD + T::P_STANCE + 1] = st[1];
-            sp[lane * PRIV_PAD + T::P_CONTACT] = ct[0] ? 1.0f : 0.0f, sp[lane * PRIV_PAD + T::P_CONTACT + 1] = ct[1] ? 1.0f : 0.0f;
+            sp[lane * PRIV_PAD + D.P_FRICTION] = clampf(friction, -clip, clip);
+            sp[lane * PRIV_PAD + D.P_MASS] = clampf(mass / 30.0f, -clip, clip);
+            sp[lane * PRIV_PAD + D.P_STANCE] = st[0], sp[lane * PRIV_PAD + D.P_STANCE + 1] = st[1];
+            sp[lane * PRIV_PAD + D.P_CONTACT] = ct[0] ? 1.0f : 0.0f, sp[lane * PRIV_PAD + D.P_CONTACT + 1] = ct[1] ? 1.0f : 0.0f;
         }
     } else {
         // ================================ ledger ================================
@@ -921,7 +975,7 @@ post_physics_kernel(const __grid_constant__ hb_env_params p, const __grid_consta
         if (with_noise && !tape_noise && emit_obs) {
             // the tile's observation noise, drawn by this otherwise idle warp while the other roles are in phase A:
             // 11 Philox calls of 4 normals per env; calls whose four columns all have zero noise scale are skipped
-            constexpr int CALLS = (OBS + 3) / 4;
+            const int CALLS = (OBS + 3) / 4;
             float *z = sm + L.z_obs;
             for (int c = lane; c < nv * CALLS; c += 32) {
                 const int e = c / CALLS, q = c - e * CALLS;
@@ -986,7 +1040,8 @@ post_physics_kernel(const __grid_constant__ hb_env_params p, const __grid_consta
         if (emit_obs) {
             // 96 threads walk the tile's frames with (row, column) advanced incrementally: no per-element division.
             // Privileged frames leave as 8-byte pairs (row starts are 8-byte aligned: 4200 r + 3920 bytes).
-            constexpr int NT = 3 * TILE, P2 = PRIV / 2;
+            constexpr int NT = 3 * TILE;
+            const int P2 = PRIV / 2;
             const int orow = p.frame_stack * OBS, prow = p.c_frame_stack * PRIV;
             const int ostride = p.obs_ld ? p.obs_ld : orow, pstride = p.priv_ld ? p.priv_ld : prow;   // row pitch
             const int t = threadIdx.x;
@@ -1291,6 +1346,99 @@ stack_finalize_kernel(const float *__restrict__ prev_a, float *__restrict__ next
     }
 }
 
+// A frame stack whose ROW / LD / FRAME are not compile-time constants: any robot's frames, any stack depth.
+// inv_ld = ceil(2^64 / LD): for e < 2^32, e / LD = umul64hi(e, inv_ld) exactly (the error term e (inv_ld LD - 2^64) / 2^64
+// stays below 1), two wide multiplies instead of a division per vector.
+struct ShiftShape {
+    uint32_t row, ld, frame;
+    unsigned long long inv_ld;
+};
+
+__device__ __forceinline__ uint32_t div_ld(uint32_t e, const ShiftShape &sh) { return (uint32_t)__umul64hi(e, sh.inv_ld); }
+
+// stack_shift_fixed with the shape as arguments; reset_buf null: no zeroing
+template <int UNROLL>
+__device__ __forceinline__ void stack_shift_rt(const float *__restrict__ prev, float *__restrict__ next, const uint32_t total,
+                                               const uint32_t blk, const ShiftShape sh, const uint8_t *__restrict__ reset_buf) {
+    const uint32_t LD = sh.ld, KEEP = sh.row - sh.frame, ROT = sh.frame & 3u, FVEC = sh.frame >> 2;
+    const bool vec_rows = (LD & 3u) == 0;
+    const uint32_t lane = threadIdx.x & 31u;
+    const uint32_t total_vec = total >> 2;
+    const uint32_t tail_vec = (total + 3u) >> 2;
+    const uint32_t warp_base = (blk * blockDim.x + (threadIdx.x - lane)) * UNROLL;
+    const float4 *p4 = reinterpret_cast<const float4 *>(prev);
+    float4 *n4 = reinterpret_cast<float4 *>(next);
+    float4 v[UNROLL], w[UNROLL];
+    uint8_t rz[UNROLL];
+#pragma unroll
+    for (int u = 0; u < UNROLL; ++u) {
+        const uint32_t s = warp_base + u * 32u + lane + FVEC;
+        const uint32_t e = (warp_base + u * 32u + lane) * 4u;
+        const uint32_t r = div_ld(e, sh);
+        rz[u] = (reset_buf && e < total) ? __ldg(reset_buf + r) : 0;
+        w[u] = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (vec_rows) {
+            const bool need = e - r * LD < KEEP + 4u;
+            v[u] = hb::ld_stream4_if(p4 + s, need && s < total_vec);
+            if (ROT != 0) w[u] = hb::ld_stream4_if(p4 + s + 1u, need && lane == 31u && s + 1u < total_vec);
+        } else {
+            v[u] = (s < total_vec) ? hb::ld_stream4(p4 + s) : ld_vec_guarded(prev, s, total);
+            if (ROT != 0 && lane == 31u)
+                w[u] = (s + 1u < total_vec) ? hb::ld_stream4(p4 + s + 1u) : ld_vec_guarded(prev, s + 1u, total);
+        }
+    }
+#pragma unroll
+    for (int u = 0; u < UNROLL; ++u) {
+        const uint32_t i = warp_base + u * 32u + lane;
+        float nx0 = __shfl_down_sync(0xffffffffu, v[u].x, 1);
+        float nx1 = __shfl_down_sync(0xffffffffu, v[u].y, 1);
+        float nx2 = __shfl_down_sync(0xffffffffu, v[u].z, 1);
+        if (lane == 31u) nx0 = w[u].x, nx1 = w[u].y, nx2 = w[u].z;
+        float4 o = v[u];
+        if (ROT == 1) o = make_float4(v[u].y, v[u].z, v[u].w, nx0);
+        else if (ROT == 2) o = make_float4(v[u].z, v[u].w, nx0, nx1);
+        else if (ROT == 3) o = make_float4(v[u].w, nx0, nx1, nx2);
+        if (i >= tail_vec) continue;
+        const uint32_t e0 = i * 4u;
+        const uint32_t r0 = div_ld(e0, sh);
+        const uint32_t c0 = e0 - r0 * LD;
+        if (vec_rows && c0 >= KEEP) continue;
+        if (c0 + 3u < KEEP && i < total_vec) {
+            if (rz[u]) o = make_float4(0.f, 0.f, 0.f, 0.f);
+            hb::st_stream4(n4 + i, o);
+        } else {
+            const float ov[4] = {o.x, o.y, o.z, o.w};
+#pragma unroll
+            for (uint32_t k = 0; k < 4u; ++k) {
+                uint32_t c = c0 + k, r = r0;
+                if (c >= LD) c -= LD, r += 1u;
+                const bool zero = reset_buf && (vec_rows ? rz[u] != 0 : reset_buf[r] != 0);
+                if (c < KEEP && e0 + k < total) next[e0 + k] = zero ? 0.0f : ov[k];
+            }
+        }
+    }
+}
+
+// stack_finalize_kernel for runtime shapes.  Without finalize blocks and with reset_buf null it is the plain shift of both
+// histories (hb_env_stack_observations).
+__global__ void __launch_bounds__(256, 4)
+stack_finalize_rt_kernel(const float *__restrict__ prev_a, float *__restrict__ next_a, uint32_t total_a, uint32_t blocks_a,
+                         const ShiftShape sa, const float *__restrict__ prev_b, float *__restrict__ next_b, uint32_t total_b,
+                         uint32_t blocks_b, const ShiftShape sb, const uint8_t *__restrict__ reset_buf,
+                         const __grid_constant__ hb_env_params p, const __grid_constant__ hb_env_buffers b, int tiles, int seg,
+                         int32_t *host_count, unsigned long long *rng_counter) {
+    hb::pdl_trigger();
+    hb::pdl_wait();
+    const uint32_t fin_blocks = gridDim.x - blocks_a - blocks_b;
+    if (blockIdx.x < fin_blocks) {
+        reset_finalize_body(p, b, nullptr, nullptr, tiles, seg, host_count, rng_counter, blockIdx.x, fin_blocks);
+    } else {
+        const uint32_t blk = blockIdx.x - fin_blocks;
+        if (blk < blocks_a) stack_shift_rt<4>(prev_a, next_a, total_a, blk, sa, reset_buf);
+        else stack_shift_rt<4>(prev_b, next_b, total_b, blk - blocks_a, sb, reset_buf);
+    }
+}
+
 // ------------------------------------------------------------------------------------------
 // LeggedRobot._get_heights (legged_robot.py:759-795; SURVEY.md §8f rank 3): terrain height under a grid of points around
 // each robot.  The points (base frame, z = 0) are rotated by the base's yaw - quat_apply_yaw (utils/math.py:39-43):
@@ -1381,6 +1529,7 @@ mirror_frames_kernel(const float *__restrict__ obs, int obs_ld, int row_a, int f
 }
 
 int g_use_bulk = 1;
+int g_runtime_task = 0;      // 1: the three built robots too run post_physics_kernel with the layout read at run time
 
 // Frame stacks of the three tasks (hector_config.py:8-20, hector_w_arm_config.py:8-20, humanoid_config.py:42-52): rows
 // either dense or at the 128-byte pitch ceil32(row + 1) (TMA-addressable: the rollout storage's slots)
@@ -1425,12 +1574,12 @@ template <typename T, bool kBulk>
 int launch_post_physics(const hb_env_params *p, const hb_env_buffers *buf, const hb_env_noise *noise, float *obs_new,
                         float *priv_new, int32_t stages, cudaStream_t st) {
     const bool with_noise = p->add_noise && (noise->z_obs || noise->rng_counter);
-    const TileLayout L = make_layout(p->num_bodies, with_noise, T::NDOF, T::OBS, T::PRIV);
+    const TileLayout L = make_layout(p->num_bodies, with_noise, p->num_dof, p->num_single_obs, p->num_single_priv);
     const size_t smem = (size_t)L.total * sizeof(float);
     const int tiles = (p->num_envs + TILE - 1) / TILE;
     static bool attr_set = false;
     if (!attr_set) {
-        HB_CUDA(cudaFuncSetAttribute(post_physics_kernel<kBulk, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024));
+        HB_CUDA(cudaFuncSetAttribute(post_physics_kernel<kBulk, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, POST_SMEM_MAX));
         attr_set = true;
     }
     HB_CUDA(hb::launch_pdl(hb::use_pdl_post(p->num_envs), post_physics_kernel<kBulk, T>, dim3(tiles), dim3(4 * TILE), smem, st, *p, *buf,
@@ -1440,12 +1589,17 @@ int launch_post_physics(const hb_env_params *p, const hb_env_buffers *buf, const
 }
 
 // The frame-stack shift of both histories: rows and pitches, built shape (0 hector, 1 hector_full, 2 XBot-L) and layout
-// (0 = not a built shape, 1 = dense rows, 2 = 128-byte pitch), and whether the fixed-shape kernels apply, with their grid
+// (0 = not a built shape, 1 = dense rows, 2 = 128-byte pitch), and whether the fixed-shape kernels apply (fast) or else the
+// runtime-shape kernel (vec: 16-byte aligned buffers), with their grid
 struct StackPlan {
     int row_a, row_b, ld_a, ld_b, shape, layout;
-    bool fast;
+    bool fast, vec;
     uint32_t total_a, total_b, blocks_a, blocks_b;
 };
+
+ShiftShape shift_shape(int row, int ld, int frame) {
+    return {(uint32_t)row, (uint32_t)ld, (uint32_t)frame, ~0ull / (unsigned long long)ld + 1ull};
+}
 
 template <typename S>
 int shape_layout(const StackPlan &s, const hb_env_params *p) {
@@ -1461,10 +1615,13 @@ StackPlan stack_plan(const hb_env_params *p, const float *obs_prev, const float 
     const int layouts[3] = {shape_layout<ShapeHector>(s, p), shape_layout<ShapeHectorFull>(s, p), shape_layout<ShapeXBot>(s, p)};
     s.shape = layouts[0] ? 0 : (layouts[1] ? 1 : 2);
     s.layout = layouts[s.shape];
-    s.fast = hb::aligned16(obs_prev) && hb::aligned16(obs_new) && hb::aligned16(priv_prev) && hb::aligned16(priv_new) &&
-             s.layout != 0 && fits_u32(p->num_envs, s.ld_a > s.ld_b ? s.ld_a : s.ld_b);
+    s.vec = hb::aligned16(obs_prev) && hb::aligned16(obs_new) && hb::aligned16(priv_prev) && hb::aligned16(priv_new) &&
+            fits_u32(p->num_envs, s.ld_a > s.ld_b ? s.ld_a : s.ld_b);
+    s.fast = s.vec && s.layout != 0;
     s.total_a = (uint32_t)p->num_envs * s.ld_a, s.total_b = (uint32_t)p->num_envs * s.ld_b;
-    s.blocks_a = shift_blocks(s.total_a), s.blocks_b = shift_blocks(s.total_b);
+    // a stack of one frame carries nothing over: no shift blocks
+    s.blocks_a = s.row_a > p->num_single_obs ? shift_blocks(s.total_a) : 0;
+    s.blocks_b = s.row_b > p->num_single_priv ? shift_blocks(s.total_b) : 0;
     return s;
 }
 
@@ -1487,6 +1644,22 @@ FinalizeGrid finalize_grid(int num_envs) {
     int seg = (tiles + hb::sm_count() - 1) / hb::sm_count();
     if (seg < 8) seg = 8;
     return {tiles, seg, (tiles + seg - 1) / seg};
+}
+
+// stack_finalize_rt_kernel: both shifts and, with `finalize`, the reset finalisation (ids, means, history zeroing)
+int launch_stack_rt(const hb_env_params *p, const hb_env_buffers *buf, const StackPlan &s, const float *obs_prev,
+                    const float *priv_prev, float *obs_new, float *priv_new, bool finalize, int32_t *host_count,
+                    uint64_t *rng_counter, cudaStream_t st) {
+    const FinalizeGrid g = finalize_grid(p->num_envs);
+    const uint32_t fin_blocks = finalize ? (uint32_t)g.blocks : 0u;
+    if (s.blocks_a + s.blocks_b + fin_blocks == 0) return HB_OK;
+    HB_CUDA(hb::launch_pdl(hb::use_pdl_stack(p->num_envs), stack_finalize_rt_kernel, dim3(fin_blocks + s.blocks_a + s.blocks_b),
+                           dim3(256), 0, st, obs_prev, obs_new, s.total_a, s.blocks_a, shift_shape(s.row_a, s.ld_a, p->num_single_obs),
+                           priv_prev, priv_new, s.total_b, s.blocks_b, shift_shape(s.row_b, s.ld_b, p->num_single_priv),
+                           finalize ? (const uint8_t *)buf->reset_buf : nullptr, *p, *buf, g.tiles, g.seg, host_count,
+                           reinterpret_cast<unsigned long long *>(rng_counter)));
+    HB_CHECK_LAUNCH("stack_finalize_rt_kernel");
+    return HB_OK;
 }
 
 PdConsts pd_consts(const hb_env_params *p) {
@@ -1525,6 +1698,10 @@ int hb_set_option(const char *name, int value) {
         g_use_bulk = value;
         return HB_OK;
     }
+    if (name && !strcmp(name, "env_runtime_task")) {
+        g_runtime_task = value != 0;
+        return HB_OK;
+    }
     if (name && !strcmp(name, "gemm_pdl")) {
         hb::g_gemm_pdl = value != 0;
         return HB_OK;
@@ -1552,6 +1729,34 @@ int hb_set_option(const char *name, int value) {
     }
     hb::set_error("hb_set_option: unknown option '%s'", name ? name : "(null)");
     return HB_ERR_BAD_ARG;
+}
+
+// The layout of a robot that post_physics_kernel reads at run time (RuntimeTask)
+static int check_runtime_task(const hb_env_params *p) {
+    const int n = p->num_dof;
+    if (n > MAX_TASK_DOF) {
+        hb::set_error("hb_env_post_physics: num_dof=%d is not supported (1 to %d joints: the observation frame 3 num_dof + 11 "
+                      "must fit %d columns)", n, MAX_TASK_DOF, HB_MAX_OBS);
+        return HB_ERR_UNSUPPORTED;
+    }
+    HB_REQUIRE(p->task_kind == HB_TASK_HECTOR || p->task_kind == HB_TASK_XBOT, "hb_env_post_physics: task_kind=%d (0 hector, 1 XBot-L)",
+               p->task_kind);
+    const TaskDims d = task_dims(n, p->task_kind == HB_TASK_XBOT ? KIND_XBOT : KIND_HECTOR, 0, 0, 0, 0);
+    HB_REQUIRE(p->num_single_obs == d.OBS && p->num_single_priv == d.PRIV,
+               "hb_env_post_physics: frames %d / %d do not match num_dof=%d task_kind=%d (%d / %d: 3 num_dof + 11 and %s)",
+               p->num_single_obs, p->num_single_priv, n, p->task_kind, d.OBS, d.PRIV,
+               p->task_kind == HB_TASK_XBOT ? "4 num_dof + 25" : "3 num_dof + 40");
+    auto pair_ok = [&](int j) { return j >= 0 && j + 1 < n; };
+    HB_REQUIRE(pair_ok(p->yaw_roll[0]) && pair_ok(p->yaw_roll[1]),
+               "hb_env_post_physics: yaw_roll (%d, %d): each pair's first joint j needs 0 <= j and j + 1 < num_dof=%d", p->yaw_roll[0],
+               p->yaw_roll[1], n);
+    HB_REQUIRE((p->arm_pair[0] == -1 && p->arm_pair[1] == -1) || (pair_ok(p->arm_pair[0]) && pair_ok(p->arm_pair[1])),
+               "hb_env_post_physics: arm_pair (%d, %d): -1, -1 (no arms) or first joints j with 0 <= j and j + 1 < num_dof=%d",
+               p->arm_pair[0], p->arm_pair[1], n);
+    for (int k = 0; k < 3; ++k)
+        HB_REQUIRE(p->ref_left[k] >= 0 && p->ref_left[k] < n && p->ref_right[k] >= 0 && p->ref_right[k] < n,
+                   "hb_env_post_physics: ref_left / ref_right [%d] = %d / %d outside [0, num_dof=%d)", k, p->ref_left[k], p->ref_right[k], n);
+    return HB_OK;
 }
 
 static int check_params(const hb_env_params *p, const hb_env_buffers *buf, const char *who) {
@@ -1628,13 +1833,6 @@ int hb_env_post_physics(const hb_env_params *p, const hb_env_buffers *buf, const
                    p->n_pen <= HB_MAX_CONTACT_BODIES, "hb_env_post_physics: too many contact bodies");
     HB_REQUIRE(noise->u_reset || noise->rng_counter, "hb_env_post_physics: u_reset or the device generator is required (any env may reset)");
     HB_REQUIRE(buf->scratch_ballots && buf->scratch_sums, "hb_env_post_physics: null scratch buffers");
-    {   // the joint pairs of default_joint_pos are constants of the three robots, compiled into the kernels
-        const bool arms = p->num_dof == 18;
-        HB_REQUIRE(p->yaw_roll[0] == 0 && p->yaw_roll[1] == p->num_dof / 2 && p->arm_pair[0] == (arms ? 5 : -1) &&
-                       p->arm_pair[1] == (arms ? p->num_dof / 2 + 5 : -1),
-                   "hb_env_post_physics: yaw_roll / arm_pair (%d, %d / %d, %d) are not the built robots' joint pairs (0, num_dof/2 / "
-                   "5, num_dof/2 + 5 with arms, -1 without)", p->yaw_roll[0], p->yaw_roll[1], p->arm_pair[0], p->arm_pair[1]);
-    }
     HB_REQUIRE((p->reward_scale[HB_R_JOINT_POS] == 0.0f && p->task_kind != HB_TASK_XBOT) || buf->ref_dof_pos,
                "hb_env_post_physics: ref_dof_pos is required (joint_pos reward / XBot-L privileged frame)");
     // bulk staging needs 16-byte aligned slabs: base pointers aligned and 32-env tiles (128-byte multiples)
@@ -1653,8 +1851,12 @@ int hb_env_post_physics(const hb_env_params *p, const hb_env_buffers *buf, const
     using HectorFull = Task<18, KIND_HECTOR, true>;
     using HectorFullSlim = Task<18, KIND_HECTOR, false>;
     using XBot = Task<12, KIND_XBOT, true>;
+    // the joint pairs of default_joint_pos are constants of the three robots, compiled into their kernels
     auto matches = [&](int ndof, int kind, int obs, int priv) {
-        return p->num_dof == ndof && p->task_kind == kind && p->num_single_obs == obs && p->num_single_priv == priv;
+        const bool arms = ndof == 18;
+        return !g_runtime_task && p->num_dof == ndof && p->task_kind == kind && p->num_single_obs == obs &&
+               p->num_single_priv == priv && p->yaw_roll[0] == 0 && p->yaw_roll[1] == ndof / 2 &&
+               p->arm_pair[0] == (arms ? 5 : -1) && p->arm_pair[1] == (arms ? ndof / 2 + 5 : -1);
     };
     // a config that scales none of the optional terms runs the kernel compiled without them
     const bool opt = p->reward_scale[HB_R_JOINT_POS] != 0.0f || p->reward_scale[HB_R_VEL_MISMATCH_EXP] != 0.0f ||
@@ -1667,9 +1869,9 @@ int hb_env_post_physics(const hb_env_params *p, const hb_env_buffers *buf, const
     if (matches(10, HB_TASK_HECTOR, Hector::OBS, Hector::PRIV)) return opt ? launch(Hector{}) : launch(HectorSlim{});
     if (matches(18, HB_TASK_HECTOR, HectorFull::OBS, HectorFull::PRIV)) return opt ? launch(HectorFull{}) : launch(HectorFullSlim{});
     if (matches(12, HB_TASK_XBOT, XBot::OBS, XBot::PRIV)) return launch(XBot{});
-    hb::set_error("hb_env_post_physics: no kernel for num_dof=%d task_kind=%d frames %d/%d (built: hector 10/41/70, hector_full "
-                  "18/65/94, XBot-L 12/47/73)", p->num_dof, p->task_kind, p->num_single_obs, p->num_single_priv);
-    return HB_ERR_UNSUPPORTED;
+    // any other robot: the kernel with the layout read from p
+    if (int rc = check_runtime_task(p)) return rc;
+    return p->task_kind == HB_TASK_XBOT ? launch(RuntimeTask<KIND_XBOT>{}) : launch(RuntimeTask<KIND_HECTOR>{});
 }
 
 int hb_env_get_heights(const float *root_states, const float *points_xy, int32_t num_points, const int16_t *height_samples,
@@ -1707,8 +1909,11 @@ int hb_env_stack_observations(const hb_env_params *p, const hb_env_buffers *buf,
         HB_CHECK_LAUNCH("stack_shift_pair_kernel");
         return HB_OK;
     }
-    if (int rc = shift_any(obs_prev, obs_new, nullptr, p->num_envs, s.row_a, s.ld_a, p->num_single_obs, st)) return rc;
-    return shift_any(priv_prev, priv_new, nullptr, p->num_envs, s.row_b, s.ld_b, p->num_single_priv, st);
+    if (s.vec) return launch_stack_rt(p, buf, s, obs_prev, priv_prev, obs_new, priv_new, false, nullptr, nullptr, st);
+    if (s.blocks_a)
+        if (int rc = shift_any(obs_prev, obs_new, nullptr, p->num_envs, s.row_a, s.ld_a, p->num_single_obs, st)) return rc;
+    if (s.blocks_b) return shift_any(priv_prev, priv_new, nullptr, p->num_envs, s.row_b, s.ld_b, p->num_single_priv, st);
+    return HB_OK;
 }
 
 int hb_env_stack_finalize(const hb_env_params *p, const hb_env_buffers *buf, const float *obs_prev, const float *priv_prev,
@@ -1719,7 +1924,9 @@ int hb_env_stack_finalize(const hb_env_params *p, const hb_env_buffers *buf, con
     HB_REQUIRE(buf->scratch_ballots && buf->scratch_sums && buf->reset_env_ids && buf->reset_count && buf->episode_means,
                "hb_env_stack_finalize: null scratch/result buffers");
     const StackPlan s = stack_plan(p, obs_prev, priv_prev, obs_new, priv_new);
-    if (!s.fast) {        // other layouts: the two separate launches
+    if (!s.fast && s.vec)
+        return launch_stack_rt(p, buf, s, obs_prev, priv_prev, obs_new, priv_new, true, host_count, rng_counter, (cudaStream_t)stream);
+    if (!s.fast) {        // unaligned or oversized buffers: the two separate launches
         if (int rc = hb_env_stack_observations(p, buf, obs_prev, priv_prev, obs_new, priv_new, stream)) return rc;
         return hb_env_reset_finalize(p, buf, obs_new, priv_new, host_count, rng_counter, stream);
     }

@@ -8,6 +8,9 @@ The env step is the same code for all three (the two hector tasks even share the
 arm term of default_joint_pos and the reward table); what differs is collected in a `TaskLayout`: joint count, where the
 privileged frame keeps its columns, and the joint-index constants the env files spell out literally.  Configs restate the
 values of the reference's config files as overrides of `HectorCfg` (only what the hot path reads).
+
+Any other robot whose env file is a copy of hector_env.py or humanoid_env.py runs on the same kernels: its config carries
+`layout = TaskLayout(...)` with its joint count (up to MAX_DOF) and joint indices (INTEGRATION.md §1).
 """
 from __future__ import annotations
 
@@ -16,6 +19,9 @@ from typing import Tuple
 
 from .._lib import HB_TASK_HECTOR, HB_TASK_XBOT
 from .hector_config import HectorCfg, HectorCfgPPO, _Cfg
+
+# the observation frame 3 ndof + 11 fits the kernels' 80 columns (HB_MAX_OBS); more joints would move the device draws
+MAX_DOF = 23
 
 
 @dataclass(frozen=True)
@@ -29,6 +35,43 @@ class TaskLayout:
     ref_right: Tuple[int, int, int]
     # _get_noise_scale_vec, literally: (start, stop) of the dof_pos, dof_vel, zeroed-actions, ang_vel and quat assignments
     noise_slices: Tuple[Tuple[int, int], ...]
+
+    def __post_init__(self):
+        def bad(field, why):
+            raise ValueError(f"TaskLayout {self.name!r}: {field} = {getattr(self, field)!r}: {why}")
+
+        if self.kind not in (HB_TASK_HECTOR, HB_TASK_XBOT):
+            bad("kind", "HB_TASK_HECTOR (hector_env.py frames) or HB_TASK_XBOT (humanoid_env.py frames)")
+        if not isinstance(self.ndof, int) or not 1 <= self.ndof <= MAX_DOF:
+            bad("ndof", f"1 to {MAX_DOF} joints (the observation frame 3 ndof + 11 must fit 80 columns)")
+        pair = lambda j: isinstance(j, int) and 0 <= j and j + 1 < self.ndof
+        if len(self.yaw_roll) != 2 or not all(pair(j) for j in self.yaw_roll):
+            bad("yaw_roll", f"two first joints j of a (yaw, roll) pair, 0 <= j and j + 1 < ndof = {self.ndof}")
+        if tuple(self.arm_pair) != (-1, -1) and (len(self.arm_pair) != 2 or not all(pair(j) for j in self.arm_pair)):
+            bad("arm_pair", f"(-1, -1) without arms, else two first joints j with 0 <= j and j + 1 < ndof = {self.ndof}")
+        for field in ("ref_left", "ref_right"):
+            v = getattr(self, field)
+            if len(v) != 3 or not all(isinstance(j, int) and 0 <= j < self.ndof for j in v):
+                bad(field, f"three joint indices in [0, ndof = {self.ndof})")
+        # (a stop past the frame is clipped, as numpy / torch slicing does: hector_env.py:155 assigns [38:42] of 41 columns)
+        if len(self.noise_slices) != 5 or not all(len(s) == 2 and 0 <= s[0] < self.num_single_obs and s[0] <= s[1]
+                                                  for s in self.noise_slices):
+            bad("noise_slices", f"five (start, stop) pairs, 0 <= start < num_single_obs = {self.num_single_obs}, start <= stop "
+                "(dof_pos, dof_vel, actions, ang_vel, quat)")
+
+    def check_config(self, cfg) -> None:
+        """ValueError naming the first config field that disagrees with this layout."""
+        want = {"env.num_actions": self.ndof, "env.num_single_obs": self.num_single_obs,
+                "env.single_num_privileged_obs": self.num_single_priv}
+        got = {"env.num_actions": cfg.env.num_actions, "env.num_single_obs": cfg.env.num_single_obs,
+               "env.single_num_privileged_obs": cfg.env.single_num_privileged_obs}
+        names = getattr(getattr(cfg, "asset", None), "dof_names", None)
+        if names is not None:
+            want["asset.dof_names"], got["asset.dof_names"] = f"{self.ndof} names", f"{len(names)} names"
+        for k in want:
+            if got[k] != want[k]:
+                raise ValueError(f"config field {k} = {got[k]} does not match TaskLayout {self.name!r} (ndof = {self.ndof}, "
+                                 f"kind = {self.kind}): expected {want[k]}")
 
     @property
     def num_single_obs(self) -> int:
@@ -52,16 +95,22 @@ XBOT = TaskLayout("humanoid_ppo", HB_TASK_XBOT, 12, (0, 6), (-1, -1), (2, 3, 4),
 
 
 def layout_for(cfg) -> TaskLayout:
-    """The layout of a config (this module's or the reference's own config object: it is recognised by its dimensions)."""
+    """The layout of a config: `cfg.layout` when it has one (checked against the config), else one of the three robots,
+    recognised by its dimensions (this module's configs or the reference's own config objects)."""
     explicit = getattr(cfg, "layout", None)
     if isinstance(explicit, TaskLayout):
+        explicit.check_config(cfg)
         return explicit
     for lay in (HECTOR, HECTOR_FULL, XBOT):
         if (cfg.env.num_actions == lay.ndof and cfg.env.num_single_obs == lay.num_single_obs
                 and cfg.env.single_num_privileged_obs == lay.num_single_priv):
             return lay
-    raise ValueError(f"no kernel layout for num_actions={cfg.env.num_actions}, frames {cfg.env.num_single_obs} / "
-                     f"{cfg.env.single_num_privileged_obs} (built: hector 10/41/70, hector_full 18/65/94, XBot-L 12/47/73)")
+    raise ValueError(
+        f"num_actions={cfg.env.num_actions}, frames {cfg.env.num_single_obs} / {cfg.env.single_num_privileged_obs} is none of "
+        "the built robots (hector 10/41/70, hector_full 18/65/94, XBot-L 12/47/73): describe the robot in its config, e.g. "
+        "cfg.layout = TaskLayout(name='my_robot', kind=HB_TASK_HECTOR, ndof=12, yaw_roll=(0, 6), arm_pair=(-1, -1), "
+        "ref_left=(2, 3, 4), ref_right=(8, 9, 10), noise_slices=((5, 17), (17, 29), (29, 41), (41, 44), (44, 47))) "
+        f"(isaac_b200.envs.tasks; up to {MAX_DOF} joints; INTEGRATION.md §1)")
 
 
 _LEG = ["hip_joint", "hip_roll_joint", "thigh_joint", "calf_joint", "toe_joint"]
@@ -242,5 +291,5 @@ TASKS = {
     "hector_full": ("HectorFullFreeEnvB200", HectorFullCfg, HectorFullCfgPPO),
     "humanoid_ppo": ("XBotLFreeEnvB200", XBotLCfg, XBotLCfgPPO),
 }
-__all__ = ["TaskLayout", "HECTOR", "HECTOR_FULL", "XBOT", "layout_for", "HectorFullCfg", "HectorFullCfgPPO", "XBotLCfg",
+__all__ = ["TaskLayout", "MAX_DOF", "HECTOR", "HECTOR_FULL", "XBOT", "layout_for", "HectorFullCfg", "HectorFullCfgPPO", "XBotLCfg",
            "XBotLCfgPPO", "TASKS", "_Cfg"]
