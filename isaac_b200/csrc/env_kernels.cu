@@ -1078,14 +1078,12 @@ post_physics_kernel(const __grid_constant__ hb_env_params p, const __grid_consta
 
 // ------------------------------------------------------------------------------------------
 // a8 (stacking): new[:, 0:(S-1)*F] = prev[:, F:S*F]  — a flat copy shifted by one frame with a
-// hole of F floats per row (the newest frame, written by post_physics_kernel).  With CHECK_RESET the
+// hole of F floats per row (the newest frame, written by post_physics_kernel).  With kZero the
 // carried frames of the envs post-physics just reset are written as zeros (reset_idx,
 // hector_env.py:256-261); without it that is left to reset_finalize_kernel.
 // Destination vectors are 16-byte aligned; the source is 4*F bytes further on, which is only
 // 4-byte aligned for F = 41, so each thread loads the aligned vector below its source window
 // and takes the missing floats from its neighbour lane (shuffle); F % 4 picks the rotation.
-// ROW and FRAME are compile-time constants for the hector layout: the per-vector row/column
-// split is a multiply-shift, indices are 32-bit.
 // ------------------------------------------------------------------------------------------
 __device__ __forceinline__ float4 ld_vec_guarded(const float *__restrict__ prev, uint32_t s, uint32_t total) {
     const uint32_t e = s * 4u;                         // ragged last vector of the buffer (N*row % 4 != 0)
@@ -1097,13 +1095,37 @@ __device__ __forceinline__ float4 ld_vec_guarded(const float *__restrict__ prev,
     return v;
 }
 
-template <int ROW, int LD, int FRAME, int UNROLL, bool CHECK_RESET = false>
-__device__ __forceinline__ void
-stack_shift_fixed(const float *__restrict__ prev, float *__restrict__ next, const uint32_t total, const uint32_t blk,
-                  const uint8_t *__restrict__ reset_buf = nullptr) {
-    constexpr uint32_t KEEP = ROW - FRAME;              // floats of a row that are carried over
-    constexpr int ROT = FRAME & 3;                      // source misalignment in floats
-    constexpr uint32_t FVEC = FRAME >> 2;               // whole vectors of shift
+// The shape of one history's stack: rows of `row` floats, the last `frame` of them the newest frame, at a pitch of `ld`
+// floats.  A built robot's shape is all constants (FixedShift): the row split of a vector index is then a multiply-shift
+// and the rotation is resolved at compile time.
+template <int ROW, int LD, int FRAME>
+struct FixedShift {
+    static constexpr bool kFixed = true;
+    static constexpr uint32_t row = ROW, ld = LD, frame = FRAME;
+    __device__ __forceinline__ static uint32_t div(uint32_t e) { return e / (uint32_t)LD; }
+};
+
+// Any other shape: any robot's frames, any stack depth.  inv_ld = ceil(2^64 / ld): for e < 2^32, e / ld =
+// umul64hi(e, inv_ld) exactly (the error term e (inv_ld ld - 2^64) / 2^64 stays below 1), two wide multiplies instead of
+// a division per vector.
+struct ShiftShape {
+    static constexpr bool kFixed = false;
+    uint32_t row, ld, frame;
+    unsigned long long inv_ld;
+    __device__ __forceinline__ uint32_t div(uint32_t e) const { return (uint32_t)__umul64hi(e, inv_ld); }
+};
+
+// Block `blk` of the shift of one history (`total` floats): 256 threads, UNROLL vectors each.  kZero: the carried frames
+// of the envs flagged in reset_buf are written as zeros.  A compiled shape shuffles only the floats its rotation needs,
+// and kZero alone decides the zeroing.  The runtime shape shuffles all three floats, with no branch on the rotation, and
+// serves the plain shift too in the same kernel, so there a null reset_buf means no zeroing.
+template <typename Shape, int UNROLL, bool kZero>
+__device__ __forceinline__ void stack_shift(const float *__restrict__ prev, float *__restrict__ next, const uint32_t total,
+                                            const uint32_t blk, const Shape sh, const uint8_t *__restrict__ reset_buf) {
+    const uint32_t LD = sh.ld, KEEP = sh.row - sh.frame;     // floats of a row that are carried over
+    const uint32_t ROT = sh.frame & 3u;                      // source misalignment in floats
+    const uint32_t FVEC = sh.frame >> 2;                     // whole vectors of shift
+    const bool vec_rows = (LD & 3u) == 0;                    // the buffer is whole vectors: predicated loads
     const uint32_t lane = threadIdx.x & 31u;
     const uint32_t total_vec = total >> 2;              // whole vectors
     const uint32_t tail_vec = (total + 3u) >> 2;
@@ -1117,13 +1139,13 @@ stack_shift_fixed(const float *__restrict__ prev, float *__restrict__ next, cons
     for (int u = 0; u < UNROLL; ++u) {
         const uint32_t s = warp_base + u * 32u + lane + FVEC;          // aligned source vector below the window
         const uint32_t e = (warp_base + u * 32u + lane) * 4u;
-        const uint32_t r = e / (uint32_t)LD;
-        rz[u] = 0;
-        if (CHECK_RESET && e < total) rz[u] = __ldg(reset_buf + r);
+        const uint32_t r = sh.div(e);
+        rz[u] = (kZero && (Shape::kFixed || reset_buf) && e < total) ? __ldg(reset_buf + r) : 0;
+        if (!Shape::kFixed) w[u] = make_float4(0.f, 0.f, 0.f, 0.f);
         // vector-aligned rows: a destination vector that lies, like the one before it, wholly in the newest-frame
         // hole or the padding needs no source (neither for itself nor for its left neighbour's spill-over)
-        if ((LD & 3) == 0) {                                            // the buffer is whole vectors: predicated loads
-            const bool need = e - r * (uint32_t)LD < KEEP + 4u;
+        if (vec_rows) {
+            const bool need = e - r * LD < KEEP + 4u;
             v[u] = hb::ld_stream4_if(p4 + s, need && s < total_vec);
             if (ROT != 0) w[u] = hb::ld_stream4_if(p4 + s + 1u, need && lane == 31u && s + 1u < total_vec);
         } else {
@@ -1136,56 +1158,37 @@ stack_shift_fixed(const float *__restrict__ prev, float *__restrict__ next, cons
     for (int u = 0; u < UNROLL; ++u) {
         const uint32_t i = warp_base + u * 32u + lane;                  // destination vector index
         float4 o = v[u];
-        if (ROT != 0) {
+        if (ROT != 0 || !Shape::kFixed) {
             float nx0 = __shfl_down_sync(0xffffffffu, v[u].x, 1);       // first floats of vector s+1
-            float nx1 = ROT > 1 ? __shfl_down_sync(0xffffffffu, v[u].y, 1) : 0.0f;
-            float nx2 = ROT > 2 ? __shfl_down_sync(0xffffffffu, v[u].z, 1) : 0.0f;
+            float nx1 = ROT > 1 || !Shape::kFixed ? __shfl_down_sync(0xffffffffu, v[u].y, 1) : 0.0f;
+            float nx2 = ROT > 2 || !Shape::kFixed ? __shfl_down_sync(0xffffffffu, v[u].z, 1) : 0.0f;
             if (lane == 31u) nx0 = w[u].x, nx1 = w[u].y, nx2 = w[u].z;
             if (ROT == 1) o = make_float4(v[u].y, v[u].z, v[u].w, nx0);
             else if (ROT == 2) o = make_float4(v[u].z, v[u].w, nx0, nx1);
-            else o = make_float4(v[u].w, nx0, nx1, nx2);
+            else if (ROT == 3) o = make_float4(v[u].w, nx0, nx1, nx2);
         }
         if (i >= tail_vec) continue;
         const uint32_t e0 = i * 4u;                      // first destination float
-        const uint32_t r0 = e0 / (uint32_t)LD;             // LD = row pitch (ROW, or ROW padded to whole vectors)
-        const uint32_t c0 = e0 - r0 * (uint32_t)LD;
-        if ((LD & 3) == 0 && c0 >= KEEP) continue;         // vector-aligned rows: newest-frame hole / padding
+        const uint32_t r0 = sh.div(e0);
+        const uint32_t c0 = e0 - r0 * LD;
+        if (vec_rows && c0 >= KEEP) continue;            // vector-aligned rows: newest-frame hole / padding
         if (c0 + 3u < KEEP && i < total_vec) {           // whole vector inside the carried part of one row
-            if (CHECK_RESET && rz[u]) o = make_float4(0.f, 0.f, 0.f, 0.f);
+            if (rz[u]) o = make_float4(0.f, 0.f, 0.f, 0.f);
             hb::st_stream4(n4 + i, o);
         } else {                                         // touches the newest-frame hole or a row boundary
             const float ov[4] = {o.x, o.y, o.z, o.w};
 #pragma unroll
             for (uint32_t k = 0; k < 4u; ++k) {
                 uint32_t c = c0 + k, r = r0;
-                if (c >= (uint32_t)LD) c -= (uint32_t)LD, r += 1u;
-                const bool zero = CHECK_RESET && ((LD & 3) == 0 ? rz[u] != 0 : reset_buf[r] != 0);   // (a vector of a pitched row stays in its row)
-                if (c < KEEP && e0 + k < total) next[e0 + k] = zero ? 0.0f : ov[k];
+                if (c >= LD) c -= LD, r += 1u;
+                if (c < KEEP && e0 + k < total) {               // (past the buffer's end r is num_envs: no flag to read)
+                    const bool zero = kZero && (Shape::kFixed || reset_buf) &&
+                                      (vec_rows ? rz[u] != 0 : reset_buf[r] != 0);   // (a vector of a pitched row stays in its row)
+                    next[e0 + k] = zero ? 0.0f : ov[k];
+                }
             }
         }
     }
-}
-
-// actor and critic histories in one launch: blocks [0, blocks_a) shift buffer a, the rest buffer b
-template <int ROW_A, int LD_A, int FRAME_A, int ROW_B, int LD_B, int FRAME_B, int UNROLL>
-__global__ void __launch_bounds__(256)
-stack_shift_pair_kernel(const float *__restrict__ prev_a, float *__restrict__ next_a, uint32_t total_a, uint32_t blocks_a,
-                        const float *__restrict__ prev_b, float *__restrict__ next_b, uint32_t total_b) {
-    // Only the launch overlaps the predecessor (post-physics): the shift itself reads nothing that kernel writes, but
-    // running this bandwidth-bound copy beside the latency-bound post-physics kernel was measured to cost more than
-    // it hides (+13 % step time at 65 536 envs), so the data movement starts after it.
-    hb::pdl_trigger();
-    hb::pdl_wait();
-    if (blockIdx.x < blocks_a)
-        stack_shift_fixed<ROW_A, LD_A, FRAME_A, UNROLL>(prev_a, next_a, total_a, blockIdx.x);
-    else
-        stack_shift_fixed<ROW_B, LD_B, FRAME_B, UNROLL>(prev_b, next_b, total_b, blockIdx.x - blocks_a);
-}
-
-template <int ROW, int FRAME, int UNROLL>
-__global__ void __launch_bounds__(256)
-stack_shift_fixed_kernel(const float *__restrict__ prev, float *__restrict__ next, uint32_t total) {
-    stack_shift_fixed<ROW, ROW, FRAME, UNROLL>(prev, next, total, blockIdx.x);
 }
 
 // generic shapes / unaligned buffers / optional per-env zeroing (reset_buf may be null)
@@ -1321,121 +1324,50 @@ reset_finalize_kernel(const __grid_constant__ hb_env_params p, const __grid_cons
     reset_finalize_body(p, b, obs_new, priv_new, tiles, seg, host_count, rng_counter, blockIdx.x, gridDim.x);
 }
 
-// The step's last launch: frame-stack shift of both histories (zeroing the carried frames of the envs post-physics
-// just reset: hector_env.py:256-261) and the shard-wide half of reset_idx (ids, count, episode means, time-out
-// latch: reset_finalize_body without the zeroing) in a few extra blocks of the same grid - one
-// launch less on the step's dependency chain than shift + reset_finalize_kernel.
-template <int ROW_A, int LD_A, int FRAME_A, int ROW_B, int LD_B, int FRAME_B, int UNROLL>
-__global__ void __launch_bounds__(256, 6)
-stack_finalize_kernel(const float *__restrict__ prev_a, float *__restrict__ next_a, uint32_t total_a, uint32_t blocks_a,
-                      const float *__restrict__ prev_b, float *__restrict__ next_b, uint32_t total_b, uint32_t blocks_b,
-                      const __grid_constant__ hb_env_params p, const __grid_constant__ hb_env_buffers b, int tiles, int seg,
-                      int32_t *host_count, unsigned long long *rng_counter) {
+// Arguments of the reset finalisation for a frame-stack launch that runs it (reset_finalize_body without the zeroing),
+// or none (NoFinalize: the plain shift)
+struct FinalizeArgs {
+    static constexpr bool kOn = true;
+    hb_env_params p;
+    hb_env_buffers b;
+    int tiles, seg;
+    int32_t *host_count;
+    unsigned long long *rng_counter;
+};
+struct NoFinalize { static constexpr bool kOn = false; };
+
+// The frame-stack shift of both histories: blocks [0, blocks_a) shift history a, the next blocks_b history b.  With
+// FinalizeArgs, the step's last launch: the carried frames of the envs post-physics just reset are zeroed (reset flags
+// fin.b.reset_buf, hector_env.py:256-261) and the shard-wide half of reset_idx (ids, count, episode means, time-out latch)
+// runs in a few extra blocks of the same grid - one launch less on the step's dependency chain than shift +
+// reset_finalize_kernel.  Blocks per SM with finalisation: 6 for a compiled shape (40 registers), 4 for the runtime shape
+// (56 registers).
+template <typename SA, typename SB, typename Fin>
+__global__ void __launch_bounds__(256, !Fin::kOn ? 0 : (SA::kFixed ? 6 : 4))
+stack_shift_kernel(const float *__restrict__ prev_a, float *__restrict__ next_a, uint32_t total_a, uint32_t blocks_a,
+                   const float *__restrict__ prev_b, float *__restrict__ next_b, uint32_t total_b, uint32_t blocks_b,
+                   const __grid_constant__ Fin fin, const SA sa, const SB sb) {
     static_assert(FIN_THREADS == 256, "shift and finalize blocks share one launch");
+    // Only the launch overlaps the predecessor (post-physics): the plain shift reads nothing that kernel writes, but
+    // running this bandwidth-bound copy beside the latency-bound post-physics kernel was measured to cost more than
+    // it hides (+13 % step time at 65 536 envs), so the data movement starts after it.
     hb::pdl_trigger();
     hb::pdl_wait();              // post-physics complete: reset flags, ballots, sums
-    // the finalize blocks come FIRST in the grid: their short latency chain (ballot scan, ids, means) then runs
-    // under the shift instead of behind its last block
-    const uint32_t fin_blocks = gridDim.x - blocks_a - blocks_b;
-    if (blockIdx.x < fin_blocks) {
-        reset_finalize_body(p, b, nullptr, nullptr, tiles, seg, host_count, rng_counter, blockIdx.x, fin_blocks);
-    } else {
-        const uint32_t blk = blockIdx.x - fin_blocks;
-        if (blk < blocks_a) stack_shift_fixed<ROW_A, LD_A, FRAME_A, UNROLL, true>(prev_a, next_a, total_a, blk, b.reset_buf);
-        else stack_shift_fixed<ROW_B, LD_B, FRAME_B, UNROLL, true>(prev_b, next_b, total_b, blk - blocks_a, b.reset_buf);
-    }
-}
-
-// A frame stack whose ROW / LD / FRAME are not compile-time constants: any robot's frames, any stack depth.
-// inv_ld = ceil(2^64 / LD): for e < 2^32, e / LD = umul64hi(e, inv_ld) exactly (the error term e (inv_ld LD - 2^64) / 2^64
-// stays below 1), two wide multiplies instead of a division per vector.
-struct ShiftShape {
-    uint32_t row, ld, frame;
-    unsigned long long inv_ld;
-};
-
-__device__ __forceinline__ uint32_t div_ld(uint32_t e, const ShiftShape &sh) { return (uint32_t)__umul64hi(e, sh.inv_ld); }
-
-// stack_shift_fixed with the shape as arguments; reset_buf null: no zeroing
-template <int UNROLL>
-__device__ __forceinline__ void stack_shift_rt(const float *__restrict__ prev, float *__restrict__ next, const uint32_t total,
-                                               const uint32_t blk, const ShiftShape sh, const uint8_t *__restrict__ reset_buf) {
-    const uint32_t LD = sh.ld, KEEP = sh.row - sh.frame, ROT = sh.frame & 3u, FVEC = sh.frame >> 2;
-    const bool vec_rows = (LD & 3u) == 0;
-    const uint32_t lane = threadIdx.x & 31u;
-    const uint32_t total_vec = total >> 2;
-    const uint32_t tail_vec = (total + 3u) >> 2;
-    const uint32_t warp_base = (blk * blockDim.x + (threadIdx.x - lane)) * UNROLL;
-    const float4 *p4 = reinterpret_cast<const float4 *>(prev);
-    float4 *n4 = reinterpret_cast<float4 *>(next);
-    float4 v[UNROLL], w[UNROLL];
-    uint8_t rz[UNROLL];
-#pragma unroll
-    for (int u = 0; u < UNROLL; ++u) {
-        const uint32_t s = warp_base + u * 32u + lane + FVEC;
-        const uint32_t e = (warp_base + u * 32u + lane) * 4u;
-        const uint32_t r = div_ld(e, sh);
-        rz[u] = (reset_buf && e < total) ? __ldg(reset_buf + r) : 0;
-        w[u] = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (vec_rows) {
-            const bool need = e - r * LD < KEEP + 4u;
-            v[u] = hb::ld_stream4_if(p4 + s, need && s < total_vec);
-            if (ROT != 0) w[u] = hb::ld_stream4_if(p4 + s + 1u, need && lane == 31u && s + 1u < total_vec);
+    if constexpr (Fin::kOn) {
+        // the finalize blocks come FIRST in the grid: their short latency chain (ballot scan, ids, means) then runs
+        // under the shift instead of behind its last block
+        const uint32_t fin_blocks = gridDim.x - blocks_a - blocks_b;
+        if (blockIdx.x < fin_blocks) {
+            reset_finalize_body(fin.p, fin.b, nullptr, nullptr, fin.tiles, fin.seg, fin.host_count, fin.rng_counter, blockIdx.x,
+                                fin_blocks);
         } else {
-            v[u] = (s < total_vec) ? hb::ld_stream4(p4 + s) : ld_vec_guarded(prev, s, total);
-            if (ROT != 0 && lane == 31u)
-                w[u] = (s + 1u < total_vec) ? hb::ld_stream4(p4 + s + 1u) : ld_vec_guarded(prev, s + 1u, total);
+            const uint32_t blk = blockIdx.x - fin_blocks;
+            if (blk < blocks_a) stack_shift<SA, 4, true>(prev_a, next_a, total_a, blk, sa, fin.b.reset_buf);
+            else stack_shift<SB, 4, true>(prev_b, next_b, total_b, blk - blocks_a, sb, fin.b.reset_buf);
         }
-    }
-#pragma unroll
-    for (int u = 0; u < UNROLL; ++u) {
-        const uint32_t i = warp_base + u * 32u + lane;
-        float nx0 = __shfl_down_sync(0xffffffffu, v[u].x, 1);
-        float nx1 = __shfl_down_sync(0xffffffffu, v[u].y, 1);
-        float nx2 = __shfl_down_sync(0xffffffffu, v[u].z, 1);
-        if (lane == 31u) nx0 = w[u].x, nx1 = w[u].y, nx2 = w[u].z;
-        float4 o = v[u];
-        if (ROT == 1) o = make_float4(v[u].y, v[u].z, v[u].w, nx0);
-        else if (ROT == 2) o = make_float4(v[u].z, v[u].w, nx0, nx1);
-        else if (ROT == 3) o = make_float4(v[u].w, nx0, nx1, nx2);
-        if (i >= tail_vec) continue;
-        const uint32_t e0 = i * 4u;
-        const uint32_t r0 = div_ld(e0, sh);
-        const uint32_t c0 = e0 - r0 * LD;
-        if (vec_rows && c0 >= KEEP) continue;
-        if (c0 + 3u < KEEP && i < total_vec) {
-            if (rz[u]) o = make_float4(0.f, 0.f, 0.f, 0.f);
-            hb::st_stream4(n4 + i, o);
-        } else {
-            const float ov[4] = {o.x, o.y, o.z, o.w};
-#pragma unroll
-            for (uint32_t k = 0; k < 4u; ++k) {
-                uint32_t c = c0 + k, r = r0;
-                if (c >= LD) c -= LD, r += 1u;
-                const bool zero = reset_buf && (vec_rows ? rz[u] != 0 : reset_buf[r] != 0);
-                if (c < KEEP && e0 + k < total) next[e0 + k] = zero ? 0.0f : ov[k];
-            }
-        }
-    }
-}
-
-// stack_finalize_kernel for runtime shapes.  Without finalize blocks and with reset_buf null it is the plain shift of both
-// histories (hb_env_stack_observations).
-__global__ void __launch_bounds__(256, 4)
-stack_finalize_rt_kernel(const float *__restrict__ prev_a, float *__restrict__ next_a, uint32_t total_a, uint32_t blocks_a,
-                         const ShiftShape sa, const float *__restrict__ prev_b, float *__restrict__ next_b, uint32_t total_b,
-                         uint32_t blocks_b, const ShiftShape sb, const uint8_t *__restrict__ reset_buf,
-                         const __grid_constant__ hb_env_params p, const __grid_constant__ hb_env_buffers b, int tiles, int seg,
-                         int32_t *host_count, unsigned long long *rng_counter) {
-    hb::pdl_trigger();
-    hb::pdl_wait();
-    const uint32_t fin_blocks = gridDim.x - blocks_a - blocks_b;
-    if (blockIdx.x < fin_blocks) {
-        reset_finalize_body(p, b, nullptr, nullptr, tiles, seg, host_count, rng_counter, blockIdx.x, fin_blocks);
     } else {
-        const uint32_t blk = blockIdx.x - fin_blocks;
-        if (blk < blocks_a) stack_shift_rt<4>(prev_a, next_a, total_a, blk, sa, reset_buf);
-        else stack_shift_rt<4>(prev_b, next_b, total_b, blk - blocks_a, sb, reset_buf);
+        if (blockIdx.x < blocks_a) stack_shift<SA, 4, false>(prev_a, next_a, total_a, blockIdx.x, sa, nullptr);
+        else stack_shift<SB, 4, false>(prev_b, next_b, total_b, blockIdx.x - blocks_a, sb, nullptr);
     }
 }
 
@@ -1542,33 +1474,14 @@ struct StackShape {
 using ShapeHector = StackShape<41, 15, 70, 15>;
 using ShapeHectorFull = StackShape<65, 15, 94, 15>;
 using ShapeXBot = StackShape<47, 15, 73, 3>;
-constexpr int ROW_OBS = ShapeHector::ROW_A, ROW_PRIV = ShapeHector::ROW_B, OBS = 41, PRIV = 70;      // hb_stack_shift's fast paths
 
 template <typename S>
 struct DenseRows : S { static constexpr int LD_A = S::ROW_A, LD_B = S::ROW_B; };     // a built shape with dense rows
 
-// blocks of stack_shift_fixed (256 threads, 4 float4 each) over `total` floats
+// blocks of stack_shift (256 threads, 4 float4 each) over `total` floats
 uint32_t shift_blocks(uint32_t total) { return ((total + 3u) / 4u + 4 * 256 - 1) / (4 * 256); }
 
 bool fits_u32(int n, int row) { return (long long)n * row + 64 * 1024 < (1ll << 32); }
-
-int shift_any(const float *prev, float *next, const uint8_t *reset_buf, int num_envs, int row, int ld, int frame,
-              cudaStream_t st) {
-    HB_REQUIRE(prev && next && prev != next, "hb_stack_shift: null or aliasing buffers");
-    HB_REQUIRE(num_envs > 0 && frame > 0 && row > frame && ld >= row, "hb_stack_shift: bad shape");
-    const bool fast = !reset_buf && ld == row && hb::aligned16(prev) && hb::aligned16(next) && fits_u32(num_envs, row);
-    const uint32_t dense_total = (uint32_t)num_envs * row;
-    if (fast && row == ROW_OBS && frame == OBS) {
-        stack_shift_fixed_kernel<ROW_OBS, OBS, 4><<<shift_blocks(dense_total), 256, 0, st>>>(prev, next, dense_total);
-    } else if (fast && row == ROW_PRIV && frame == PRIV) {
-        stack_shift_fixed_kernel<ROW_PRIV, PRIV, 4><<<shift_blocks(dense_total), 256, 0, st>>>(prev, next, dense_total);
-    } else {
-        const long long total = (long long)num_envs * ld;
-        stack_shift_scalar_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(prev, next, reset_buf, total, row, ld, frame);
-    }
-    HB_CHECK_LAUNCH("stack_shift_kernel");
-    return HB_OK;
-}
 
 template <typename T, bool kBulk>
 int launch_post_physics(const hb_env_params *p, const hb_env_buffers *buf, const hb_env_noise *noise, float *obs_new,
@@ -1588,52 +1501,68 @@ int launch_post_physics(const hb_env_params *p, const hb_env_buffers *buf, const
     return HB_OK;
 }
 
-// The frame-stack shift of both histories: rows and pitches, built shape (0 hector, 1 hector_full, 2 XBot-L) and layout
-// (0 = not a built shape, 1 = dense rows, 2 = 128-byte pitch), and whether the fixed-shape kernels apply (fast) or else the
-// runtime-shape kernel (vec: 16-byte aligned buffers), with their grid
+// The frame-stack shift of both histories (a: actor, b: critic): shapes and grid, which built shape they are (0 hector,
+// 1 hector_full, 2 XBot-L) and in which layout (0 = not a built shape, 1 = dense rows, 2 = 128-byte pitch), and whether
+// the compiled kernel of that shape applies (fast) or else the runtime-shape kernel (vec: 16-byte aligned buffers).
+// reset_buf: the envs whose carried frames a shift without finalisation zeroes (null: none).
 struct StackPlan {
-    int row_a, row_b, ld_a, ld_b, shape, layout;
+    ShiftShape a, b;
+    int num_envs, shape, layout;
     bool fast, vec;
     uint32_t total_a, total_b, blocks_a, blocks_b;
+    const uint8_t *reset_buf;
 };
 
+// (ld 0: a stack of no frames in the caller's params, which shifts nothing - no reciprocal, no division by zero)
 ShiftShape shift_shape(int row, int ld, int frame) {
-    return {(uint32_t)row, (uint32_t)ld, (uint32_t)frame, ~0ull / (unsigned long long)ld + 1ull};
+    return {(uint32_t)row, (uint32_t)ld, (uint32_t)frame, ld > 0 ? ~0ull / (unsigned long long)ld + 1ull : 0ull};
 }
 
 template <typename S>
-int shape_layout(const StackPlan &s, const hb_env_params *p) {
-    if (s.row_a != S::ROW_A || p->num_single_obs != S::FRAME_A || s.row_b != S::ROW_B || p->num_single_priv != S::FRAME_B) return 0;
-    return s.ld_a == S::ROW_A && s.ld_b == S::ROW_B ? 1 : (s.ld_a == S::LD_A && s.ld_b == S::LD_B ? 2 : 0);
+int shape_layout(const StackPlan &s) {
+    if (s.a.row != S::ROW_A || s.a.frame != S::FRAME_A || s.b.row != S::ROW_B || s.b.frame != S::FRAME_B) return 0;
+    return s.a.ld == S::ROW_A && s.b.ld == S::ROW_B ? 1 : (s.a.ld == S::LD_A && s.b.ld == S::LD_B ? 2 : 0);
 }
 
-StackPlan stack_plan(const hb_env_params *p, const float *obs_prev, const float *priv_prev, const float *obs_new,
-                     const float *priv_new) {
+StackPlan stack_plan(int num_envs, ShiftShape a, ShiftShape b, bool aligned) {
     StackPlan s;
-    s.row_a = p->frame_stack * p->num_single_obs, s.row_b = p->c_frame_stack * p->num_single_priv;
-    s.ld_a = p->obs_ld ? p->obs_ld : s.row_a, s.ld_b = p->priv_ld ? p->priv_ld : s.row_b;
-    const int layouts[3] = {shape_layout<ShapeHector>(s, p), shape_layout<ShapeHectorFull>(s, p), shape_layout<ShapeXBot>(s, p)};
+    s.a = a, s.b = b, s.num_envs = num_envs, s.reset_buf = nullptr;
+    const int layouts[3] = {shape_layout<ShapeHector>(s), shape_layout<ShapeHectorFull>(s), shape_layout<ShapeXBot>(s)};
     s.shape = layouts[0] ? 0 : (layouts[1] ? 1 : 2);
     s.layout = layouts[s.shape];
-    s.vec = hb::aligned16(obs_prev) && hb::aligned16(obs_new) && hb::aligned16(priv_prev) && hb::aligned16(priv_new) &&
-            fits_u32(p->num_envs, s.ld_a > s.ld_b ? s.ld_a : s.ld_b);
+    s.vec = aligned && fits_u32(num_envs, a.ld > b.ld ? a.ld : b.ld);
     s.fast = s.vec && s.layout != 0;
-    s.total_a = (uint32_t)p->num_envs * s.ld_a, s.total_b = (uint32_t)p->num_envs * s.ld_b;
+    s.total_a = (uint32_t)num_envs * a.ld, s.total_b = (uint32_t)num_envs * b.ld;
     // a stack of one frame carries nothing over: no shift blocks
-    s.blocks_a = s.row_a > p->num_single_obs ? shift_blocks(s.total_a) : 0;
-    s.blocks_b = s.row_b > p->num_single_priv ? shift_blocks(s.total_b) : 0;
+    s.blocks_a = a.row > a.frame ? shift_blocks(s.total_a) : 0;
+    s.blocks_b = b.row > b.frame ? shift_blocks(s.total_b) : 0;
     return s;
 }
 
-// The fixed-shape kernel of a fast plan: instantiate(R{}) with R = the StackShape (pitched rows) or its DenseRows, whose
-// ROW / LD / FRAME constants are the kernel's template arguments
-template <typename F>
-auto stack_kernel(const StackPlan &s, F &&instantiate) {
-    auto rows = [&](auto shape) {
-        using S = decltype(shape);
-        return s.layout == 2 ? instantiate(S{}) : instantiate(DenseRows<S>{});
-    };
-    return s.shape == 0 ? rows(ShapeHector{}) : (s.shape == 1 ? rows(ShapeHectorFull{}) : rows(ShapeXBot{}));
+// The env's two histories
+StackPlan stack_plan(const hb_env_params *p, const float *obs_prev, const float *priv_prev, const float *obs_new,
+                     const float *priv_new) {
+    const int row_a = p->frame_stack * p->num_single_obs, row_b = p->c_frame_stack * p->num_single_priv;
+    return stack_plan(p->num_envs, shift_shape(row_a, p->obs_ld ? p->obs_ld : row_a, p->num_single_obs),
+                      shift_shape(row_b, p->priv_ld ? p->priv_ld : row_b, p->num_single_priv),
+                      hb::aligned16(obs_prev) && hb::aligned16(obs_new) && hb::aligned16(priv_prev) && hb::aligned16(priv_new));
+}
+
+// One dense history (hb_stack_shift), in slot b if it has the shape of hector's critic history, else in slot a; the other
+// slot is empty.  Hector's two dense histories, without reset flags, run the compiled kernel of hector's dense stack.
+StackPlan stack_plan(int num_envs, int row, int frame, bool aligned, const uint8_t *reset_buf) {
+    using H = DenseRows<ShapeHector>;
+    const bool in_b = row == H::ROW_B && frame == H::FRAME_B;
+    StackPlan s = {};
+    (in_b ? s.b : s.a) = shift_shape(row, row, frame);
+    const uint32_t total = (uint32_t)num_envs * row;
+    (in_b ? s.total_b : s.total_a) = total;
+    (in_b ? s.blocks_b : s.blocks_a) = shift_blocks(total);
+    s.num_envs = num_envs, s.reset_buf = reset_buf;
+    s.shape = 0, s.layout = in_b || (row == H::ROW_A && frame == H::FRAME_A) ? 1 : 0;
+    s.vec = aligned && fits_u32(num_envs, row);
+    s.fast = s.vec && s.layout != 0 && !reset_buf;
+    return s;
 }
 
 // Grid of the shard-wide reset finalisation: each CTA owns a contiguous segment of at least 8 32-env tiles
@@ -1646,19 +1575,55 @@ FinalizeGrid finalize_grid(int num_envs) {
     return {tiles, seg, (tiles + seg - 1) / seg};
 }
 
-// stack_finalize_rt_kernel: both shifts and, with `finalize`, the reset finalisation (ids, means, history zeroing)
-int launch_stack_rt(const hb_env_params *p, const hb_env_buffers *buf, const StackPlan &s, const float *obs_prev,
-                    const float *priv_prev, float *obs_new, float *priv_new, bool finalize, int32_t *host_count,
-                    uint64_t *rng_counter, cudaStream_t st) {
-    const FinalizeGrid g = finalize_grid(p->num_envs);
-    const uint32_t fin_blocks = finalize ? (uint32_t)g.blocks : 0u;
+// The frame-stack launch of plan s: the compiled kernel of a built shape (fast), else the runtime-shape kernel (vec),
+// else the scalar shift of each history.  With `finalize` the reset finalisation of p / buf runs too: in the same grid,
+// its blocks first, or behind the scalar shift as reset_finalize_kernel.  p null: a lone shift (hb_stack_shift), launched
+// without PDL.
+int launch_stack(const hb_env_params *p, const hb_env_buffers *buf, const StackPlan &s, const float *prev_a, const float *prev_b,
+                 float *next_a, float *next_b, bool finalize, int32_t *host_count, uint64_t *rng_counter, cudaStream_t st) {
+    if (!s.vec) {           // unaligned or oversized buffers
+        const ShiftShape *sh[2] = {&s.a, &s.b};
+        const float *prev[2] = {prev_a, prev_b};
+        float *next[2] = {next_a, next_b};
+        for (int h = 0; h < 2; ++h) {
+            if (sh[h]->row <= sh[h]->frame) continue;       // carries nothing over (the block counts may have wrapped here)
+            const long long total = (long long)s.num_envs * sh[h]->ld;
+            stack_shift_scalar_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(prev[h], next[h], s.reset_buf, total,
+                                                                                       sh[h]->row, sh[h]->ld, sh[h]->frame);
+            HB_CHECK_LAUNCH("stack_shift_scalar_kernel");
+        }
+        return finalize ? hb_env_reset_finalize(p, buf, next_a, next_b, host_count, rng_counter, st) : HB_OK;
+    }
+    FinalizeArgs fin = {};
+    uint32_t fin_blocks = 0;
+    if (finalize) {
+        const FinalizeGrid g = finalize_grid(s.num_envs);
+        fin = {*p, *buf, g.tiles, g.seg, host_count, reinterpret_cast<unsigned long long *>(rng_counter)};
+        fin_blocks = (uint32_t)g.blocks;
+    } else {
+        fin.b.reset_buf = const_cast<uint8_t *>(s.reset_buf);      // the runtime-shape kernel's zeroing (only read)
+    }
     if (s.blocks_a + s.blocks_b + fin_blocks == 0) return HB_OK;
-    HB_CUDA(hb::launch_pdl(hb::use_pdl_stack(p->num_envs), stack_finalize_rt_kernel, dim3(fin_blocks + s.blocks_a + s.blocks_b),
-                           dim3(256), 0, st, obs_prev, obs_new, s.total_a, s.blocks_a, shift_shape(s.row_a, s.ld_a, p->num_single_obs),
-                           priv_prev, priv_new, s.total_b, s.blocks_b, shift_shape(s.row_b, s.ld_b, p->num_single_priv),
-                           finalize ? (const uint8_t *)buf->reset_buf : nullptr, *p, *buf, g.tiles, g.seg, host_count,
-                           reinterpret_cast<unsigned long long *>(rng_counter)));
-    HB_CHECK_LAUNCH("stack_finalize_rt_kernel");
+    const bool pdl_stack = p && hb::use_pdl_stack(s.num_envs);
+    auto launch = [&](auto kernel, bool pdl, auto fin_, auto sa, auto sb) {
+        return hb::launch_pdl(pdl, kernel, dim3(fin_blocks + s.blocks_a + s.blocks_b), dim3(256), 0, st, prev_a, next_a, s.total_a,
+                              s.blocks_a, prev_b, next_b, s.total_b, s.blocks_b, fin_, sa, sb);
+    };
+    // a built shape: the kernel whose FixedShift constants are its StackShape (pitched rows) or DenseRows
+    auto built = [&](auto shape) {
+        using R = decltype(shape);
+        using A = FixedShift<R::ROW_A, R::LD_A, R::FRAME_A>;
+        using B = FixedShift<R::ROW_B, R::LD_B, R::FRAME_B>;
+        return finalize ? launch(stack_shift_kernel<A, B, FinalizeArgs>, pdl_stack, fin, A{}, B{})
+                        : launch(stack_shift_kernel<A, B, NoFinalize>, p && hb::use_pdl(s.num_envs), NoFinalize{}, A{}, B{});
+    };
+    auto rows = [&](auto shape) {
+        using S = decltype(shape);
+        return s.layout == 2 ? built(S{}) : built(DenseRows<S>{});
+    };
+    HB_CUDA(!s.fast ? launch(stack_shift_kernel<ShiftShape, ShiftShape, FinalizeArgs>, pdl_stack, fin, s.a, s.b)
+                    : (s.shape == 0 ? rows(ShapeHector{}) : (s.shape == 1 ? rows(ShapeHectorFull{}) : rows(ShapeXBot{}))));
+    HB_CHECK_LAUNCH("stack_shift_kernel");
     return HB_OK;
 }
 
@@ -1889,7 +1854,12 @@ int hb_env_get_heights(const float *root_states, const float *points_xy, int32_t
 
 int hb_stack_shift(const float *prev, float *next, const uint8_t *reset_buf, int32_t num_envs, int32_t row,
                    int32_t frame, void *stream) {
-    return shift_any(prev, next, reset_buf, num_envs, row, row, frame, (cudaStream_t)stream);
+    HB_REQUIRE(prev && next && prev != next, "hb_stack_shift: null or aliasing buffers");
+    HB_REQUIRE(num_envs > 0 && frame > 0 && row > frame, "hb_stack_shift: bad shape");
+    const StackPlan s = stack_plan(num_envs, row, frame, hb::aligned16(prev) && hb::aligned16(next), reset_buf);
+    const bool in_b = s.b.row != 0;                     // the history went to slot b
+    return launch_stack(nullptr, nullptr, s, in_b ? nullptr : prev, in_b ? prev : nullptr, in_b ? nullptr : next,
+                        in_b ? next : nullptr, false, nullptr, nullptr, (cudaStream_t)stream);
 }
 
 int hb_env_stack_observations(const hb_env_params *p, const hb_env_buffers *buf, const float *obs_prev,
@@ -1897,23 +1867,8 @@ int hb_env_stack_observations(const hb_env_params *p, const hb_env_buffers *buf,
     if (int rc = check_params(p, buf, "hb_env_stack_observations")) return rc;
     HB_REQUIRE(obs_prev && priv_prev && obs_new && priv_new, "hb_env_stack_observations: null buffer");
     HB_REQUIRE(obs_prev != obs_new && priv_prev != priv_new, "hb_env_stack_observations: prev and new must not alias");
-    cudaStream_t st = (cudaStream_t)stream;
-    const StackPlan s = stack_plan(p, obs_prev, priv_prev, obs_new, priv_new);
-    if (s.fast) {
-        auto kernel = stack_kernel(s, [](auto rows) {
-            using R = decltype(rows);
-            return stack_shift_pair_kernel<R::ROW_A, R::LD_A, R::FRAME_A, R::ROW_B, R::LD_B, R::FRAME_B, 4>;
-        });
-        HB_CUDA(hb::launch_pdl(hb::use_pdl(p->num_envs), kernel, dim3(s.blocks_a + s.blocks_b), dim3(256), 0, st, obs_prev, obs_new,
-                               s.total_a, s.blocks_a, priv_prev, priv_new, s.total_b));
-        HB_CHECK_LAUNCH("stack_shift_pair_kernel");
-        return HB_OK;
-    }
-    if (s.vec) return launch_stack_rt(p, buf, s, obs_prev, priv_prev, obs_new, priv_new, false, nullptr, nullptr, st);
-    if (s.blocks_a)
-        if (int rc = shift_any(obs_prev, obs_new, nullptr, p->num_envs, s.row_a, s.ld_a, p->num_single_obs, st)) return rc;
-    if (s.blocks_b) return shift_any(priv_prev, priv_new, nullptr, p->num_envs, s.row_b, s.ld_b, p->num_single_priv, st);
-    return HB_OK;
+    return launch_stack(p, buf, stack_plan(p, obs_prev, priv_prev, obs_new, priv_new), obs_prev, priv_prev, obs_new, priv_new,
+                        false, nullptr, nullptr, (cudaStream_t)stream);
 }
 
 int hb_env_stack_finalize(const hb_env_params *p, const hb_env_buffers *buf, const float *obs_prev, const float *priv_prev,
@@ -1923,23 +1878,8 @@ int hb_env_stack_finalize(const hb_env_params *p, const hb_env_buffers *buf, con
     HB_REQUIRE(obs_prev != obs_new && priv_prev != priv_new, "hb_env_stack_finalize: prev and new must not alias");
     HB_REQUIRE(buf->scratch_ballots && buf->scratch_sums && buf->reset_env_ids && buf->reset_count && buf->episode_means,
                "hb_env_stack_finalize: null scratch/result buffers");
-    const StackPlan s = stack_plan(p, obs_prev, priv_prev, obs_new, priv_new);
-    if (!s.fast && s.vec)
-        return launch_stack_rt(p, buf, s, obs_prev, priv_prev, obs_new, priv_new, true, host_count, rng_counter, (cudaStream_t)stream);
-    if (!s.fast) {        // unaligned or oversized buffers: the two separate launches
-        if (int rc = hb_env_stack_observations(p, buf, obs_prev, priv_prev, obs_new, priv_new, stream)) return rc;
-        return hb_env_reset_finalize(p, buf, obs_new, priv_new, host_count, rng_counter, stream);
-    }
-    const FinalizeGrid g = finalize_grid(p->num_envs);
-    auto kernel = stack_kernel(s, [](auto rows) {
-        using R = decltype(rows);
-        return stack_finalize_kernel<R::ROW_A, R::LD_A, R::FRAME_A, R::ROW_B, R::LD_B, R::FRAME_B, 4>;
-    });
-    HB_CUDA(hb::launch_pdl(hb::use_pdl_stack(p->num_envs), kernel, dim3(s.blocks_a + s.blocks_b + (uint32_t)g.blocks), dim3(256), 0,
-                           (cudaStream_t)stream, obs_prev, obs_new, s.total_a, s.blocks_a, priv_prev, priv_new, s.total_b, s.blocks_b,
-                           *p, *buf, g.tiles, g.seg, host_count, reinterpret_cast<unsigned long long *>(rng_counter)));
-    HB_CHECK_LAUNCH("stack_finalize_kernel");
-    return HB_OK;
+    return launch_stack(p, buf, stack_plan(p, obs_prev, priv_prev, obs_new, priv_new), obs_prev, priv_prev, obs_new, priv_new,
+                        true, host_count, rng_counter, (cudaStream_t)stream);
 }
 
 int hb_env_mirror_frames(const float *obs, int32_t obs_ld, int32_t obs_row, int32_t obs_frame, const float *priv, int32_t priv_ld,

@@ -1,4 +1,4 @@
-"""A few eager env steps at [envs] for ncu (-k regex:"post_physics|stack_finalize"): python scripts/profile_env_step.py [envs]"""
+"""A few eager env steps at [envs] for ncu (-k regex:"post_physics|stack_shift_kernel"): python scripts/profile_env_step.py [envs]"""
 import os
 import sys
 

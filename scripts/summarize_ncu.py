@@ -30,7 +30,8 @@ def raw(src, dst):
            f"{'kernel':78s} " + " ".join(f"{t:>9s}" for _, t in keys)]
     traffic = {}
     for r in body:
-        name = short(r[col["Kernel Name"]])
+        full = r[col["Kernel Name"]]
+        name = short(full)
         vals = []
         for k, t in keys:
             v = r[col[k]]
@@ -44,7 +45,7 @@ def raw(src, dst):
             except ValueError:
                 vals.append(f"{v:>9s}")
         out.append(f"{name:78s} " + " ".join(vals))
-        if name.startswith("stack_finalize_kernel"):
+        if "stack_shift_kernel" in full and "FixedShift" in full and "FinalizeArgs" in full:      # the step's compiled stack launch
             rd, wr = float(r[col["dram__bytes_read.sum"]]), float(r[col["dram__bytes_write.sum"]])
             scale = {"Mbyte": 1e6, "Kbyte": 1e3, "byte": 1.0, "Gbyte": 1e9}
             traffic = {"dram_bytes_read": rd * scale.get(units[col["dram__bytes_read.sum"]], 1.0),
