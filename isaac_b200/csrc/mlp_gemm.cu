@@ -492,6 +492,19 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_consta
                             for (int k = 0; k < 4; ++k) v[4 * j + k] *= hb::act_grad<ACT>(h[k]);
                         }
                     }
+                    if ((g.N & 3) && n + 32 > g.N) {
+                        // The TMA store writes whole 16-byte chunks: the chunk holding column N - 1 would also overwrite the
+                        // columns behind it up to the next multiple of 4, which belong to the caller (the ones column
+                        // behind an MLP's hidden activations).  A block whose ragged edge falls inside a chunk is stored
+                        // per lane instead.
+                        if (mw + lane < g.M) {
+                            float *drow = g.D + (size_t)(mw + lane) * g.ldd + n;
+#pragma unroll
+                            for (int j = 0; j < 32; ++j)
+                                if (n + j < g.N) drow[j] = v[j];
+                        }
+                        continue;
+                    }
                     if (lane == 0) tma_store_wait_read();        // the previous block's store has read the tile
                     __syncwarp();
 #pragma unroll
@@ -771,8 +784,14 @@ int launch_auto(const hb_gemm_desc *d, const hb_gemm_desc *d1, cudaStream_t st) 
 template <int BN, int EPI>
 int dispatch_major(const hb_gemm_desc *d, const hb_gemm_desc *d1, cudaStream_t st) {
     if (!d->a_mn_major && !d->b_mn_major) return launch_auto<BN, false, false, EPI>(d, d1, st);
-    if (!d->a_mn_major && d->b_mn_major) return launch_auto<BN, false, true, EPI>(d, d1, st);
-    if (d->a_mn_major && d->b_mn_major) return launch_auto<BN, true, true, EPI>(d, d1, st);
+    if (d->b_mn_major) {
+        if constexpr (BN < 128) {      // only N <= 64 picks these widths, and check_desc refuses an MN-major B there: not built
+            hb::set_error("hb_gemm_tf32: MN-major B needs N > 64");
+            return HB_ERR_BAD_ARG;
+        } else {
+            return d->a_mn_major ? launch_auto<BN, true, true, EPI>(d, d1, st) : launch_auto<BN, false, true, EPI>(d, d1, st);
+        }
+    }
     hb::set_error("hb_gemm_tf32: A MN-major with B K-major is not instantiated");
     return HB_ERR_UNSUPPORTED;
 }
