@@ -309,16 +309,34 @@ pd_torque_scalar_kernel(const float *__restrict__ dof_state, const float *__rest
 // per env is a quarter of the fused version, and each warp only fetches its own slice of code.
 // Phase A (rewards, reset flag) | barrier | phase B (reset_idx effects, newest frames, write-back)
 // | barrier | coalesced store of the frames.
+//
+// post_physics_wide_kernel: eight warps, each role a pair of halves (warps 0-2 the first halves of base / joints / feet, 3-5 their second
+// halves, 6-7 the ledger pair).  At one or two tiles per SM nothing hides a warp's dependent chain, so the pair splits
+// it.  The split is by term: every reward term, frame column, write-back and draw is computed by one half with exactly
+// the four-warp kernel's operations (values both halves need are computed by both, the same way), so the two widths
+// write bit-identical results.
+//   base    first: base_lin/ang_vel, projected_gravity, euler, orientation, vel_mismatch_exp and their columns
+//           second: command resampling + heading, push, base_acc, tracking_*, track_vel_hard, low_speed, the root and
+//           command write-back and columns
+//   joints  first: action_smoothness, default_joint_pos, joint_pos; after barrier 1 the reset of the dofs, the
+//           reference trajectory and the privileged columns
+//           second: dof_acc, dof_vel, torques, the last_* roll-forward; after barrier 1 the noisy observation columns
+//   feet    first: termination, gait, feet_air_time, feet_contact_forces, feet_contact_number, foot_slip, the reset
+//           flag and the episode / contact state
+//           second: collision, base_height, feet_clearance (and its state), feet_distance, knee_distance, the columns
+//   ledger  first: the alphabetical reward sum; second: the episode sums and their reset-env means; both: the noise
 // ------------------------------------------------------------------------------------------
 struct TileLayout {          // float offsets into the CTA's shared-memory tile
     int root, dof, contact, actions, last_actions, last_last_actions, last_dof_vel, torques, last_root_vel,
-        commands, z_obs, terms, gait_s, gait_c, flags, so, sp, total;
+        commands, z_obs, terms, gait_s, gait_c, flags, rsums, so, sp, total;
 };
 
 // The staged inputs are dead once every role has passed barrier 1 (each lane keeps its env's values in
 // registers), so the newest-frame staging tiles so/sp reuse the same bytes: ~19 KB per CTA instead of
 // ~38 KB, which is what bounds the number of resident tiles per SM.
-__host__ __device__ constexpr TileLayout make_layout(int nbody, bool with_noise, int NDOF, int OBS, int PRIV) {
+// The wide kernel's ledger pair keeps the reset envs' episode sums apart from the terms (rsums), which the other half
+// is still reading.
+__host__ __device__ constexpr TileLayout make_layout(int nbody, bool with_noise, int NDOF, int OBS, int PRIV, bool wide = false) {
     TileLayout L{};
     int o = 0;
     L.root = o, o += TILE * 13;
@@ -340,6 +358,7 @@ __host__ __device__ constexpr TileLayout make_layout(int nbody, bool with_noise,
     L.gait_s = o, o += TILE;
     L.gait_c = o, o += TILE;
     L.flags = o, o += TILE;
+    L.rsums = o, o += wide ? HB_NUM_REWARDS * TILE : 0;
     L.total = o;
     return L;
 }
@@ -347,11 +366,21 @@ __host__ __device__ constexpr TileLayout make_layout(int nbody, bool with_noise,
 // XBot-L privileged frame, 32 bodies, observation noise)
 constexpr int POST_SMEM_MAX = 96 * 1024;
 static_assert(make_layout(32, true, MAX_TASK_DOF, task_dims(MAX_TASK_DOF, KIND_XBOT, 0, 0, 0, 0).OBS,
-                          task_dims(MAX_TASK_DOF, KIND_XBOT, 0, 0, 0, 0).PRIV).total * 4 <= POST_SMEM_MAX,
+                          task_dims(MAX_TASK_DOF, KIND_XBOT, 0, 0, 0, 0).PRIV, true).total * 4 <= POST_SMEM_MAX,
               "the largest task's tile fits the dynamic shared memory of post_physics_kernel");
 
-// all four warps of the tile (named barrier 1: the roles meet at different program points)
-__device__ __forceinline__ void tile_barrier() { asm volatile("bar.sync 1, 128;" ::: "memory"); }
+// a compile-time flag passed as an argument (which halves of its role a post_physics_kernel warp computes)
+template <bool V>
+struct On {
+    __device__ constexpr operator bool() const { return V; }
+};
+
+// all warps of the tile (named barrier 1: the roles meet at different program points)
+template <bool kWide = false>
+__device__ __forceinline__ void tile_barrier() {
+    if constexpr (kWide) asm volatile("bar.sync 1, 256;" ::: "memory");
+    else asm volatile("bar.sync 1, 128;" ::: "memory");
+}
 
 __device__ __forceinline__ float norm3(const float *f) { return sqrtf((f[0] * f[0] + f[1] * f[1]) + f[2] * f[2]); }
 
@@ -381,8 +410,9 @@ __device__ __noinline__ Vec3 euler_xyz_wrapped_nl(float x, float y, float z, flo
 }
 
 #ifdef HB_POST_TIMING
-// debug build: per-(tile, warp) SM-clock stamps at the phase boundaries of post_physics_kernel
-__device__ long long g_post_stamps[4096 * 4 * 8];
+// debug build: per-(tile, warp) SM-clock stamps at the phase boundaries of post_physics_kernel (8 warp rows per tile:
+// the four-warp kernel fills the first four)
+__device__ long long g_post_stamps[4096 * 8 * 8];
 __device__ unsigned long long g_post_gt[4096 * 3];          // globaltimer ns: CTA start, stores done, tail done
 __device__ __forceinline__ unsigned long long gtime() {
     unsigned long long t;
@@ -395,7 +425,7 @@ __device__ __forceinline__ unsigned long long gtime() {
     } while (0)
 #define HB_STAMP(slot)                                                                                   \
     do {                                                                                                 \
-        if (lane == 0 && blockIdx.x < 4096) g_post_stamps[(blockIdx.x * 4 + warp) * 8 + (slot)] = clock64(); \
+        if (lane == 0 && blockIdx.x < 4096) g_post_stamps[(blockIdx.x * 8 + warp) * 8 + (slot)] = clock64(); \
     } while (0)
 #else
 #define HB_STAMP(slot) do { } while (0)
@@ -1076,6 +1106,732 @@ post_physics_kernel(const __grid_constant__ hb_env_params p, const __grid_consta
     HB_GT(1);
 }
 
+// The eight-warp kernel (described above): the roles' code of post_physics_kernel with each term under the flag of the half
+// that computes it.  It runs where at most a few tiles share an SM: its register budget is that of two resident tiles.
+template <bool kBulk, typename T>
+__global__ void __launch_bounds__(8 * TILE, 2)
+post_physics_wide_kernel(const __grid_constant__ hb_env_params p, const __grid_constant__ hb_env_buffers b,
+                    const __grid_constant__ hb_env_noise nz, float *__restrict__ obs_new,
+                    float *__restrict__ priv_new, int stages) {
+    constexpr int KIND = T::KIND, CAP = T::CAP;
+    const auto D = T::dims(p);      // (the three robots: every D.X below is a constant expression)
+    const int NDOF = D.NDOF, OBS = D.OBS, PRIV = D.PRIV, PRIV_PAD = D.PRIV, U_RESET = D.U_RESET;
+    extern __shared__ __align__(128) float sm[];
+    __shared__ __align__(8) uint64_t bar;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int role = warp < 6 ? warp % 3 : 3;      // 0 base, 1 joints, 2 feet, 3 ledger
+    const bool second = warp < 6 ? warp >= 3 : warp == 7;      // the warp runs its role's second half
+    // A role body takes (h0, h1): whether it computes its role's first / second half of the terms, as compile-time
+    // constants so that each half's code is compiled on its own
+    auto run = [&](auto &&body) {
+        if (!second) body(On<true>{}, On<false>{});
+        else body(On<false>{}, On<true>{});
+    };
+    const int N = p.num_envs;
+    const int env0 = blockIdx.x * TILE;
+    const int nv = min(TILE, N - env0);
+    const int env = env0 + lane;
+    const bool valid = lane < nv;
+    const int ln = valid ? lane : 0;
+    // HB_STAGE_STEP is the whole of post_physics_step in one launch; the finer bits run one of the reference's hooks on
+    // its own (check_termination, compute_reward, compute_observations, and the head / tail of post_physics_step), so that
+    // a host that calls - or overrides - them one by one gets the same buffers as the fused launch
+    const bool do_step = stages & HB_STAGE_STEP;
+    const bool do_prepare = do_step || (stages & HB_STAGE_PREPARE);
+    const bool do_term = do_step || (stages & HB_STAGE_TERMINATION);
+    const bool do_rew = do_step || (stages & HB_STAGE_REWARD);
+    const bool do_last = do_step || (stages & HB_STAGE_LAST);
+    const bool derive = do_prepare || (stages & HB_STAGE_DERIVE);
+    const bool emit_obs = do_step || (stages & HB_STAGE_OBS);
+    const bool any_reset = do_step || (stages & (HB_STAGE_RESET_ALL | HB_STAGE_RESET_MASK));
+    const Rng rng = make_rng(nz);
+    const bool with_noise = p.add_noise && (nz.z_obs != nullptr || rng.on);
+    const bool tape_noise = p.add_noise && nz.z_obs != nullptr;
+    HB_STAMP(0);
+    HB_GT(0);
+    const TileLayout L = make_layout(p.num_bodies, with_noise, NDOF, OBS, PRIV, true);
+    const int crow = p.num_bodies * 3;
+    const float dt = p.dt;
+    const float clip = p.clip_observations;
+    float *terms = sm + L.terms;
+    float *so = sm + L.so, *sp = sm + L.sp;
+    // obs_now = frame + (randn * noise_scale_vec) * noise_level, then the +-clip of step() (hector_env.py:241-243,
+    // legged_robot.py:104-105); k is a compile-time column after unrolling
+    auto noisy_clip = [&](float v, int k) {
+        if (with_noise) v = v + (sm[L.z_obs + ln * OBS + k] * p.noise_scale_vec[k]) * p.noise_level;
+        return clampf(v, -clip, clip);
+    };
+    int *flags = reinterpret_cast<int *>(sm + L.flags);
+
+    // ---------------- stage the tile's input slabs into shared memory ----------------
+    hb::pdl_trigger();
+    hb::pdl_wait();              // everything above overlapped the tail of the last PD sub-step
+    const size_t e0 = env0;
+    const bool full = (nv == TILE);
+    const bool bulk = kBulk && full;
+    if (bulk && threadIdx.x == 0) {
+        hb::mbar_init(&bar, 1);
+        hb::fence_mbar_init();
+        hb::mbar_expect_tx(&bar, TILE * 4u * (13 + 2 * NDOF + crow + 5 * NDOF + 6 + 4 + (tape_noise ? OBS : 0)));
+    }
+    auto stage = [&](const float *src, int dst, int row) {
+        if (bulk) {
+            if (threadIdx.x == 0) hb::bulk_g2s(sm + dst, src, TILE * 4u * row, &bar);
+        } else {
+            const int count = nv * row;
+            for (int k = threadIdx.x; k < count; k += blockDim.x) sm[dst + k] = __ldg(src + k);
+        }
+    };
+    stage(b.root_states + e0 * 13, L.root, 13);
+    stage(b.dof_state + e0 * NDOF * 2, L.dof, NDOF * 2);
+    stage(b.contact_forces + e0 * crow, L.contact, crow);
+    stage(b.actions + e0 * NDOF, L.actions, NDOF);
+    stage(b.last_actions + e0 * NDOF, L.last_actions, NDOF);
+    stage(b.last_last_actions + e0 * NDOF, L.last_last_actions, NDOF);
+    stage(b.last_dof_vel + e0 * NDOF, L.last_dof_vel, NDOF);
+    stage(b.torques + e0 * NDOF, L.torques, NDOF);
+    stage(b.last_root_vel + e0 * 6, L.last_root_vel, 6);
+    stage(b.commands + e0 * 4, L.commands, 4);
+    if (tape_noise) stage(nz.z_obs + e0 * OBS, L.z_obs, OBS);
+
+    __syncthreads();                             // mbarrier init / plain staging visible to every warp
+    // Each role first issues its own global loads (they overlap the bulk copies), then waits for the tile.
+
+    // =========================================================================================
+    auto base = [&](auto h0, auto h1) {
+        long long ep_len = 0;
+        float push_f[2] = {0.f, 0.f}, push_t[3] = {0.f, 0.f, 0.f};
+        if (h1 && valid) {
+            ep_len = b.episode_length_buf[env];
+            push_f[0] = b.rand_push_force[env * 3], push_f[1] = b.rand_push_force[env * 3 + 1];
+#pragma unroll
+            for (int k = 0; k < 3; ++k) push_t[k] = b.rand_push_torque[env * 3 + k];
+        }
+        if (bulk) hb::mbar_wait(&bar, 0);
+        HB_STAMP(1);
+        float root[13], cmd[4];
+#pragma unroll
+        for (int k = 0; k < 13; ++k) root[k] = sm[L.root + ln * 13 + k];
+#pragma unroll
+        for (int k = 0; k < 4; ++k) cmd[k] = sm[L.commands + ln * 4 + k];
+        Vec3 lin = {0.f, 0.f, 0.f}, ang = {0.f, 0.f, 0.f}, grav = {0.f, 0.f, 0.f}, eul = {0.f, 0.f, 0.f};
+        const float *quat = root + 3;
+        if (derive) {        // legged_robot.py:127-135 (and _init_buffers :452,477-479)
+            lin = quat_rotate_inverse(quat, {root[7], root[8], root[9]});
+            ang = quat_rotate_inverse(quat, {root[10], root[11], root[12]});
+            grav = quat_rotate_inverse(quat, {0.0f, 0.0f, -1.0f});
+        } else if (valid) {  // reset / observation-only pass: keep the stored values
+            lin = {b.base_lin_vel[env * 3], b.base_lin_vel[env * 3 + 1], b.base_lin_vel[env * 3 + 2]};
+            ang = {b.base_ang_vel[env * 3], b.base_ang_vel[env * 3 + 1], b.base_ang_vel[env * 3 + 2]};
+            grav = {b.projected_gravity[env * 3], b.projected_gravity[env * 3 + 1], b.projected_gravity[env * 3 + 2]};
+        }
+        if (h0) eul = euler_xyz_wrapped_nl(quat[0], quat[1], quat[2], quat[3]);
+        if (h1 && do_prepare) {
+            ep_len += 1;
+            // -------- _post_physics_step_callback, legged_robot.py:303-335 --------
+            if (valid && (ep_len % p.resample_interval) == 0 && (nz.u_cmd || rng.on)) {
+                float u[3];
+                if (nz.u_cmd) u[0] = nz.u_cmd[(size_t)env * 3], u[1] = nz.u_cmd[(size_t)env * 3 + 1], u[2] = nz.u_cmd[(size_t)env * 3 + 2];
+                else rng_uniforms(rng, env, SLOT_U_CMD, 0, 3, u);
+                cmd[0] = p.cmd_span[0] * u[0] + p.cmd_lo[0];
+                cmd[1] = p.cmd_span[1] * u[1] + p.cmd_lo[1];
+                cmd[3] = p.cmd_span[2] * u[2] + p.cmd_lo[2];
+                const float keep = (sqrtf(cmd[0] * cmd[0] + cmd[1] * cmd[1]) > 0.2f) ? 1.0f : 0.0f;
+                cmd[0] *= keep, cmd[1] *= keep;
+            }
+            if (p.heading_command) {
+                const Vec3 fwd = quat_apply(quat, {1.0f, 0.0f, 0.0f});
+                const float heading = atan2f(fwd.y, fwd.x);
+                float e = mod_two_pi(cmd[3] - heading);                 // wrap_to_pi, utils/math.py:46-49
+                e = e - TWO_PI_F * ((e > PI_F) ? 1.0f : 0.0f);
+                cmd[2] = clampf(0.5f * e, -1.0f, 1.0f);
+            }
+            if ((stages & HB_STAGE_PUSH) && valid && (nz.u_push || rng.on)) {       // _push_robots, hector_env.py:53-68
+                float u[5];
+                if (nz.u_push) {
+#pragma unroll
+                    for (int k = 0; k < 5; ++k) u[k] = nz.u_push[(size_t)env * 5 + k];
+                } else {
+                    rng_uniforms(rng, env, SLOT_U_PUSH, 0, 5, u);
+                }
+                push_f[0] = p.push_lin_span * u[0] + p.push_lin_lo;
+                push_f[1] = p.push_lin_span * u[1] + p.push_lin_lo;
+                root[7] = push_f[0], root[8] = push_f[1];
+#pragma unroll
+                for (int k = 0; k < 3; ++k) {
+                    push_t[k] = p.push_ang_span * u[2 + k] + p.push_ang_lo;
+                    root[10 + k] = push_t[k];
+                }
+                b.rand_push_force[env * 3] = push_f[0], b.rand_push_force[env * 3 + 1] = push_f[1];
+#pragma unroll
+                for (int k = 0; k < 3; ++k) b.rand_push_torque[env * 3 + k] = push_t[k];
+            }
+        }
+        if (do_rew) {
+            if (h1) {   // base_acc, hector_env.py:385-392 (root velocity after the push)
+                float ss = 0.f;
+#pragma unroll
+                for (int k = 0; k < 6; ++k) {
+                    const float d = sm[L.last_root_vel + ln * 6 + k] - root[7 + k];
+                    ss += d * d;
+                }
+                terms[HB_R_BASE_ACC * TILE + lane] = expf(-sqrtf(ss) * 3.0f);
+            }
+            if (h0) {   // orientation, :341-348
+                const float a = expf(-(fabsf(eul.x) + fabsf(eul.y)) * 10.0f);
+                const float g = expf(-sqrtf(grav.x * grav.x + grav.y * grav.y) * 20.0f);
+                terms[HB_R_ORIENTATION * TILE + lane] = (a + g) / 2.0f;
+            }
+            if (h1) {   // tracking_ang_vel :435-443, tracking_lin_vel :426-433
+                const float ea = (cmd[2] - ang.z) * (cmd[2] - ang.z);
+                terms[HB_R_TRACKING_ANG_VEL * TILE + lane] = expf(-ea * p.tracking_sigma);
+                const float ex = cmd[0] - lin.x, ey = cmd[1] - lin.y;
+                terms[HB_R_TRACKING_LIN_VEL * TILE + lane] = expf(-(ex * ex + ey * ey) * p.tracking_sigma);
+            }
+            if (h0 && T::OPT && p.reward_scale[HB_R_VEL_MISMATCH_EXP] != 0.0f) {      // hector_env.py:395-405
+                const float lm = expf(-(lin.z * lin.z) * 10.0f);
+                const float am = expf(-sqrtf(ang.x * ang.x + ang.y * ang.y) * 5.0f);
+                terms[HB_R_VEL_MISMATCH_EXP * TILE + lane] = (lm + am) / 2.0f;
+            }
+            if (h1 && T::OPT && p.reward_scale[HB_R_TRACK_VEL_HARD] != 0.0f) {        // :407-424
+                const float ex = cmd[0] - lin.x, ey = cmd[1] - lin.y;
+                const float le = sqrtf(ex * ex + ey * ey), ae = fabsf(cmd[2] - ang.z);
+                terms[HB_R_TRACK_VEL_HARD * TILE + lane] = (expf(-le * 10.0f) + expf(-ae * 10.0f)) / 2.0f - 0.2f * (le + ae);
+            }
+            if (h1 && T::OPT && p.reward_scale[HB_R_LOW_SPEED] != 0.0f) {             // :468-499
+                const float sp_abs = fabsf(lin.x), cm_abs = fabsf(cmd[0]);
+                const bool too_low = sp_abs < 0.5f * cm_abs, too_high = sp_abs > 1.2f * cm_abs;
+                const float sgn_v = (lin.x > 0.0f) ? 1.0f : ((lin.x < 0.0f) ? -1.0f : 0.0f);
+                const float sgn_c = (cmd[0] > 0.0f) ? 1.0f : ((cmd[0] < 0.0f) ? -1.0f : 0.0f);
+                float r = 0.0f;
+                if (too_low) r = -1.0f;
+                if (too_high) r = 0.0f;
+                if (!(too_low || too_high)) r = 1.2f;
+                if (sgn_v != sgn_c) r = -2.0f;
+                r = r * ((cm_abs > 0.1f) ? 1.0f : 0.0f);
+                terms[HB_R_LOW_SPEED * TILE + lane] = r;
+            }
+        }
+        HB_STAMP(2);
+        tile_barrier<true>();                                     // ---- barrier 1 ----
+        HB_STAMP(3);
+        const bool reset = valid && (flags[lane] & 1);
+        const float gs = reset ? 0.0f : sm[L.gait_s + lane], gc = reset ? 1.0f : sm[L.gait_c + lane];
+        if (reset) {         // _reset_root_states + _resample_commands + the gravity/euler fix-up (:373-396,321-335,211-214)
+            if (h1) {
+                float u5[5];        // root xy jitter (2) and the command draws (3): columns NDOF .. NDOF+4 of the reset draws
+                if (nz.u_reset) {
+#pragma unroll
+                    for (int k = 0; k < 5; ++k) u5[k] = nz.u_reset[(size_t)env * U_RESET + NDOF + k];
+                } else {
+                    rng_uniforms(rng, env, SLOT_U_RESET, NDOF, 5, u5);
+                }
+#pragma unroll
+                for (int k = 0; k < 13; ++k) root[k] = p.base_init_state[k];
+#pragma unroll
+                for (int k = 0; k < 3; ++k) root[k] += b.env_origins[env * 3 + k];
+                if (p.custom_origins) {
+                    root[0] += p.reset_xy_span * u5[0] + p.reset_xy_lo;
+                    root[1] += p.reset_xy_span * u5[1] + p.reset_xy_lo;
+                }
+                cmd[0] = p.cmd_span[0] * u5[2] + p.cmd_lo[0];
+                cmd[1] = p.cmd_span[1] * u5[3] + p.cmd_lo[1];
+                cmd[3] = p.cmd_span[2] * u5[4] + p.cmd_lo[2];
+                const float keep = (sqrtf(cmd[0] * cmd[0] + cmd[1] * cmd[1]) > 0.2f) ? 1.0f : 0.0f;
+                cmd[0] *= keep, cmd[1] *= keep;
+            }
+            grav = {p.reset_gravity[0], p.reset_gravity[1], p.reset_gravity[2]};
+            eul = {p.reset_euler[0], p.reset_euler[1], p.reset_euler[2]};
+        }
+        if (valid) {
+            if (h1 && reset) {
+#pragma unroll
+                for (int k = 0; k < 13; ++k) b.root_states[(size_t)env * 13 + k] = root[k];
+            } else if (h1 && (stages & HB_STAGE_PUSH)) {
+                b.root_states[(size_t)env * 13 + 7] = root[7], b.root_states[(size_t)env * 13 + 8] = root[8];
+#pragma unroll
+                for (int k = 0; k < 3; ++k) b.root_states[(size_t)env * 13 + 10 + k] = root[10 + k];
+            }
+            if (h0 && derive) {
+                b.base_lin_vel[env * 3] = lin.x, b.base_lin_vel[env * 3 + 1] = lin.y, b.base_lin_vel[env * 3 + 2] = lin.z;
+                b.base_ang_vel[env * 3] = ang.x, b.base_ang_vel[env * 3 + 1] = ang.y, b.base_ang_vel[env * 3 + 2] = ang.z;
+            }
+            if (h1 && do_last) {
+#pragma unroll
+                for (int k = 0; k < 6; ++k) b.last_root_vel[(size_t)env * 6 + k] = root[7 + k];
+            }
+            if (h0) {
+                b.projected_gravity[env * 3] = grav.x, b.projected_gravity[env * 3 + 1] = grav.y, b.projected_gravity[env * 3 + 2] = grav.z;
+                b.base_euler_xyz[env * 3] = eul.x, b.base_euler_xyz[env * 3 + 1] = eul.y, b.base_euler_xyz[env * 3 + 2] = eul.z;
+            }
+            if (h1) {
+#pragma unroll
+                for (int k = 0; k < 4; ++k) b.commands[(size_t)env * 4 + k] = cmd[k];
+            }
+        }
+        if (emit_obs) {      // command input, base velocities, euler, root position, push (hector_env.py:186-226)
+            const int B0 = D.B0;
+            float o[11];
+            o[0] = gs, o[1] = gc;
+            o[2] = cmd[0] * p.obs_lin_vel, o[3] = cmd[1] * p.obs_lin_vel, o[4] = cmd[2] * p.obs_ang_vel;
+            o[5] = ang.x * p.obs_ang_vel, o[6] = ang.y * p.obs_ang_vel, o[7] = ang.z * p.obs_ang_vel;
+            o[8] = eul.x * p.obs_quat, o[9] = eul.y * p.obs_quat, o[10] = eul.z * p.obs_quat;
+            if (h1) {
+#pragma unroll
+                for (int k = 0; k < 5; ++k) {
+                    so[lane * OBS + k] = noisy_clip(o[k], k);
+                    sp[lane * PRIV_PAD + k] = clampf(o[k], -clip, clip);
+                }
+            }
+            if (h0) {
+#pragma unroll
+                for (int k = 0; k < 6; ++k) {
+                    sp[lane * PRIV_PAD + D.P_ANG + k] = clampf(o[5 + k], -clip, clip);
+                    so[lane * OBS + B0 + k] = noisy_clip(o[5 + k], B0 + k);
+                }
+                sp[lane * PRIV_PAD + D.P_LIN] = clampf(lin.x * p.obs_lin_vel, -clip, clip);
+                sp[lane * PRIV_PAD + D.P_LIN + 1] = clampf(lin.y * p.obs_lin_vel, -clip, clip);
+                sp[lane * PRIV_PAD + D.P_LIN + 2] = clampf(lin.z * p.obs_lin_vel, -clip, clip);
+            }
+            if (h1) {
+                if (KIND == KIND_HECTOR) {
+#pragma unroll
+                    for (int k = 0; k < 3; ++k) sp[lane * PRIV_PAD + D.P_ROOT + k] = clampf(root[k], -clip, clip);
+                }
+                sp[lane * PRIV_PAD + D.P_PUSH_F] = clampf(push_f[0], -clip, clip);
+                sp[lane * PRIV_PAD + D.P_PUSH_F + 1] = clampf(push_f[1], -clip, clip);
+#pragma unroll
+                for (int k = 0; k < 3; ++k) sp[lane * PRIV_PAD + D.P_PUSH_T + k] = clampf(push_t[k], -clip, clip);
+            }
+        }
+    };
+    auto joints = [&](auto h0, auto h1) {
+        // ================================ joints ================================
+        if (bulk) hb::mbar_wait(&bar, 0);
+        HB_STAMP(1);
+        // Only q, qd and the actions stay live across the barrier; the previous-step buffers are consumed
+        // (and, on a step, rolled forward: legged_robot.py:146-148) joint by joint before it.
+        // The reference trajectory (compute_ref_state, hector_env.py:90-111 / humanoid_env.py:120-142) is STATE: it is
+        // refreshed inside compute_observations, so the joint_pos reward of a step sees the one the previous step left.
+        const bool joint_pos_on = T::OPT && p.reward_scale[HB_R_JOINT_POS] != 0.0f;
+        const bool use_ref = T::OPT && (KIND == KIND_XBOT || joint_pos_on) && b.ref_dof_pos != nullptr;
+        long long ep_len = 0;
+        if (use_ref && valid) ep_len = b.episode_length_buf[env] + (do_prepare ? 1 : 0);
+        float q[CAP], qd[CAP], act[CAP];
+#pragma unroll
+        for (int j = 0; j < CAP; ++j) {
+            if (T::RUNTIME && j == NDOF) break;
+            q[j] = sm[L.dof + ln * NDOF * 2 + 2 * j];
+            qd[j] = sm[L.dof + ln * NDOF * 2 + 2 * j + 1];
+            act[j] = sm[L.actions + ln * NDOF + j];
+        }
+        if (do_rew || do_last) {
+            float t1 = 0.f, t2 = 0.f, t3 = 0.f, ss = 0.f, acc = 0.f, vel = 0.f, tq = 0.f, rr = 0.f;
+            float dy0 = 0.f, dy1 = 0.f, dy2 = 0.f, dy3 = 0.f, da0 = 0.f, da1 = 0.f, da2 = 0.f, da3 = 0.f;
+            const int yl = D.YAW_L, yr_ = D.YAW_R, al = D.ARM_L, ar_ = D.ARM_R;      // (checked against p by the launcher)
+#pragma unroll
+            for (int j = 0; j < CAP; ++j) {
+                if (T::RUNTIME && j == NDOF) break;
+                const float lact = sm[L.last_actions + ln * NDOF + j];
+                const float llact = sm[L.last_last_actions + ln * NDOF + j];
+                const float ldv = sm[L.last_dof_vel + ln * NDOF + j];
+                if (h0) {
+                    const float d1 = lact - act[j];                    // action_smoothness, hector_env.py:529-539
+                    t1 += d1 * d1;
+                    const float d2 = (act[j] + llact) - 2.0f * lact;
+                    t2 += d2 * d2;
+                    t3 += fabsf(act[j]);
+                    const float d = q[j] - p.default_dof_pos[j];       // default_joint_pos, :357-367
+                    ss += d * d;
+                    // hip yaw / roll of both legs (and, hector_full, the first two arm joints of both arms:
+                    // hector_w_arm_env.py:371-378); the index pairs are task constants
+                    // (j is a compile-time value in the unrolled loop: these are plain register copies)
+                    dy0 = (j == yl) ? d : dy0, dy1 = (j == yl + 1) ? d : dy1;
+                    dy2 = (j == yr_) ? d : dy2, dy3 = (j == yr_ + 1) ? d : dy3;
+                    if (D.HAS_ARMS) {
+                        da0 = (j == al) ? d : da0, da1 = (j == al + 1) ? d : da1;
+                        da2 = (j == ar_) ? d : da2, da3 = (j == ar_ + 1) ? d : da3;
+                    }
+                    if (joint_pos_on && use_ref && do_rew) {           // joint_pos, hector_env.py:264-275
+                        const float e = q[j] - (valid ? b.ref_dof_pos[(size_t)env * NDOF + j] : 0.0f);
+                        rr += e * e;
+                    }
+                }
+                if (h1) {
+                    const float a = (ldv - qd[j]) / dt;                // dof_acc :515-520
+                    acc += a * a;
+                    vel += qd[j] * qd[j];                              // dof_vel :508-513
+                    const float tau = sm[L.torques + ln * NDOF + j];   // torques :501-506
+                    tq += tau * tau;
+                    if (valid && do_last) {                            // legged_robot.py:146-148 (reset envs: zeroed below)
+                        b.last_last_actions[(size_t)env * NDOF + j] = lact;
+                        b.last_actions[(size_t)env * NDOF + j] = act[j];
+                        b.last_dof_vel[(size_t)env * NDOF + j] = qd[j];
+                    }
+                }
+            }
+            if (do_rew && h0) {
+                terms[HB_R_ACTION_SMOOTHNESS * TILE + lane] = (t1 + t2) + 0.05f * t3;
+                float yr = sqrtf(dy0 * dy0 + dy1 * dy1) + sqrtf(dy2 * dy2 + dy3 * dy3);
+                yr = clampf(yr - 0.1f, 0.0f, 50.0f);
+                float djp = expf(-yr * 100.0f);
+                if (D.HAS_ARMS) {
+                    float ar = sqrtf(da0 * da0 + da1 * da1) + sqrtf(da2 * da2 + da3 * da3);
+                    ar = clampf(ar - 0.1f, 0.0f, 25.0f);
+                    djp = djp + expf(-ar * 2.0f);
+                }
+                terms[HB_R_DEFAULT_JOINT_POS * TILE + lane] = djp - 0.01f * sqrtf(ss);
+                if (joint_pos_on) {
+                    const float nrm = sqrtf(rr);
+                    terms[HB_R_JOINT_POS * TILE + lane] = expf(-2.0f * nrm) - 0.2f * clampf(nrm, 0.0f, 0.5f);
+                }
+            }
+            if (do_rew && h1) {
+                terms[HB_R_DOF_ACC * TILE + lane] = acc;
+                terms[HB_R_DOF_VEL * TILE + lane] = vel;
+                terms[HB_R_TORQUES * TILE + lane] = tq;
+            }
+        }
+        HB_STAMP(2);
+        tile_barrier<true>();                                     // ---- barrier 1 ----
+        HB_STAMP(3);
+        const bool reset = valid && (flags[lane] & 1);
+        if (reset) {         // _reset_dofs (legged_robot.py:358-372) + buffer zeroing (:186-191)
+            float u[CAP];
+            if (nz.u_reset) {
+#pragma unroll
+                for (int j = 0; j < CAP; ++j) {
+                    if (T::RUNTIME && j == NDOF) break;
+                    u[j] = nz.u_reset[(size_t)env * U_RESET + j];
+                }
+            } else {
+                rng_uniforms(rng, env, SLOT_U_RESET, 0, NDOF, u);
+            }
+#pragma unroll
+            for (int j = 0; j < CAP; ++j) {
+                if (T::RUNTIME && j == NDOF) break;
+                q[j] = p.default_dof_pos[j] + (p.reset_dof_span * u[j] + p.reset_dof_lo);
+                qd[j] = 0.0f;
+                act[j] = 0.0f;
+                if (h0) {
+                    b.dof_state[((size_t)env * NDOF + j) * 2] = q[j];
+                    b.dof_state[((size_t)env * NDOF + j) * 2 + 1] = 0.0f;
+                    b.actions[(size_t)env * NDOF + j] = 0.0f;
+                    b.last_actions[(size_t)env * NDOF + j] = 0.0f;
+                    b.last_last_actions[(size_t)env * NDOF + j] = 0.0f;
+                    b.last_dof_vel[(size_t)env * NDOF + j] = 0.0f;
+                }
+            }
+        }
+        if (emit_obs) {
+            float sl = 0.0f, sr = 0.0f;
+            if (h0 && use_ref) {       // compute_ref_state of this compute_observations call
+                if (reset) ep_len = 0;
+                const float sn = sinf(TWO_PI_F * (((float)ep_len * dt) / p.cycle_time));
+                sl = fminf(sn, 0.0f), sr = fmaxf(sn, 0.0f);
+                if (fabsf(sn) < 0.1f) sl = sr = 0.0f;               // double support
+            }
+#pragma unroll
+            for (int j = 0; j < CAP; ++j) {
+                if (T::RUNTIME && j == NDOF) break;
+                if (h0 && use_ref) {
+                    float ref = 0.0f;
+#pragma unroll
+                    for (int k = 0; k < 3; ++k) {
+                        const float sc = (k == 1) ? p.ref_scale[1] : p.ref_scale[0];
+                        if (j == p.ref_left[k]) ref = sl * sc;
+                        if (j == p.ref_right[k]) ref = sr * sc;
+                    }
+                    if (valid) b.ref_dof_pos[(size_t)env * NDOF + j] = ref;
+                    if (KIND == KIND_XBOT) sp[lane * PRIV_PAD + D.P_DIFF + j] = clampf(q[j] - ref, -clip, clip);
+                }
+                float v0 = (q[j] - p.default_dof_pos[j]) * p.obs_dof_pos, v1 = qd[j] * p.obs_dof_vel;
+                if (h0) {
+                    sp[lane * PRIV_PAD + 5 + j] = clampf(v0, -clip, clip);
+                    sp[lane * PRIV_PAD + 5 + NDOF + j] = clampf(v1, -clip, clip);
+                    sp[lane * PRIV_PAD + 5 + 2 * NDOF + j] = clampf(act[j], -clip, clip);
+                }
+                if (h1) {
+                    so[lane * OBS + 5 + j] = noisy_clip(v0, 5 + j);
+                    so[lane * OBS + 5 + NDOF + j] = noisy_clip(v1, 5 + NDOF + j);
+                    so[lane * OBS + 5 + 2 * NDOF + j] = noisy_clip(act[j], 5 + 2 * NDOF + j);
+                }
+            }
+        }
+    };
+    auto feet = [&](auto h0, auto h1) {
+        // ================================ feet / contacts / gait ================================
+        long long ep_len = 0;
+        float foot_pos[2][3], foot_vel[2][3], knee_xy[2][2], air[2], fh[2], lz[2];
+        bool last_ct[2];
+        float friction, mass;
+        {
+            const int ev = valid ? env : env0;         // invalid lanes of a ragged tile mirror the tile's first env
+            ep_len = b.episode_length_buf[ev];
+            friction = b.env_frictions[ev], mass = b.body_mass[ev];
+            const float *rs = b.rigid_state + (size_t)ev * p.num_bodies * 13;
+#pragma unroll
+            for (int f = 0; f < 2; ++f) {
+                const float *r = rs + p.feet[f] * 13;
+#pragma unroll
+                for (int k = 0; k < 3; ++k) foot_pos[f][k] = __ldg(r + k), foot_vel[f][k] = __ldg(r + 7 + k);
+                const float *kr = rs + p.knees[f] * 13;
+                knee_xy[f][0] = __ldg(kr), knee_xy[f][1] = __ldg(kr + 1);
+                air[f] = b.feet_air_time[ev * 2 + f];
+                fh[f] = b.feet_height[ev * 2 + f];
+                lz[f] = b.last_feet_z[ev * 2 + f];
+                last_ct[f] = b.last_contacts[ev * 2 + f] != 0;
+            }
+        }
+        if (bulk) hb::mbar_wait(&bar, 0);
+        HB_STAMP(1);
+        const float *cf = sm + L.contact + ln * crow;
+        float foot_f[2][3];
+#pragma unroll
+        for (int f = 0; f < 2; ++f)
+#pragma unroll
+            for (int k = 0; k < 3; ++k) foot_f[f][k] = cf[p.feet[f] * 3 + k];
+        const float root_z = sm[L.root + ln * 13 + 2];
+        bool term = false, time_out = false;
+        float gs = 0.0f, gc = 1.0f, st[2] = {1.0f, 1.0f};
+        const bool ct[2] = {foot_f[0][2] > 5.0f, foot_f[1][2] > 5.0f};
+        if (do_prepare) ep_len += 1;
+        if (h0 && do_term) {   // -------- check_termination, legged_robot.py:155-160 --------
+#pragma unroll 1
+            for (int i = 0; i < p.n_term; ++i) term |= norm3(cf + p.term_bodies[i] * 3) > 1.0f;
+            time_out = ep_len > (long long)p.max_episode_length;
+            term |= time_out;
+        }
+        if (h1 && do_rew) {    // collision, hector_env.py:522-527
+            float coll = 0.f;
+#pragma unroll 1
+            for (int i = 0; i < p.n_pen; ++i) coll += (norm3(cf + p.pen_bodies[i] * 3) > 0.1f) ? 1.0f : 0.0f;
+            terms[HB_R_COLLISION * TILE + lane] = coll;
+        }
+        bool reset = do_step && term;        // the fused step resets what it has just found terminated
+        {   // -------- gait phase, hector_env.py:70-88 --------
+            const float arg = TWO_PI_F * (((float)ep_len * dt) / p.cycle_time);
+            sincosf(arg, &gs, &gc);
+            st[0] = (gs >= 0.0f) ? 1.0f : 0.0f, st[1] = (gs < 0.0f) ? 1.0f : 0.0f;
+            if (fabsf(gs) < 0.1f) st[0] = st[1] = 1.0f;
+        }
+        if (do_rew) {
+            if (h1) {   // base_height, :369-383
+                const float ground = (foot_pos[0][2] * st[0] + foot_pos[1][2] * st[1]) / (st[0] + st[1]);
+                const float h = root_z - (ground - 0.05f);
+                terms[HB_R_BASE_HEIGHT * TILE + lane] = expf(-fabsf(h - p.base_height_target) * 100.0f);
+            }
+            float r_air = 0.f, r_clr = 0.f, cfz = 0.f, num = 0.f, slip = 0.f;
+#pragma unroll
+            for (int f = 0; f < 2; ++f) {
+                if (h0) {   // feet_air_time, :315-329 (stateful)
+                    const bool filt = ct[f] || (st[f] != 0.0f) || last_ct[f];
+                    last_ct[f] = ct[f];
+                    const bool first = (air[f] > 0.0f) && filt;
+                    air[f] += dt;
+                    r_air += clampf(air[f], 0.0f, 0.5f) * (first ? 1.0f : 0.0f);
+                    air[f] *= filt ? 0.0f : 1.0f;
+                }
+                if (h1) {   // feet_clearance, :445-466 (stateful)
+                    const float z = foot_pos[f][2] - 0.05f;
+                    fh[f] += z - lz[f];
+                    lz[f] = z;
+                    const float hit = (fabsf(fh[f] - p.target_feet_height) < 0.01f) ? 1.0f : 0.0f;
+                    r_clr += hit * (1.0f - st[f]);
+                    fh[f] *= ct[f] ? 0.0f : 1.0f;
+                }
+                if (h0) {   // feet_contact_forces :350-355, feet_contact_number :331-339, foot_slip :303-313
+                    cfz += clampf(norm3(foot_f[f]) - p.max_contact_force, 0.0f, 400.0f);
+                    num += (ct[f] == (st[f] != 0.0f)) ? 1.0f : -0.3f;
+                    const float spd = sqrtf(sqrtf(foot_vel[f][0] * foot_vel[f][0] + foot_vel[f][1] * foot_vel[f][1]));
+                    slip += spd * (ct[f] ? 1.0f : 0.0f);
+                }
+            }
+            if (h0) terms[HB_R_FEET_AIR_TIME * TILE + lane] = r_air;
+            if (h1) terms[HB_R_FEET_CLEARANCE * TILE + lane] = r_clr;
+            if (h0) {
+                terms[HB_R_FEET_CONTACT_FORCES * TILE + lane] = cfz;
+                terms[HB_R_FEET_CONTACT_NUMBER * TILE + lane] = num / 2.0f;
+                terms[HB_R_FOOT_SLIP * TILE + lane] = slip;
+            }
+            if (h1) {   // feet_distance :277-287, knee_distance :290-300
+                float dx = foot_pos[0][0] - foot_pos[1][0], dy = foot_pos[0][1] - foot_pos[1][1];
+                float d = sqrtf(dx * dx + dy * dy);
+                float dmin = clampf(d - p.min_dist, -0.5f, 0.0f), dmax = clampf(d - p.max_dist, 0.0f, 0.5f);
+                terms[HB_R_FEET_DISTANCE * TILE + lane] = (expf(-fabsf(dmin) * 100.0f) + expf(-fabsf(dmax) * 100.0f)) / 2.0f;
+                dx = knee_xy[0][0] - knee_xy[1][0], dy = knee_xy[0][1] - knee_xy[1][1];
+                d = sqrtf(dx * dx + dy * dy);
+                dmin = clampf(d - p.min_dist, -0.5f, 0.0f), dmax = clampf(d - p.max_dist / 2.0f, 0.0f, 0.5f);
+                terms[HB_R_KNEE_DISTANCE * TILE + lane] = (expf(-fabsf(dmin) * 100.0f) + expf(-fabsf(dmax) * 100.0f)) / 2.0f;
+            }
+        }
+        if (h0) {
+            if (stages & HB_STAGE_RESET_ALL) reset = true;
+            if ((stages & HB_STAGE_RESET_MASK) && valid) reset = reset || (b.reset_buf[env] != 0);   // reset_idx(env_ids)
+            reset = reset && valid;
+            flags[lane] = (reset ? 1 : 0) | (time_out ? 2 : 0);
+            sm[L.gait_s + lane] = gs, sm[L.gait_c + lane] = gc;
+        }
+        HB_STAMP(2);
+        tile_barrier<true>();                                     // ---- barrier 1 ----
+        HB_STAMP(3);
+        if (!h0) reset = (flags[lane] & 1) != 0;                 // (the first half's flag)
+        if (reset) {
+            ep_len = 0, air[0] = air[1] = 0.0f;
+            st[0] = st[1] = 1.0f;                                   // phase 0: sin = 0 -> double support
+        }
+        if (valid) {
+            if (h0) {
+                b.feet_air_time[env * 2] = air[0], b.feet_air_time[env * 2 + 1] = air[1];
+                b.episode_length_buf[env] = ep_len;
+                if (any_reset) b.reset_buf[env] = reset ? 1 : 0;
+                else if (do_term) b.reset_buf[env] = term ? 1 : 0;           // check_termination on its own: the mask only
+                if (do_term) b.time_out_buf[env] = time_out ? 1 : 0;
+            }
+            if (do_rew) {
+#pragma unroll
+                for (int f = 0; f < 2; ++f) {
+                    if (h0) b.last_contacts[env * 2 + f] = last_ct[f] ? 1 : 0;
+                    if (h1) b.feet_height[env * 2 + f] = fh[f], b.last_feet_z[env * 2 + f] = lz[f];
+                }
+            }
+        }
+        if (h1 && emit_obs) {
+            if (KIND == KIND_HECTOR) {
+#pragma unroll
+                for (int f = 0; f < 2; ++f)
+#pragma unroll
+                    for (int k = 0; k < 3; ++k) {
+                        sp[lane * PRIV_PAD + D.P_FEET_POS + f * 3 + k] = clampf(foot_pos[f][k], -clip, clip);
+                        sp[lane * PRIV_PAD + D.P_FEET_VEL + f * 3 + k] = clampf(foot_vel[f][k], -clip, clip);
+                    }
+            }
+            sp[lane * PRIV_PAD + D.P_FRICTION] = clampf(friction, -clip, clip);
+            sp[lane * PRIV_PAD + D.P_MASS] = clampf(mass / 30.0f, -clip, clip);
+            sp[lane * PRIV_PAD + D.P_STANCE] = st[0], sp[lane * PRIV_PAD + D.P_STANCE + 1] = st[1];
+            sp[lane * PRIV_PAD + D.P_CONTACT] = ct[0] ? 1.0f : 0.0f, sp[lane * PRIV_PAD + D.P_CONTACT + 1] = ct[1] ? 1.0f : 0.0f;
+        }
+    };
+    auto ledger = [&](auto h0, auto h1) {
+        // ================================ ledger ================================
+        // (terms with scale 0 are not part of the task: the reference has no episode sum for them - their rows stay zero
+        // and are neither read nor written)
+        float sums[HB_NUM_REWARDS];
+#pragma unroll
+        for (int k = 0; k < HB_NUM_REWARDS; ++k)
+            sums[k] = (valid && p.reward_scale[k] != 0.0f) ? b.episode_sums[(size_t)k * N + env] : 0.0f;
+        if (with_noise && !tape_noise && emit_obs) {
+            // the tile's observation noise, drawn by this otherwise idle warp while the other roles are in phase A:
+            // 11 Philox calls of 4 normals per env; calls whose four columns all have zero noise scale are skipped
+            const int CALLS = (OBS + 3) / 4;
+            float *z = sm + L.z_obs;
+            for (int c = h0 ? lane : lane + 32; c < nv * CALLS; c += 64) {      // (the pair interleaves)
+                const int e = c / CALLS, q = c - e * CALLS;
+                bool any = false;
+#pragma unroll
+                for (int k = 0; k < 4; ++k) any = any || (q * 4 + k < OBS && p.noise_scale_vec[q * 4 + k] != 0.0f);
+                float z4[4] = {0.f, 0.f, 0.f, 0.f};
+                if (any) rng_normal4(rng, env0 + e, SLOT_Z_OBS + q, z4);
+#pragma unroll
+                for (int k = 0; k < 4; ++k)
+                    if (q * 4 + k < OBS) z[e * OBS + q * 4 + k] = z4[k];
+            }
+        }
+        HB_STAMP(2);
+        tile_barrier<true>();                                     // ---- barrier 1 ----
+        HB_STAMP(3);
+        const bool reset = valid && (flags[lane] & 1);
+        float *rsums = sm + L.rsums;                           // the reset envs' sums (the first half still reads terms)
+        if (do_rew) {        // compute_reward, legged_robot.py:216-234: alphabetical accumulation
+            float rew = 0.0f;
+#pragma unroll
+            for (int k = 0; k < HB_NUM_REWARDS; ++k) {
+                if (p.reward_scale[k] != 0.0f) {
+                    const float r = terms[k * TILE + lane] * p.reward_scale[k];
+                    rew += r;
+                    sums[k] += r;
+                }
+            }
+            if (h0) {
+                if (p.only_positive_rewards) rew = fmaxf(rew, 0.0f);
+                if (valid) b.rew_buf[env] = rew;
+            }
+        }
+        const unsigned ballot = __ballot_sync(0xffffffffu, reset);
+        __syncwarp();
+#pragma unroll
+        for (int k = 0; k < HB_NUM_REWARDS; ++k) {
+            if (h1 && p.reward_scale[k] != 0.0f) {
+                rsums[k * TILE + lane] = reset ? sums[k] : 0.0f;    // episode sums of the envs being reset (:198-201)
+                if (reset) sums[k] = 0.0f;
+                if (valid) b.episode_sums[(size_t)k * N + env] = sums[k];
+            }
+        }
+        __syncwarp();
+        // ---------------- reset ids + episode means ----------------
+        // Each tile publishes its ballot; reset_finalize_kernel turns the ballots into the ascending id
+        // list (like reset_buf.nonzero()) and the count.  The per-term sums of the reset envs
+        // (legged_robot.py:198-201) go straight into 18 fp64 accumulators: fp64 addition of these
+        // fp32 values is order-independent far below fp32 resolution.
+        if (h1 && ballot && lane < HB_NUM_REWARDS && p.reward_scale[lane] != 0.0f) {
+            float v = 0.0f;
+#pragma unroll 8
+            for (int e = 0; e < TILE; ++e) v += rsums[lane * TILE + ((e + lane) & 31)];
+            atomicAdd(b.scratch_sums + lane, (double)v);
+        }
+        if (h0 && lane == 0) b.scratch_ballots[blockIdx.x] = ballot;     // consumed by reset_finalize_kernel
+    };
+    if (role == 0) run(base);
+    else if (role == 1) run(joints);
+    else if (role == 2) run(feet);
+    else run(ledger);
+
+    // ---------------- coalesced store of the newest frames into the last slot of the stacked buffers ----------------
+    // by the three roles that wrote them (named barrier 2, 96 threads; wide: their six warps, 192 threads); the ledger is
+    // busy with its ticket
+    HB_STAMP(4);
+    constexpr int NT = 6 * TILE;
+    if (warp < NT / 32) {
+        asm volatile("bar.sync 2, 192;" ::: "memory");            // ---- barrier 2 ----
+        HB_STAMP(5);
+        if (emit_obs) {
+            // NT threads walk the tile's frames with (row, column) advanced incrementally: no per-element division.
+            // Privileged frames leave as 8-byte pairs (row starts are 8-byte aligned: 4200 r + 3920 bytes).
+            const int P2 = PRIV / 2;
+            const int orow = p.frame_stack * OBS, prow = p.c_frame_stack * PRIV;
+            const int ostride = p.obs_ld ? p.obs_ld : orow, pstride = p.priv_ld ? p.priv_ld : prow;   // row pitch
+            const int t = threadIdx.x;
+            if ((PRIV & 1) == 0 && ((pstride | prow) & 1) == 0 && (reinterpret_cast<uintptr_t>(priv_new) & 7u) == 0) {
+                int r = t / P2, c2 = t - r * P2;
+                float2 *dst = reinterpret_cast<float2 *>(priv_new + (size_t)env0 * pstride + (prow - PRIV));
+                const float2 *src = reinterpret_cast<const float2 *>(sp);
+                const int half = pstride / 2;
+                while (r < nv) {
+                    dst[(size_t)r * half + c2] = src[r * P2 + c2];
+                    r += NT / P2, c2 += NT % P2;
+                    if (c2 >= P2) c2 -= P2, r += 1;
+                }
+            } else {
+                int r = t / PRIV, c = t - r * PRIV;
+                while (r < nv) {
+                    priv_new[(size_t)(env0 + r) * pstride + (prow - PRIV) + c] = sp[r * PRIV + c];
+                    r += NT / PRIV, c += NT % PRIV;
+                    if (c >= PRIV) c -= PRIV, r += 1;
+                }
+            }
+            int r = t / OBS, c = t - r * OBS;
+            float *dst = obs_new + (size_t)env0 * ostride + (orow - OBS);
+            while (r < nv) {
+                dst[(size_t)r * ostride + c] = so[r * OBS + c];
+                r += NT / OBS, c += NT % OBS;
+                if (c >= OBS) c -= OBS, r += 1;
+            }
+        }
+    }
+    HB_STAMP(6);
+    HB_GT(1);
+}
+
 // ------------------------------------------------------------------------------------------
 // a8 (stacking): new[:, 0:(S-1)*F] = prev[:, F:S*F]  — a flat copy shifted by one frame with a
 // hole of F floats per row (the newest frame, written by post_physics_kernel).  With kZero the
@@ -1462,6 +2218,11 @@ mirror_frames_kernel(const float *__restrict__ obs, int obs_ld, int row_a, int f
 
 int g_use_bulk = 1;
 int g_runtime_task = 0;      // 1: the three built robots too run post_physics_kernel with the layout read at run time
+int g_post_warps = 0;        // warps per post_physics_kernel tile, 4 or 8 (0: by shard width)
+// Shards of at most this many 32-env tiles per SM run the eight-warp post-physics kernel: there the tiles of an SM are too
+// few to hide one another's dependent chains (DESIGN.md §3, scripts/ab_post_physics.py: faster at 2.4 and 2.6 tiles per
+// SM, slower from 3.0)
+constexpr float POST_WIDE_MAX_TILES_PER_SM = 2.5f;
 
 // Frame stacks of the three tasks (hector_config.py:8-20, hector_w_arm_config.py:8-20, humanoid_config.py:42-52): rows
 // either dense or at the 128-byte pitch ceil32(row + 1) (TMA-addressable: the rollout storage's slots)
@@ -1483,19 +2244,21 @@ uint32_t shift_blocks(uint32_t total) { return ((total + 3u) / 4u + 4 * 256 - 1)
 
 bool fits_u32(int n, int row) { return (long long)n * row + 64 * 1024 < (1ll << 32); }
 
-template <typename T, bool kBulk>
+template <typename T, bool kBulk, bool kWide>
 int launch_post_physics(const hb_env_params *p, const hb_env_buffers *buf, const hb_env_noise *noise, float *obs_new,
                         float *priv_new, int32_t stages, cudaStream_t st) {
     const bool with_noise = p->add_noise && (noise->z_obs || noise->rng_counter);
-    const TileLayout L = make_layout(p->num_bodies, with_noise, p->num_dof, p->num_single_obs, p->num_single_priv);
+    const TileLayout L = make_layout(p->num_bodies, with_noise, p->num_dof, p->num_single_obs, p->num_single_priv, kWide);
+    const auto kernel = kWide ? post_physics_wide_kernel<kBulk, T> : post_physics_kernel<kBulk, T>;
     const size_t smem = (size_t)L.total * sizeof(float);
     const int tiles = (p->num_envs + TILE - 1) / TILE;
     static bool attr_set = false;
     if (!attr_set) {
-        HB_CUDA(cudaFuncSetAttribute(post_physics_kernel<kBulk, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, POST_SMEM_MAX));
+        HB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, POST_SMEM_MAX));
         attr_set = true;
     }
-    HB_CUDA(hb::launch_pdl(hb::use_pdl_post(p->num_envs), post_physics_kernel<kBulk, T>, dim3(tiles), dim3(4 * TILE), smem, st, *p, *buf,
+    HB_CUDA(hb::launch_pdl(hb::use_pdl_post(p->num_envs), kernel, dim3(tiles), dim3((kWide ? 8 : 4) * TILE),
+                           smem, st, *p, *buf,
                            *noise, obs_new, priv_new, (int)stages));
     HB_CHECK_LAUNCH("post_physics_kernel");
     return HB_OK;
@@ -1667,6 +2430,11 @@ int hb_set_option(const char *name, int value) {
         g_runtime_task = value != 0;
         return HB_OK;
     }
+    if (name && !strcmp(name, "post_warps")) {
+        HB_REQUIRE(value == 0 || value == 4 || value == 8, "hb_set_option: post_warps must be 0, 4 or 8");
+        g_post_warps = value;
+        return HB_OK;
+    }
     if (name && !strcmp(name, "gemm_pdl")) {
         hb::g_gemm_pdl = value != 0;
         return HB_OK;
@@ -1826,10 +2594,15 @@ int hb_env_post_physics(const hb_env_params *p, const hb_env_buffers *buf, const
     // a config that scales none of the optional terms runs the kernel compiled without them
     const bool opt = p->reward_scale[HB_R_JOINT_POS] != 0.0f || p->reward_scale[HB_R_VEL_MISMATCH_EXP] != 0.0f ||
                      p->reward_scale[HB_R_TRACK_VEL_HARD] != 0.0f || p->reward_scale[HB_R_LOW_SPEED] != 0.0f;
+    const int tiles = (p->num_envs + TILE - 1) / TILE;
+    const bool wide = g_post_warps ? g_post_warps == 8 : tiles <= POST_WIDE_MAX_TILES_PER_SM * hb::sm_count();
     auto launch = [&](auto task) {
         using T = decltype(task);
-        return bulk ? launch_post_physics<T, true>(p, buf, noise, obs_new, priv_new, stages, st)
-                    : launch_post_physics<T, false>(p, buf, noise, obs_new, priv_new, stages, st);
+        if (wide)
+            return bulk ? launch_post_physics<T, true, true>(p, buf, noise, obs_new, priv_new, stages, st)
+                        : launch_post_physics<T, false, true>(p, buf, noise, obs_new, priv_new, stages, st);
+        return bulk ? launch_post_physics<T, true, false>(p, buf, noise, obs_new, priv_new, stages, st)
+                    : launch_post_physics<T, false, false>(p, buf, noise, obs_new, priv_new, stages, st);
     };
     if (matches(10, HB_TASK_HECTOR, Hector::OBS, Hector::PRIV)) return opt ? launch(Hector{}) : launch(HectorSlim{});
     if (matches(18, HB_TASK_HECTOR, HectorFull::OBS, HectorFull::PRIV)) return opt ? launch(HectorFull{}) : launch(HectorFullSlim{});
